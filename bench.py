@@ -10,7 +10,13 @@ functions and grid points are sharded over ranks (strong scaling of the same pro
 NCCL all-reduce of the MO-space partial sigma.
 
 One JSON line on stdout (rank 0).  `value` = sigma-vectors/s with vectors resident in HBM; `e2e` = the same
-through the reference-facing `vind` with HOST vectors (H2D + D2H inside the timed region).
+through the reference-facing `vind` with HOST vectors (H2D + D2H inside the timed region).  `--steps` / `--warmup` set the
+timed and untimed calls of every timed loop (headline, e2e, configs table).
+
+    python bench.py ... --dump-outputs DIR                   also write the last timed step's sigma vectors to DIR/sigma.npy
+                                                             (git ignores bench_outputs/)
+
+The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -85,7 +91,41 @@ def parse():
                     help="at N=1 with the headline config: append compact records of BASELINE configs 1-4 measured in the same run")
     ap.add_argument("--exchange-slices", type=int, default=int(os.environ.get("XTD_OZAKI", "-1")),
                     help="exchange contraction: 0 = FP64 DMMA, 3..8 = INT8 tensor-core emulation with that many 7-bit digits, -1 = default")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the sigma vectors of the last timed step to DIR/sigma.npy (float64, "
+                         f"a fixed seeded sample of columns when larger than {DUMP_LIMIT_BYTES // 10**6} MB)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup < 0:
+        ap.error("--warmup must not be negative")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the B200 arm computed")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 * 10**6      # everything --dump-outputs writes, headers included
+DUMP_SEED = 20240917
+
+
+def sample_columns(a: np.ndarray, max_bytes: int, seed: int = DUMP_SEED):
+    """`a` itself if it fits in `max_bytes`, else all its rows at a seeded, sorted sample of columns that does.
+    Returns (array, column indices or None)."""
+    if a.nbytes <= max_bytes:
+        return a, None
+    ncol = max(1, max_bytes // (a.shape[0] * a.itemsize))
+    cols = np.sort(np.random.default_rng(seed).choice(a.shape[1], size=ncol, replace=False))
+    return np.ascontiguousarray(a[:, cols]), cols
+
+
+def dump_outputs(out_dir: str, name: str, a: np.ndarray) -> dict:
+    """Write `a` (float64, [rows, cols]) as out_dir/<name>.npy, sampled by columns to stay within DUMP_LIMIT_BYTES."""
+    os.makedirs(out_dir, exist_ok=True)
+    kept, cols = sample_columns(np.asarray(a, dtype=np.float64), DUMP_LIMIT_BYTES - 4096)
+    path = os.path.join(out_dir, f"{name}.npy")
+    np.save(path, kept)
+    return {"file": path, "shape": list(kept.shape), "full_shape": list(a.shape), "dtype": "float64",
+            "columns": "all" if cols is None else f"{cols.size} sampled with numpy default_rng({DUMP_SEED}), sorted"}
 
 
 # ---------------------------------------------------------------------------------------------------------
@@ -444,6 +484,10 @@ def main():
             phase_flops[k] = phase_flops.get(k, 0.0) + v
     e1.record()
     barrier()
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # what the caller of the timed path receives from the last timed step (all ranks hold the reduced sigma)
+        dumped = {"sigma": dump_outputs(args.dump_outputs, "sigma", out.cpu().numpy())}
     ms_total = e0.elapsed_time(e1)
     launches = eng.lib.xtd_launch_count() - launches0
     flops = eng.stats()["flops_gemm"]
@@ -587,6 +631,8 @@ def main():
     }
     if dav is not None:
         out_json["davidson"] = dav
+    if dumped is not None:
+        out_json["dumped_outputs"] = dumped
     if world == 1 and not args.no_cpu_baseline:
         cb = cpu_reference_rate(dp)
         if dav is not None and cb.get("value"):
@@ -602,11 +648,11 @@ def main():
         table = []
         for c in (1, 2, 3, 4):
             try:
-                table.append(compact_config_record(c))
+                table.append(compact_config_record(c, steps=args.steps, warmup=args.warmup))
             except Exception as ex:      # a failed side measurement must not lose the headline record
                 table.append({"config": c, "error": f"{type(ex).__name__}: {ex}"})
         try:
-            table.append(zvector_record(4))
+            table.append(zvector_record(4, steps=args.steps, warmup=args.warmup))
         except Exception as ex:
             table.append({"config": 4, "method": "zvector_roks", "error": f"{type(ex).__name__}: {ex}"})
         out_json["configs"] = table

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""Generate golden sigma vectors by executing the REFERENCE's own code (read from /root/reference,
-which exists only in the build container) on seeded synthetic inputs.
+"""Generate golden sigma vectors by executing the REFERENCE's own code (a checkout of the original XTDDFT source,
+named by the XTDDFT_REFERENCE environment variable; it is not part of this repository) on seeded synthetic inputs.
 
 What runs verbatim from the reference (after the two minimal Appendix-D fixes: the full-width comma at
 XSF_TDA.py:1137 and the bare-module imports):
@@ -17,7 +17,7 @@ supplied by the stub below, coded independently of `oracle/` from the published 
   numint block_loop / rho evaluator / nr_uks_fxc / sparse AO helpers (dense loops), a Slater-exchange
   `eval_xc_eff`, SCF accessors (make_rdm1, get_veff, get_hcore) returning the synthetic Fock matrices.
 
-Usage (build container only):  python tests/golden/make_golden.py
+Usage:  XTDDFT_REFERENCE=<checkout of the original XTDDFT> python tests/golden/make_golden.py
 Writes tests/golden/*.npz.  Inputs are regenerated from the seed stored in each file.
 """
 import importlib
@@ -32,7 +32,7 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 OUT = os.environ.get("XTD_GOLDEN_OUT", HERE)      # tests regenerate into a temporary directory and diff
 ROOT = os.path.dirname(os.path.dirname(HERE))
-REF = "/root/reference"
+REF = os.environ.get("XTDDFT_REFERENCE", "")          # checkout of the original XTDDFT source
 sys.path.insert(0, ROOT)
 
 from xtddft_b200.synth import make_problem  # noqa: E402  (input generator, product side)
@@ -437,7 +437,9 @@ def install_stubs():
 
 
 def load_reference_modules():
-    """Import the reference package from /root/reference with the Appendix-D source fixes applied in memory."""
+    """Import the reference package from $XTDDFT_REFERENCE with the Appendix-D source fixes applied in memory."""
+    if not (REF and os.path.isdir(os.path.join(REF, "xtddft"))):
+        raise SystemExit("set XTDDFT_REFERENCE to a checkout of the original XTDDFT source (the directory holding xtddft/)")
     sys.path.insert(0, REF)
     sys.path.insert(0, os.path.join(REF, "xtddft", "utils"))     # bare `import Davidson`
     sys.path.insert(0, os.path.join(REF, "xtddft"))              # bare `from utils import ...`

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Golden vectors for the post-Davidson property pass (SURVEY 8f row f1), produced by executing the REFERENCE's own
-methods from /root/reference (build container only) on seeded synthetic states and one-electron integrals:
+methods from $XTDDFT_REFERENCE (see make_golden.py) on seeded synthetic states and one-electron integrals:
 
   xtddft/XTDA.py          XTDA.osc_str, XTDA.rot_str, XTDA.deltaS2                (ground -> excited moments)
   xtddft/XSF_TDA_GPU.py   XSF_TDA_GPU.calculate_TDM_R / calculate_TDM_U           (state-to-state oscillator matrix;

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Golden vectors for the Z-vector equation of the spin-flip-up TDA gradients (SURVEY 8f row f3), produced by executing the
-REFERENCE's own `grad_elec` functions from /root/reference (build container only) on seeded synthetic inputs:
+REFERENCE's own `grad_elec` functions from $XTDDFT_REFERENCE (see make_golden.py) on seeded synthetic inputs:
 
   xtddft/grad_hb/tdroks_sfu.py   grad_elec: internal variables, `_contract_xc_kernel` (collinear kernel), the Q matrix / right-hand
                                  side `w` (:207-274), the ROHF orbital-Hessian closure `matvec` (:284-321)

@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -28,6 +30,27 @@ def test_reference_arm_json_line():
     assert cb["kind"] == "port" and cb["cores"] >= 1 and cb["value"] == d["value"] and "sample" in cb
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert d["value"] > 0
+
+
+def test_step_counts_and_dump_flag_are_checked():
+    for args in (["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        res = _run(args, timeout=120)
+        assert res.returncode == 2 and "error:" in res.stderr, args
+
+
+def test_dump_sample_is_seeded_and_bounded():
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_under_test", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    a = np.arange(3 * 1000, dtype=np.float64).reshape(3, 1000)
+    kept, cols = bench.sample_columns(a, a.nbytes)
+    assert kept is a and cols is None
+    kept, cols = bench.sample_columns(a, 3 * 8 * 100 + 7)
+    assert kept.shape == (3, 100) and kept.nbytes <= 3 * 8 * 100 + 7
+    assert np.all(np.diff(cols) > 0) and np.array_equal(kept, a[:, cols])
+    again, cols2 = bench.sample_columns(a, 3 * 8 * 100 + 7)
+    assert np.array_equal(cols, cols2) and np.array_equal(kept, again)
 
 
 def test_b200_arm_has_no_cpu_fallback():

@@ -1,8 +1,6 @@
 """SURVEY 8f row f3 on the B200: the Z-vector operator (engine plan with the transposed-density exchange term and the transposed local
 couplings) against the fixtures of the reference's own `matvec` / `fvind` closures and against the oracle, through the C-ABI; the
 device Krylov solve against dense solves of the oracle's operator.  Needs a B200."""
-import os
-
 import numpy as np
 import pytest
 
@@ -121,9 +119,6 @@ def test_workload_route_solves(torch_cuda):
     eng.close()
 
 
-@pytest.mark.skipif(os.environ.get("XTD_RUN_PENDING") != "1",
-                    reason="first GPU run pending: written after the round's GPU budget was spent (CPU-verified through the plan "
-                           "interpreter, tests/test_zvector_cpu.py); run with XTD_RUN_PENDING=1")
 @pytest.mark.parametrize("tag", TAGS)
 def test_rhs_and_w_matrix_on_device(torch_cuda, golden_dir, tag):
     """`ZVector.rhs` / `ZVector.w_matrix` (whole-MO-space engine plans) against the right-hand side and the W matrix the reference's own

@@ -1,8 +1,8 @@
 """Host-side pieces of the PRODUCT (not the oracle) against the fixtures the reference's own code produced:
 initial guesses (row a4: XTDA.get_init_guess, SF_TDA.init_guess, XSF_TDA._build_initial_guess_from_gaps), amplitude layouts
-(row a18: order_pyscf2my, so2st, st2so, deal_v_davidson, get_vect) -- and, where /root/reference exists (the build
-container), a regeneration of every fixture into a temporary directory that must reproduce the committed files bit for
-bit.  CPU only."""
+(row a18: order_pyscf2my, so2st, st2so, deal_v_davidson, get_vect) -- and, where XTDDFT_REFERENCE names a checkout of the
+original XTDDFT source (not part of this repository), a regeneration of every fixture into a temporary directory that must
+reproduce the committed files bit for bit.  CPU only."""
 import os
 import subprocess
 import sys
@@ -73,7 +73,11 @@ def test_xsf_init_guess(golden_dir, tag):
     assert np.array_equal(x0, d["x0"])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/xtddft"), reason="the reference tree exists only in the build container")
+REFERENCE = os.environ.get("XTDDFT_REFERENCE", "")
+
+
+@pytest.mark.skipif(not (REFERENCE and os.path.isdir(os.path.join(REFERENCE, "xtddft"))),
+                    reason="needs XTDDFT_REFERENCE: a checkout of the original XTDDFT source, which is not part of this repository")
 def test_goldens_regenerate_bit_for_bit(golden_dir, tmp_path):
     """Re-run the reference's own code (make_golden.py, make_golden_properties.py, make_golden_zvector.py) and diff against the
     committed files."""
