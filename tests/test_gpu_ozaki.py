@@ -110,13 +110,10 @@ def test_ozaki_many_groups_and_splits(torch_cuda):
 # ---- the engine's exchange contraction on the emulated path ------------------------------------------------------------
 @pytest.mark.parametrize("slices,tol", [(8, 1e-12), (7, 1e-12), (6, 1e-11), (5, 1e-9)])
 @pytest.mark.parametrize("method", ["sf", "xtda"])
-@pytest.mark.parametrize("fuse", ["1", "0"])
-def test_engine_emulated_exchange(torch_cuda, monkeypatch, slices, tol, method, fuse):
+def test_engine_emulated_exchange(torch_cuda, monkeypatch, slices, tol, method):
     """SF-TDA / X-TDA sigma with the uniform-weight exchange contraction on the INT8 tensor cores against the oracle, with
-    several aux chunks (ragged last group: naux = 61), several tiles in M and N, 5 vectors.  fuse = 1: the half-transform
-    U = Loo . z runs on the INT8 tensor cores too and writes the digit planes of U directly (a-priori row scales);
-    fuse = 0: DMMA half-transform + slicing pass with exact row maxima."""
-    monkeypatch.setenv("XTD_OZ_FUSE", fuse)
+    several aux chunks (ragged last group: naux = 61), several tiles in M and N, 5 vectors.  The half-transform
+    U = Loo . z runs on the INT8 tensor cores too and writes the digit planes of U directly (a-priori row scales)."""
     from oracle import sigma as osig
     from xtddft_b200 import plan as planmod
     from xtddft_b200.engine import SigmaEngine
@@ -243,8 +240,9 @@ def test_engine_emulated_block_weighted_exchange(torch_cuda, monkeypatch, nc, no
 def test_engine_emulated_split_gradient_grid_path(torch_cuda, monkeypatch, method, restricted, short_k):
     """Value + gradient kernels (UKS GGA of X-TDA on two channels, multicollinear GGA spin flip) in the split-gradient form with
     its four value GEMMs on the INT8 tensor cores (two of them batched over the trial vectors), two grid chunks with a ragged
-    last block; the streaming kernel between them is the fp64 one.  short_k = 512 (the default): the occupied-side forward GEMM,
-    whose contraction length is the occupied count, stays on the DMMA GEMM; short_k = 0 forces all four onto the INT8 kernel."""
+    last block; the streaming kernel between them is the fp64 one.  short_k = 512 (above the occupied count, as the default of 100 is
+    here): the occupied-side forward GEMM, whose contraction length is the occupied count, stays on the DMMA GEMM; short_k = 0 forces
+    all four onto the INT8 kernel."""
     monkeypatch.setenv("XTD_OZ_SHORT_K", short_k)
     from oracle import sigma as osig
     from xtddft_b200 import plan as planmod

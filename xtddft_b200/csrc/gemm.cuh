@@ -360,8 +360,6 @@ struct GemmContext {
   bool naive = false;        // XTD_GEMM=naive
   double* split_ws = nullptr;  // workspace for split-K partials
   size_t split_ws_bytes = 0;
-  bool attr_set = false;
-  bool tails = true;         // partial last tiles get their own warp layout (XTD_GEMM_TAILS=0 disables)
   // statistics
   double flops = 0.0;        // executed useful flops (2*M*N*K*nouter*batches)
   unsigned long long launches = 0;
@@ -380,7 +378,6 @@ inline int gemm_context_init(GemmContext& ctx) {
   XTD_CUDA(cudaDeviceGetAttribute(&ctx.num_sms, cudaDevAttrMultiProcessorCount, dev));
   const char* e = getenv("XTD_GEMM");
   ctx.naive = (e && e[0] == 'n');
-  ctx.tails = !(getenv("XTD_GEMM_TAILS") && getenv("XTD_GEMM_TAILS")[0] == '0');
   return XTD_OK;
 }
 
@@ -522,8 +519,8 @@ inline int gemm(GemmContext& ctx, const GemmDesc& d, cudaStream_t stream) {
               "gemm: C must be 16-byte aligned with even ldc");
   // A short last tile in M or N (<= 64 of 128) gets a warp layout that covers only its live part (dmma_consume).
   const int m_tail = d.M % BM, n_tail = d.N % BN;
-  if (ctx.tails && m_tail > 0 && m_tail <= 64) kp.m_tail_cfg = m_tail <= 16 ? 4 : 3;
-  if (ctx.tails && n_tail > 0 && n_tail <= 64) kp.n_tail_cfg = n_tail <= 32 ? 2 : 1;
+  if (m_tail > 0 && m_tail <= 64) kp.m_tail_cfg = m_tail <= 16 ? 4 : 3;
+  if (n_tail > 0 && n_tail <= 64) kp.n_tail_cfg = n_tail <= 32 ? 2 : 1;
   const dim3 grd(tm, tn, (unsigned)(d.batches * splits));
   const bool tails = kp.m_tail_cfg || kp.n_tail_cfg;
 #define XTD_LAUNCH(AK, BK_)                                                        \

@@ -950,18 +950,6 @@ inline int oz_gemm_launch_cn(const OzGemmParams& p, cudaStream_t st) {
   return XTD_OK;
 }
 
-// cluster width along N: the widest of 4, 2, 1 that divides the number of column tiles (XTD_OZ_CLUSTER overrides)
-inline int oz_cluster_width(int nnt) {
-  static int forced = -1;
-  if (forced < 0) {
-    const char* e = getenv("XTD_OZ_CLUSTER");
-    forced = e ? atoi(e) : 0;
-  }
-  int cn = forced > 0 ? forced : 2;
-  while (cn > 1 && nnt % cn) cn /= 2;
-  return cn;
-}
-
 template <int S>
 inline int oz_gemm_p_launch(const OzGemmParams& p, cudaStream_t st) {
   static bool attr_set[64] = {false};
@@ -984,26 +972,18 @@ inline int oz_gemm_p_launch(const OzGemmParams& p, cudaStream_t st) {
 // Which kernel runs a contraction: the persistent one pays off when a tile holds one or two accumulation groups (grid GEMMs, short
 // contractions: config 5 grid GEMMs 163 -> 148 ms at a LOWER clock), the one-tile-per-CTA kernel with its cluster multicast of the A
 // tile for long contractions (exchange: 587 vs 646 ms -- the step is power-capped and the multicast halves the A traffic per SM).
-// XTD_OZ_PERSISTENT = 0 never / 1 always / unset: by the number of groups per tile.
 inline bool oz_persistent(const OzGemmParams& p) {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("XTD_OZ_PERSISTENT");
-    v = e ? atoi(e) : 2;
-  }
-  if (v != 2) return v != 0;
   const int ngroups = (p.nq + p.group - 1) / p.group;
   return ngroups <= 2 * p.splits;
 }
 
+// The one-tile-per-CTA kernel multicasts the A tile to a cluster of 2 CTAs along N when the column-tile count is even
+// (4 CTAs measured slower: 16 SMs strand).
 template <int S>
 inline int oz_gemm_launch(const OzGemmParams& p, cudaStream_t st) {
   if (oz_persistent(p)) return oz_gemm_p_launch<S>(p, st);
-  switch (oz_cluster_width(p.nnt)) {
-    case 4: return oz_gemm_launch_cn<S, 4>(p, st);
-    case 2: return oz_gemm_launch_cn<S, 2>(p, st);
-    default: return oz_gemm_launch_cn<S, 1>(p, st);
-  }
+  if (p.nnt % 2 == 0) return oz_gemm_launch_cn<S, 2>(p, st);
+  return oz_gemm_launch_cn<S, 1>(p, st);
 }
 
 inline int oz_gemm(int S, const OzGemmParams& p, cudaStream_t st) {

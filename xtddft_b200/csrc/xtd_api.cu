@@ -101,12 +101,7 @@ struct Channel {
 };
 
 constexpr long XC_SPLIT_SMEM_MAX = 200 * 1024;   // shared memory of the split-gradient streaming kernel (MO values of one point)
-// contraction lengths below this stay on the FP64 DMMA GEMM where a kernel offers the choice (XTD_OZ_SHORT_K overrides; tests use 0)
-static int oz_short_k() {
-  const char* e = getenv("XTD_OZ_SHORT_K");
-  return e ? atoi(e) : 100;
-}
-#define OZ_SHORT_K (oz_short_k())
+constexpr int XC_OP_MAX_NVEC = 8;   // batches up to this size take the orbital-range streaming kernel (xc_weight_split_op_kernel)
 constexpr int OZ_XC_KQ = 8192;   // grid points per int32 accumulation group of the backward grid GEMM (8192 * S * 2^14 < 2^31)
 constexpr int NARROW_MAX = 16;   // widest first virtual block that takes the narrow-output exchange pass
 
@@ -139,6 +134,21 @@ struct DiagRec {
   DevBuf D;
 };
 
+// Environment switches that force a path the engine also takes by itself on some inputs (tests use them to reach those paths at
+// small sizes) or that place a profiler range.  Read once, in xtd_create, so every decision of an engine sees the same values.
+struct EnvSwitches {
+  // XTD_CHUNK_AUX / XTD_CHUNK_GRID: upper bounds on the aux / grid chunk of a call (tests force the multi-chunk loops that
+  // BASELINE-size runs take at oracle-sized inputs); the chunk counts of the last call are reported by xtd_last_chunks
+  long max_pc = 0, max_gb = 0;
+  // XTD_OZ_SHORT_K: contraction lengths below this stay on the FP64 DMMA GEMM where a kernel offers the choice (tests use 0)
+  int oz_short_k = 100;
+  int xc_split = -1;          // XTD_XC_SPLIT: 1 / 0 forces the split-gradient / four-component grid form, -1 chooses by cost
+  bool no_narrow = false;     // XTD_NO_NARROW set: block-weighted exchange without the narrow-output pass
+  bool j_stream = false;      // XTD_J_STREAM set: Coulomb blocks on the streaming kernels only
+  // XTD_PROFILE_PHASE=<XTD_T_* id>: cudaProfilerStart/Stop around that phase (ncu --profile-from-start off)
+  int prof_phase = -1;
+};
+
 struct Arena {
   char* base = nullptr;
   size_t cap = 0, used = 0;
@@ -162,7 +172,7 @@ struct xtd_engine {
   cudaStream_t stream = 0;
   GemmContext gemm;
   Arena arena;
-  size_t split_ws_bytes = 0;
+  EnvSwitches env;
   // orbitals
   const double* C[2] = {nullptr, nullptr};
   long ldC[2] = {0, 0};
@@ -223,12 +233,6 @@ struct xtd_engine {
   unsigned long long launches0 = 0;
   double flops0 = 0;
   double phase_flops[12] = {0};   // GEMM flops per phase of the last call
-  // XTD_PROFILE_PHASE=<XTD_T_* id>: cudaProfilerStart/Stop around that phase (ncu --profile-from-start off)
-  int prof_phase = -1;
-  // XTD_CHUNK_AUX / XTD_CHUNK_GRID: upper bounds on the aux / grid chunk of a call (tests force the multi-chunk loops that
-  // BASELINE-size runs take at oracle-sized inputs); the chunk counts of the last call are reported by xtd_last_chunks
-  long max_pc = 0, max_gb = 0;
-  bool oz_fuse = true;            // emulated path: half-transform on the INT8 tensor cores too, fused with the slicing (XTD_OZ_FUSE=0: DMMA + slicing pass)
   int oz_slices = 0;              // 0: FP64 DMMA exchange contraction; 3..8: INT8 tensor-core emulation with that many slices
   long last_aux_chunks = 0, last_grid_chunks = 0;
   // Launch-bound calls (small molecules: ~50-100 launches of a few microseconds each) are replayed as CUDA graphs: the
@@ -239,7 +243,7 @@ struct xtd_engine {
     unsigned long long launches; double flops; double phase_flops[12];
   };
   std::vector<GraphRec> graphs;
-  int graph_mode = -1;            // XTD_GRAPH: 0 never, 1 always, unset: when a call issues < 2e10 GEMM flops
+  bool graphs_off = false;        // set when a capture failed: later calls run eagerly
   bool capturing = false;
   cudaStream_t cap_stream = nullptr;   // calls are recorded on this stream (the caller's may be the legacy default stream,
                                        // which cannot be captured) and replayed on the caller's
@@ -265,14 +269,14 @@ struct PhaseTimer {
     }
     slot = h->ev_used++;
     h->evpool[slot].id = id;
-    if (id == h->prof_phase) cudaProfilerStart();
+    if (id == h->env.prof_phase) cudaProfilerStart();
     cudaEventRecord(h->evpool[slot].a, h->stream);
   }
   ~PhaseTimer() {
     h->phase_flops[phase] += h->gemm.flops - f0;
     if (slot == (size_t)-1) return;
     cudaEventRecord(h->evpool[slot].b, h->stream);
-    if (h->evpool[slot].id == h->prof_phase) cudaProfilerStop();
+    if (h->evpool[slot].id == h->env.prof_phase) cudaProfilerStop();
   }
 };
 
@@ -392,7 +396,7 @@ int grid_commit(xtd_engine* h) {
       e.C = c->phiv.p; e.ldc = c->ldphiv; e.c_batch_stride = h->ng * c->ldphiv;
       XTD_TRY(gemm(h->gemm, e, s));
       bool split_oz = false;
-      if (h->oz_slices > 0 && h->nvar_eff == 4 && !h->tau && !(getenv("XTD_XC_SPLIT") && atoi(getenv("XTD_XC_SPLIT")) == 0)) {
+      if (h->oz_slices > 0 && h->nvar_eff == 4 && !h->tau && h->env.xc_split != 0) {
         int no2[2] = {0, 0}, nv2[2] = {0, 0};
         for (size_t k = 0; k < h->ch.size(); ++k) { no2[k] = h->ch[k]->no; nv2[k] = h->ch[k]->nv; }
         split_oz = xc_split_smem_doubles((int)h->ch.size(), no2, nv2) * 8 <= XC_SPLIT_SMEM_MAX;
@@ -414,13 +418,13 @@ int grid_commit(xtd_engine* h) {
           // ... and of the value component of phi (occupied side of the split-gradient form)
           c->ozOF.set((int)h->ng, OZ_BM, c->no);
           c->ozOB.set(c->no, OZ_BM, OZ_XC_KQ);
-          if (c->no >= OZ_SHORT_K) {
+          if (c->no >= h->env.oz_short_k) {
             XTD_CUDA(cudaMalloc((void**)&c->phiF, c->ozOF.slice_bytes(1, S)));
             XTD_CUDA(cudaMalloc((void**)&c->phiFs, c->ozOF.scale_doubles(1, 1) * 8));
           }
           XTD_CUDA(cudaMalloc((void**)&c->phiB, c->ozOB.slice_bytes(nqg, S)));
           XTD_CUDA(cudaMalloc((void**)&c->phiBs, c->ozOB.scale_doubles(nqg, 1) * 8));
-          if (c->no >= OZ_SHORT_K) XTD_TRY(oz_slice(S, c->phiF, c->phiFs, c->ozOF, c->phi.p, c->ldphi, 0, 1, 1, s));
+          if (c->no >= h->env.oz_short_k) XTD_TRY(oz_slice(S, c->phiF, c->phiFs, c->ozOF, c->phi.p, c->ldphi, 0, 1, 1, s));
           XTD_TRY(oz_slice(S, c->phiB, c->phiBs, c->ozOB, c->phi.p, c->ldphi, (long)OZ_XC_KQ * c->ldphi, (int)nqg, 1, s, true, h->ng));
         }
         XTD_CUDA(cudaStreamSynchronize(s));
@@ -488,11 +492,14 @@ int xtd_create(xtd_handle* out, int nao, long workspace_bytes) {
   cudaEventCreate(&h->ev_total[0]);
   cudaEventCreate(&h->ev_total[1]);
   h->ev_ok = true;
-  if (const char* e = getenv("XTD_PROFILE_PHASE")) h->prof_phase = atoi(e);
-  if (const char* e = getenv("XTD_GRAPH")) h->graph_mode = atoi(e);
-  if (const char* e = getenv("XTD_OZ_FUSE")) h->oz_fuse = atoi(e) != 0;
-  if (const char* e = getenv("XTD_CHUNK_AUX")) h->max_pc = atol(e);
-  if (const char* e = getenv("XTD_CHUNK_GRID")) h->max_gb = atol(e);
+  EnvSwitches& env = h->env;
+  if (const char* e = getenv("XTD_CHUNK_AUX")) env.max_pc = atol(e);
+  if (const char* e = getenv("XTD_CHUNK_GRID")) env.max_gb = atol(e);
+  if (const char* e = getenv("XTD_OZ_SHORT_K")) env.oz_short_k = atoi(e);
+  if (const char* e = getenv("XTD_XC_SPLIT")) env.xc_split = atoi(e) != 0;
+  env.no_narrow = getenv("XTD_NO_NARROW") != nullptr;
+  env.j_stream = getenv("XTD_J_STREAM") != nullptr;
+  if (const char* e = getenv("XTD_PROFILE_PHASE")) env.prof_phase = atoi(e);
   *out = h;
   return XTD_OK;
 }
@@ -731,7 +738,7 @@ int xtd_df_begin(xtd_handle h, int tensor, long naux_local) {
       for (const KTermRec& k : h->kterms)
         if (k.tensor == tensor && h->ch[k.ch] == c) (k.uniform ? n_uni : n_blk)++;
       if (n_blk == 0) c->use_oz[tensor] = n_uni > 0;
-      else if (n_uni == 0 && !(getenv("XTD_OZ_BLOCKED") && atoi(getenv("XTD_OZ_BLOCKED")) == 0)) {
+      else if (n_uni == 0) {
         if (c->v_blocks.size() == 1) c->use_oz[tensor] = true;
         else if (c->need_narrow[tensor]) { c->use_oz[tensor] = true; c->oz_col0[tensor] = c->v_blocks[1].first; }
       }
@@ -1083,7 +1090,7 @@ int xtd_finalize(xtd_handle h, int max_nvec) {
   // small problems: the local GEMM and diagonal terms become one launch
   long max_elems = 0;
   for (auto* c : h->ch) max_elems = std::max<long>(max_elems, (long)c->no * c->nv);
-  h->small_local = max_elems <= 16384 && !(getenv("XTD_LOCAL_BATCH") && atoi(getenv("XTD_LOCAL_BATCH")) == 0);
+  h->small_local = max_elems <= 16384;
   if (h->small_local && (!h->lgemms.empty() || !h->diags.empty())) {
     std::vector<LocalTermDev> lt, ld;
     for (auto* l : h->lgemms) {
@@ -1173,10 +1180,8 @@ static int launch_xc_split(const XcArgs2& a, cudaStream_t s) {
     XTD_CUDA(cudaFuncSetAttribute(xc_weight_split_kernel<XC_KIND_MCOL, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)XC_SPLIT_SMEM_MAX));
     attr_set = true;
   }
-  // few trial vectors: the warps of a CTA share the point by orbital range (xc_weight_split_op_kernel); XTD_XC_OP_MAX_NVEC moves
-  // the switch-over (0: never)
-  static int op_max = getenv("XTD_XC_OP_MAX_NVEC") ? atoi(getenv("XTD_XC_OP_MAX_NVEC")) : 8;
-  if (a.nvec <= op_max) {
+  // few trial vectors: the warps of a CTA share the point by orbital range (xc_weight_split_op_kernel)
+  if (a.nvec <= XC_OP_MAX_NVEC) {
     constexpr int NRK = (KIND == XC_KIND_UKS ? 2 : 1) * 4;
     static bool op_attr_dev[64] = {false};
     bool& op_set = op_attr_dev[dev & 63];
@@ -1214,7 +1219,7 @@ static bool xc_use_split(const xtd_engine* h, int nvec) {
     for (size_t c = 0; c < h->ch.size(); ++c) { no[c] = h->ch[c]->no; nv[c] = h->ch[c]->nv; }
     if (xc_split_smem_doubles((int)h->ch.size(), no, nv) * 8 > XC_SPLIT_SMEM_MAX) return false;   // MO values of a point must fit shared memory
   }
-  if (const char* e = getenv("XTD_XC_SPLIT")) return atoi(e) != 0;
+  if (h->env.xc_split >= 0) return h->env.xc_split != 0;
   auto tile = [](long n) { return (double)(cdiv(n, 128) * 128); };
   double four = 0.0, split = 0.0;
   for (auto* c : h->ch) {
@@ -1249,7 +1254,7 @@ static int run_xc_emulated(xtd_engine* h, int nvec) {
   XTD_REQUIRE(h->scratch_doubles > fixed + per_g * OZ_XC_KQ, XTD_ERR_NOMEM, "workspace too small for one block of the emulated grid path");
   long GB = (long)((h->scratch_doubles - fixed) / per_g);
   GB = std::min<long>(GB, 1 << 16);
-  if (h->max_gb > 0) GB = std::min<long>(GB, std::max<long>(h->max_gb, OZ_XC_KQ));
+  if (h->env.max_gb > 0) GB = std::min<long>(GB, std::max<long>(h->env.max_gb, OZ_XC_KQ));
   GB = GB / OZ_XC_KQ * OZ_XC_KQ;
   h->last_grid_chunks = cdiv(h->ng, GB);
   // carve the scratch region
@@ -1358,7 +1363,7 @@ static int run_xc_split_emulated(xtd_engine* h, int nvec) {
   XTD_REQUIRE(h->scratch_doubles > fixed + per_g * (OZ_XC_KQ + 128), XTD_ERR_NOMEM, "workspace too small for one block of the emulated grid path");
   long GB = (long)((h->scratch_doubles - fixed) / per_g) - 128;
   GB = std::min<long>(GB, 1 << 16);
-  if (h->max_gb > 0) GB = std::min<long>(GB, std::max<long>(h->max_gb, OZ_XC_KQ));
+  if (h->env.max_gb > 0) GB = std::min<long>(GB, std::max<long>(h->env.max_gb, OZ_XC_KQ));
   GB = GB / OZ_XC_KQ * OZ_XC_KQ;
   h->last_grid_chunks = cdiv(h->ng, GB);
   double* cur = h->scratch;
@@ -1385,7 +1390,7 @@ static int run_xc_split_emulated(xtd_engine* h, int nvec) {
     for (int c = 0; c < nch; ++c) {
       Channel* ch = h->ch[c];
       XTD_TRY(oz_slice(S, zS[c], zsc[c], shZ[c], h->Z[c], ch->ldz, 0, 1, 1, s));
-      if (ch->no >= OZ_SHORT_K) XTD_TRY(oz_slice(S, ztS[c], ztsc[c], shZt[c], h->ZT[c], ch->ldzt, (long)ch->nv * ch->ldzt, nvec, 1, s));
+      if (ch->no >= h->env.oz_short_k) XTD_TRY(oz_slice(S, ztS[c], ztsc[c], shZt[c], h->ZT[c], ch->ldzt, (long)ch->nv * ch->ldzt, nvec, 1, s));
     }
   }
   for (long g0 = 0; g0 < h->ng; g0 += GB) {
@@ -1404,7 +1409,7 @@ static int run_xc_split_emulated(xtd_engine* h, int nvec) {
         p.Mpad = (int)mpad_g; p.Npad = shZ[c].rows_pad; p.splits = 1; p.W = Y[c]; p.alpha = 1.0;
         XTD_TRY(oz_gemm(S, p, s));
         h->gemm.flops += 2.0 * gb * (double)(nvec * ch->no) * ch->nv;
-        if (ch->no < OZ_SHORT_K) {
+        if (ch->no < h->env.oz_short_k) {
           // F2 has the occupied count as its contraction length: a few k-steps per tile, where the INT8 kernel is all epilogue
           // (measured at no = 137: 7.4 ms per 40 960-point chunk against 5.4 ms on the DMMA GEMM) -- keep it on FP64 DMMA
           GemmDesc e;
@@ -1513,7 +1518,7 @@ static int run_xc(xtd_engine* h, int nvec) {
   }
   long GB = (long)(h->scratch_doubles / per_g);
   GB = std::min<long>(GB, 1 << 16);
-  if (h->max_gb > 0) GB = std::min<long>(GB, std::max<long>(h->max_gb, 128));
+  if (h->env.max_gb > 0) GB = std::min<long>(GB, std::max<long>(h->env.max_gb, 128));
   GB = (GB / 128) * 128;
   XTD_REQUIRE(GB >= 128, XTD_ERR_NOMEM, "workspace too small for a 128-point grid chunk");
   h->last_grid_chunks = cdiv(h->ng, GB);
@@ -1622,15 +1627,14 @@ static int run_xc(xtd_engine* h, int nvec) {
   return XTD_OK;
 }
 
-// Uniform-weight exchange term with the contraction over (P, b) emulated on the INT8 tensor cores:
-//   K1 (DMMA)   U[P][(i,x)][b] = sum_j Loo[(P,i)][j] zt[x][b][j]            as in run_k
-//   slice       U -> S int8 digit planes + one power-of-two scale per (row, group of aux functions)
+// Uniform-weight exchange term with both contractions on the INT8 tensor cores:
+//   K1 (oz_k1_kernel)   U[P][(i,x)][b] = sum_j Loo[(P,i)][j] zt[x][b][j]; U never exists in fp64: the epilogue writes its S int8 digit
+//                       planes (the A operand of K2) directly, under an a-priori power-of-two scale per (row, group of aux functions)
 //   K2 (tcgen05.mma kind::i8, TMEM)   SIG[x][i][a] += w sum_P sum_b U[P][(i,x)][b] Lvv[P][a][b]   against the int8 planes of Lvv
-// ... with the half-transform fused (oz_k1_kernel): U never exists in fp64; the A planes of the contraction are written directly.
 // Block-weighted terms (XSF Delta A): the wide second virtual block [col0, nv) is emulated -- one half-transform per occupied
 // row block ib with the trial vectors scaled by w(ib, 1, :, :), each filling its rows of the A planes, then ONE contraction
 // against the planes of Lvv[col0:, :]; the narrow first block was done by the DMMA narrow pass of run_k.
-static int run_k_fused(xtd_engine* h, const KTermRec& k, int nvec) {
+static int run_k_emulated(xtd_engine* h, const KTermRec& k, int nvec) {
   cudaStream_t s = h->stream;
   Channel* ch = h->ch[k.ch];
   const long naux = h->naux[k.tensor];
@@ -1673,7 +1677,7 @@ static int run_k_fused(xtd_engine* h, const KTermRec& k, int nvec) {
   long pc = (long)((h->scratch_doubles - w_doubles - zt_doubles - 4096) / per_p);
   pc = std::min<long>(pc, naux);
   if (pc > 32768) pc = 32768;
-  if (h->max_pc > 0) pc = std::min<long>(pc, h->max_pc);
+  if (h->env.max_pc > 0) pc = std::min<long>(pc, h->env.max_pc);
   if (pc < naux) pc = std::max<long>(pc / G * G, G);
   h->last_aux_chunks = std::max<long>(h->last_aux_chunks, cdiv(naux, pc));
   double* cur = h->scratch;
@@ -1748,74 +1752,6 @@ static int run_k_fused(xtd_engine* h, const KTermRec& k, int nvec) {
   return XTD_OK;
 }
 
-static int run_k_emulated(xtd_engine* h, const KTermRec& k, int nvec) {
-  if (h->oz_fuse || !k.uniform) return run_k_fused(h, k, nvec);
-  cudaStream_t s = h->stream;
-  Channel* ch = h->ch[k.ch];
-  const long naux = h->naux[k.tensor];
-  const int S = h->oz_slices, G = ch->oz_group;
-  OzShape shA;
-  shA.set(nvec * ch->no, OZ_BM, ch->nv);
-  const OzShape& shB = ch->ozB;
-  const int tiles = shA.nrt * shB.nrt;
-  // scratch: W [splits][Mpad][Npad] | per aux function: U fp64 + int8 planes (+ scales per group)
-  int splits_max = std::min<long>(64, std::max<long>(1, cdiv(naux, G)));
-  size_t w_doubles = (size_t)splits_max * shA.rows_pad * shB.rows_pad;
-  while (splits_max > 1 && w_doubles * 4 > h->scratch_doubles) { splits_max /= 2; w_doubles = (size_t)splits_max * shA.rows_pad * shB.rows_pad; }
-  const size_t u_per_p = (size_t)nvec * ch->no * ch->ldz;
-  const size_t a_per_p = shA.slice_bytes(1, S) / 8;
-  const size_t per_p = u_per_p + a_per_p + (size_t)cdiv(shA.rows_pad, G) + 1;
-  XTD_REQUIRE(h->scratch_doubles > w_doubles + (size_t)G * per_p + 4096, XTD_ERR_NOMEM,
-              "workspace too small for one group of the emulated exchange contraction");
-  long pc = (long)((h->scratch_doubles - w_doubles - 4096) / per_p);
-  pc = std::min<long>(pc, naux);
-  if ((long)pc * nvec > 65535) pc = 65535 / nvec;
-  if (pc > 32768) pc = 32768;
-  if (h->max_pc > 0) pc = std::min<long>(pc, h->max_pc);
-  if (pc < naux) pc = std::max<long>(pc / G * G, G);
-  h->last_aux_chunks = std::max<long>(h->last_aux_chunks, cdiv(naux, pc));
-  double* W = h->scratch;
-  double* U = W + ((w_doubles + 31) & ~(size_t)31);
-  int8_t* As = reinterpret_cast<int8_t*>(U + (((size_t)pc * u_per_p + 31) & ~(size_t)31));
-  double* sa = reinterpret_cast<double*>(As) + (((size_t)pc * a_per_p + 31) & ~(size_t)31);
-  const double* Loo = ch->Loo[k.tensor].p;
-  for (long P0 = 0; P0 < naux; P0 += pc) {
-    const int pn = (int)std::min<long>(pc, naux - P0);
-    {
-      PhaseTimer t(h, XTD_T_K1);
-      GemmDesc d;
-      d.A = view2d(Loo + P0 * ch->no * ch->ldoo, ch->ldoo, pn * ch->no, ch->no);
-      d.B = view3d(h->ZT[k.ch], ch->ldzt, (long)ch->nv * ch->ldzt, nvec, ch->nv, ch->no);
-      d.M = pn * ch->no; d.N = ch->nv; d.K = ch->no;
-      d.batches = nvec; d.z_div = 1; d.a_hi = 0; d.b_hi = 1;
-      d.C = U; d.ldc = (long)nvec * ch->ldz; d.c_batch_stride = ch->ldz;
-      XTD_TRY(gemm(h->gemm, d, s));
-    }
-    {
-      PhaseTimer t(h, XTD_T_K2_SLICE);
-      XTD_TRY(oz_slice(S, As, sa, shA, U, ch->ldz, (long)u_per_p, pn, G, s));
-    }
-    {
-      PhaseTimer t(h, XTD_T_K2);
-      OzGemmParams p;
-      p.A = As; p.B = ch->LvvS[k.tensor]; p.sa = sa; p.sb = ch->LvvScale[k.tensor];
-      p.nmt = shA.nrt; p.nnt = shB.nrt; p.nkb = shA.nkb; p.nq = pn; p.group = G; p.b_q0 = (int)P0;
-      p.Mpad = shA.rows_pad; p.Npad = shB.rows_pad;
-      p.splits = std::min(splits_max, oz_choose_splits(tiles, (int)cdiv(pn, G), h->gemm.num_sms));
-      p.W = W; p.alpha = k.w[0][0][0][0];
-      XTD_TRY(oz_gemm(S, p, s));
-      const int M = nvec * ch->no, N = ch->nv;
-      const long nblk = cdiv((long)M * N, 256);
-      reduce_splits_kernel<<<dim3((unsigned)(nblk > 4096 ? 4096 : nblk), 1), 256, 0, s>>>(
-          h->SIG + h->sig_base[k.ch], ch->ldz, 0, W, shB.rows_pad, 0, (long)shA.rows_pad * shB.rows_pad, p.splits, M, N, 1, nvec, ch->ldz,
-          (long)ch->no * ch->ldz);
-      LAUNCH_CHECK();
-      h->gemm.flops += 2.0 * M * N * (double)ch->nv * pn;      // FP64-equivalent flops of the contraction
-    }
-  }
-  return XTD_OK;
-}
-
 static int run_k(xtd_engine* h, int nvec) {
   cudaStream_t s = h->stream;
   for (const KTermRec& k : h->kterms) {
@@ -1834,7 +1770,7 @@ static int run_k(xtd_engine* h, int nvec) {
     XTD_REQUIRE(pc >= 1, XTD_ERR_NOMEM, "workspace too small for the exchange intermediate of one aux function");
     pc = std::min<long>(pc, naux);
     if ((long)pc * nvec > 65535) pc = 65535 / nvec;
-    if (h->max_pc > 0) pc = std::min<long>(pc, h->max_pc);
+    if (h->env.max_pc > 0) pc = std::min<long>(pc, h->env.max_pc);
     h->last_aux_chunks = std::max<long>(h->last_aux_chunks, cdiv(naux, pc));
     double* U = h->scratch;
     std::vector<std::pair<int, int>> iblks, ablks;
@@ -1858,7 +1794,7 @@ static int run_k(xtd_engine* h, int nvec) {
     const size_t zs_doubles = (size_t)nvec * ch->no * ch->ldz;
     const int wmax = std::max(v2off, ch->tail_w);
     if (!k.uniform && ch->need_narrow[k.tensor] && ablks.size() == 2 &&
-        zs_doubles + (size_t)nvec * naux * wmax * ldj <= h->scratch_doubles && (long)nvec * naux < (1L << 30) && !getenv("XTD_NO_NARROW")) {
+        zs_doubles + (size_t)nvec * naux * wmax * ldj <= h->scratch_doubles && (long)nvec * naux < (1L << 30) && !h->env.no_narrow) {
       double* Zs = h->scratch;
       double* R = h->scratch + zs_doubles;
       // (rows of Lvv gathered per aux function, first output column, width, column block whose weights apply)
@@ -1988,7 +1924,7 @@ static int run_kt(xtd_engine* h, int nvec) {
     long pc = (long)(h->scratch_doubles / per_p);
     XTD_REQUIRE(pc >= 1, XTD_ERR_NOMEM, "workspace too small for the transposed-exchange intermediate of one aux function");
     pc = std::min<long>(pc, naux);
-    if (h->max_pc > 0) pc = std::min<long>(pc, h->max_pc);
+    if (h->env.max_pc > 0) pc = std::min<long>(pc, h->env.max_pc);
     h->last_aux_chunks = std::max<long>(h->last_aux_chunks, cdiv(naux, pc));
     double* W = h->scratch;
     for (long P0 = 0; P0 < naux; P0 += pc) {
@@ -2031,9 +1967,8 @@ static int run_j(xtd_engine* h, int nvec) {
   // A block that spans the full width of its channel is contiguous in (i, a) for every aux function and vector, so both
   // Coulomb steps are plain GEMMs over the flattened pair index (the streaming kernels re-read all trial vectors from L2
   // once per aux function); sub-blocks (XSF Delta A) keep the streaming kernels.
-  const bool no_gemm = getenv("XTD_J_STREAM") != nullptr;
   auto flat = [&](const JBlockRec* j) {      // (the flattened pair index is the N dimension of the second GEMM: grid.y limit)
-    return !no_gemm && j->c0 == 0 && j->ld == h->ch[j->ch]->ldz && (long)j->nr * j->ld <= 65535L * 128;
+    return !h->env.j_stream && j->c0 == 0 && j->ld == h->ch[j->ch]->ldz && (long)j->nr * j->ld <= 65535L * 128;
   };
   for (int b = 0; b < njb; ++b) {
     JBlockRec* j = h->jblocks[b];
@@ -2162,7 +2097,7 @@ int xtd_sigma_partial(xtd_handle h, int nvec, const double* z_dev) {
   h->ev_used = 0;
   for (int i = 0; i < 12; ++i) h->phase_flops[i] = 0.0;
   h->last_aux_chunks = h->last_grid_chunks = 0;
-  if (h->prof_phase == XTD_T_TOTAL && !h->capturing) cudaProfilerStart();
+  if (h->env.prof_phase == XTD_T_TOTAL && !h->capturing) cudaProfilerStart();
   if (h->ev_ok && !h->capturing) cudaEventRecord(h->ev_total[0], s);
   XTD_TRY(setup_call_buffers(h, nvec));
   long base[2], total;
@@ -2227,7 +2162,7 @@ int xtd_sigma_finish(xtd_handle h, int nvec, double* hz_dev) {
     LAUNCH_CHECK();
   }
   if (h->ev_ok && !h->capturing) cudaEventRecord(h->ev_total[1], s);
-  if (h->prof_phase == XTD_T_TOTAL && !h->capturing) cudaProfilerStop();
+  if (h->env.prof_phase == XTD_T_TOTAL && !h->capturing) cudaProfilerStop();
   return XTD_OK;
 }
 
@@ -2249,16 +2184,16 @@ static int launch_graph(xtd_engine* h, const xtd_engine::GraphRec& g) {
 
 int xtd_sigma(xtd_handle h, int nvec, const double* z_dev, double* hz_dev) {
   XTD_REQUIRE(h && h->finalized, XTD_ERR_STATE, "xtd_sigma before xtd_finalize");
-  if (h->graph_mode == 0 || h->prof_phase >= 0) return sigma_eager(h, nvec, z_dev, hz_dev);
+  if (h->graphs_off || h->env.prof_phase >= 0) return sigma_eager(h, nvec, z_dev, hz_dev);
   for (const auto& g : h->graphs)
     if (g.nvec == nvec && g.z == z_dev && g.hz == hz_dev) {
       g_launch_count += g.launches;                  // the kernels of the recorded call run again
       h->gemm.flops += g.flops;
       return launch_graph(h, g);
     }
-  // second call with the same arguments, and the first one was launch-bound (or graphs are forced): capture it
+  // second call with the same arguments, and the first one was launch-bound: capture it
   const bool repeat = h->last_eager_nvec == nvec && h->last_eager_z == z_dev && h->last_eager_hz == hz_dev;
-  if (repeat && (h->graph_mode == 1 || h->last_eager_flops < 2e10) && h->graphs.size() < 64) {
+  if (repeat && h->last_eager_flops < 2e10 && h->graphs.size() < 64) {
     if (!h->cap_stream && cudaStreamCreateWithFlags(&h->cap_stream, cudaStreamNonBlocking) != cudaSuccess) h->cap_stream = nullptr;
     cudaStream_t s = h->cap_stream, user_stream = h->stream;
     const unsigned long long l0 = g_launch_count;
@@ -2284,10 +2219,10 @@ int xtd_sigma(xtd_handle h, int nvec, const double* z_dev, double* hz_dev) {
       if (graph) cudaGraphDestroy(graph);
       cudaGetLastError();
       g_launch_count = l0; h->gemm.flops = f0;
-      h->graph_mode = 0;
+      h->graphs_off = true;
     } else {
       cudaGetLastError();
-      h->graph_mode = 0;
+      h->graphs_off = true;
     }
   }
   const double f0 = h->gemm.flops;
