@@ -36,10 +36,45 @@ constexpr int OZ_K1_THREADS = 320;     // producer + MMA issuer + 8 epilogue war
 
 __device__ __forceinline__ uint32_t oz_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
+// ---- packed rows ----------------------------------------------------------------------------------------------------------
+// The A operand of the fused half-transform packs the rows (P, i) of G aux functions into one q-slice, so a 128-row tile spans aux
+// functions instead of padding every aux function's `no` rows to a multiple of 128.  Rows are ordered (occupied row block, P, i)
+// with the row blocks [0, o2) and [o2, no), so a pass over one row block of a block-weighted term reads a contiguous row range:
+//   r < G o2:  P = r / o2,  i = r % o2;     else  r' = r - G o2,  P = r' / (no - o2),  i = o2 + r' % (no - o2)     (r' < G (no - o2))
+__host__ __device__ __forceinline__ bool oz_unpack_row(int r, int G, int o2, int no, int& P, int& i) {
+  if (r < G * o2) {
+    P = r / o2;
+    i = r - P * o2;
+    return true;
+  }
+  const int n1 = no - o2, r1 = r - G * o2;
+  if (r1 >= G * n1) return false;
+  P = r1 / n1;
+  i = o2 + (r1 - P * n1);
+  return true;
+}
+// first and one-past-last packed row of a pass over the orbitals [i_lo, i_hi) (exact when the range is a row block or all rows)
+inline int oz_packed_row_lo(int i_lo, int G, int o2) { return i_lo >= o2 ? G * o2 : 0; }
+inline int oz_packed_row_hi(int i_hi, int G, int o2, int no) { return i_hi <= o2 ? G * o2 : G * no; }
+
+// Source of a packed-row slicing (OzRowPack::G > 0): row r of q-slice q is aux function q G + P (valid while < np), orbital i, at
+// X[q * sq + P * sp + i * ld].  G = 0: plain rows.
+struct OzRowPack {
+  int G = 0, o2 = 0, no = 0, np = 0;
+  long sp = 0;
+};
+// offset of row `row` of q-slice q relative to X + q * sq, or -1 for a row with no source (zero)
+__device__ __forceinline__ long oz_src_row(const OzRowPack& pk, int q, int row, int rows, long ld) {
+  if (pk.G == 0) return row < rows ? (long)row * ld : -1L;
+  int P, i;
+  if (!oz_unpack_row(row, pk.G, pk.o2, pk.no, P, i) || q * pk.G + P >= pk.np) return -1L;
+  return (long)P * pk.sp + (long)i * ld;
+}
+
 // ---- slicing ------------------------------------------------------------------------------------------------------------
-// Source element (q, row, k):  X[q * sq + row * ld + k]   (K-contiguous rows), or for a TRANSPOSED source (the contraction
-// index is the row index of the array, e.g. grid points)  X[q * sq + k * ld + row].  Only k with q * K + k < k_valid are read
-// (a ragged last q-slice); everything else is zero.
+// Source element (q, row, k):  X[q * sq + row * ld + k]   (K-contiguous rows; X[q * sq + oz_src_row(..) + k] with packed rows),
+// or for a TRANSPOSED source (the contraction index is the row index of the array, e.g. grid points)  X[q * sq + k * ld + row].
+// Only k with q * K + k < k_valid are read (a ragged last q-slice); everything else is zero.
 __device__ __forceinline__ double oz_scale_of(double m) {
   if (!(m > 1e-280 && m < 1e280)) return 0.0;
   int e;
@@ -71,16 +106,16 @@ __global__ void oz_rowmax_t_kernel(double* __restrict__ scale, int rows_pad, con
 
 // scale[g][row] = 2^(e - 6) with max |x| over the row's group < 2^e (0 for an all-zero / padding row)
 __global__ void oz_rowmax_kernel(double* __restrict__ scale, int rows_pad, const double* __restrict__ X, long ld, long sq, int rows, int K,
-                                 int nq, int group, long k_valid) {
+                                 int nq, int group, long k_valid, const OzRowPack pack) {
   const int row = blockIdx.x, g = blockIdx.y;
   double m = 0.0;
-  if (row < rows) {
-    const int q1 = min(nq, (g + 1) * group);
-    for (int q = g * group; q < q1; ++q) {
-      const int kmax = (int)min((long)K, k_valid - (long)q * K);
-      const double* x = X + (long)q * sq + (long)row * ld;
-      for (int k = threadIdx.x; k < kmax; k += blockDim.x) m = fmax(m, fabs(x[k]));
-    }
+  const int q1 = min(nq, (g + 1) * group);
+  for (int q = g * group; q < q1; ++q) {
+    const long off = oz_src_row(pack, q, row, rows, ld);
+    if (off < 0) continue;
+    const int kmax = (int)min((long)K, k_valid - (long)q * K);
+    const double* x = X + (long)q * sq + off;
+    for (int k = threadIdx.x; k < kmax; k += blockDim.x) m = fmax(m, fabs(x[k]));
   }
   __shared__ double red[8];
   for (int o = 16; o > 0; o >>= 1) m = fmax(m, __shfl_xor_sync(0xffffffffu, m, o));
@@ -159,7 +194,7 @@ __device__ __forceinline__ void oz_digits16(const double (&t)[16], uint32_t (&pk
 template <int S, bool TRANS>
 __global__ void __launch_bounds__(128) oz_slice_kernel(int8_t* __restrict__ out, const double* __restrict__ scale, int rows_pad,
                                                        const double* __restrict__ X, long ld, long sq, int rows, int K, int RT, int nkb,
-                                                       int group, int stacked, long k_valid) {
+                                                       int group, int stacked, long k_valid, const OzRowPack pack) {
   const int c2 = blockIdx.x, q = blockIdx.z;
   const int row = blockIdx.y * 128 + threadIdx.x;
   const int rt = row / RT, r = row - rt * RT, nrt = rows_pad / RT;
@@ -168,7 +203,8 @@ __global__ void __launch_bounds__(128) oz_slice_kernel(int8_t* __restrict__ out,
 #pragma unroll
   for (int k = 0; k < 16; ++k) x[k] = 0.0;
   double sc = 0.0;
-  if (row < rows) {
+  const long off = TRANS ? (row < rows ? 0L : -1L) : oz_src_row(pack, q, row, rows, ld);
+  if (off >= 0) {
     sc = scale[(long)(q / group) * rows_pad + row];
     const int kmax = (int)min((long)K, k_valid - (long)q * K);      // valid k of this q-slice
     if (TRANS) {
@@ -177,7 +213,7 @@ __global__ void __launch_bounds__(128) oz_slice_kernel(int8_t* __restrict__ out,
       for (int k = 0; k < 16; ++k)
         if (k0 + k < kmax) x[k] = src[(long)k * ld];
     } else {
-      const double* src = X + (long)q * sq + (long)row * ld + k0;
+      const double* src = X + (long)q * sq + off + k0;
       if (k0 + 16 <= kmax) {
 #pragma unroll
         for (int k = 0; k < 16; k += 2) {
@@ -605,28 +641,55 @@ __global__ void __launch_bounds__(OZ_K1_THREADS, 1) oz_gemm_p_kernel(const OzGem
 //
 //   U[P][(x,i)][b] = sum_j Loo[P][i][j] zt[x][b][j]            (K = occupied count: a few k-steps per tile)
 //
-// A = int8 planes of Loo (static, one q-slice per aux function, rows padded to 128 per aux function), B = planes of zt (per
-// call, one q-slice per trial vector).  A persistent CTA walks tiles (P, 128 rows i, x, 64 columns b); its epilogue recombines the
-// levels in fp64, and instead of storing fp64 U it cuts the value into the digit planes of row m = x no + i of the NEXT GEMM's A
-// operand, under an a-priori power-of-two scale per (row, group) -- the Cauchy-Schwarz bound |U| <= |Loo[P,i,:]| |z[x,:,b]| --
-// so the 190 GB fp64 intermediate of a config-5 step (written once, read twice by the slicing pass) never exists.
+// A = int8 planes of Loo (static; one q-slice per group of `group` aux functions, whose rows (P, i) are packed as oz_unpack_row
+// describes and padded to 128 per group), B = planes of zt (per call, one q-slice per trial vector).  A persistent CTA walks tiles
+// (group, 128 packed rows, x, 64 columns b); its epilogue recombines the levels in fp64, and instead of storing fp64 U it cuts the
+// value into the digit planes of row m = x no + i of the NEXT GEMM's A operand, under an a-priori power-of-two scale per (row, group)
+// -- the Cauchy-Schwarz bound |U| <= |Loo[P,i,:]| |z[x,:,b]| -- so the 190 GB fp64 intermediate of a config-5 step (written once, read
+// twice by the slicing pass) never exists.
+// The CTAs run in clusters of 2 that take the same row tile and two consecutive (x, b tile) items: each loads half of every A stage
+// and multicasts it to both, so the L2 -> SM traffic per tile drops from A + B to A / 2 + B (the kernel needs about as many bytes per
+// clock from L2 as the L2 delivers to all SMs when every CTA loads its own A).
 struct OzK1Params {
-  const int8_t* A;    // [np][nit][nkb1][S][128 x 32]
+  const int8_t* A;    // [groups][ntg][nkb1][S][128 x 32]
   const int8_t* B;    // [nvec][nbt][nkb1][2][S][64 x 16]
-  const double* sa;   // [np][nit * 128]      row scales of the Loo planes
+  const double* sa;   // [groups][ntg * 128]  row scales of the Loo planes (packed rows)
   const double* sb;   // [nvec][nbt * 64]     row scales of the zt planes
   const double* so;   // [groups][Mpad2]      output row scales (2^(e-6), |U| < 2^e guaranteed by the bound)
   int8_t* out;        // [np][nmt2][nkb2][S][128 x 32]
-  int np, nit, nbt, nkb1, nvec, no, group, nmt2, nkb2, Mpad2;
-  int it0, nit_run;   // row tiles [it0, it0 + nit_run) of every aux function are computed ...
-  int i_lo, i_hi;     // ... and only rows i in [i_lo, i_hi) are written (a row block of a block-weighted term)
-  long ntiles;        // np * nit_run * nvec * nbt
+  int np, ntg, nbt, nkb1, nvec, no, o2, group, nmt2, nkb2, Mpad2;
+  int t0, nt_run;     // row tiles [t0, t0 + nt_run) of every group are computed ...
+  int i_lo, i_hi;     // ... and only rows with i in [i_lo, i_hi) are written (a row block of a block-weighted term)
+  long npairs;        // groups * nt_run * cdiv(nvec * nbt, 2): items of a CTA pair
 };
+
+// The item of CTA `crank` in pair item u: group gl, row tile, vector x, column tile bt.  When nvec * nbt is odd the second CTA of the
+// last pair of a row tile repeats its partner's item (it still loads B and its half of A for the partner) and stores nothing.
+struct OzK1Item {
+  int gl, tile, x, bt;
+  bool live;
+};
+__device__ __forceinline__ OzK1Item oz_k1_item(const OzK1Params& p, long u, uint32_t crank) {
+  const long nxb = (long)p.nvec * p.nbt, nxb2 = (nxb + 1) >> 1, per_g = (long)p.nt_run * nxb2;
+  OzK1Item t;
+  t.gl = (int)(u / per_g);
+  const long r0 = u - (long)t.gl * per_g;
+  const int itile = (int)(r0 / nxb2);
+  t.tile = p.t0 + itile;
+  long xb = 2 * (r0 - (long)itile * nxb2) + crank;
+  t.live = xb < nxb;
+  if (!t.live) xb = nxb - 1;
+  t.x = (int)(xb / p.nbt);
+  t.bt = (int)(xb - (long)t.x * p.nbt);
+  return t;
+}
 
 template <int S>
 __global__ void __launch_bounds__(OZ_K1_THREADS, 1) oz_k1_kernel(const OzK1Params p) {
   constexpr int A_SLICE = OZ_BM * OZ_KB, B_SLICE = OZ_BN * OZ_KB;
   constexpr int A_BYTES = S * A_SLICE, B_BYTES = S * B_SLICE, STAGE = A_BYTES + B_BYTES;
+  constexpr int A_HALF = A_BYTES / 2;
+  constexpr uint16_t cmask = 3;
   extern __shared__ __align__(128) uint8_t oz_smem[];
   uint64_t* full = reinterpret_cast<uint64_t*>(oz_smem + OZ_STAGES * STAGE);
   uint64_t* empty = full + OZ_STAGES;
@@ -634,11 +697,13 @@ __global__ void __launch_bounds__(OZ_K1_THREADS, 1) oz_k1_kernel(const OzK1Param
   uint64_t* tmem_empty = tmem_full + 1;
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_empty + 1);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const uint32_t crank = oz_cluster_rank();
+  const long pair0 = blockIdx.x >> 1, npair_ctas = gridDim.x >> 1;
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < OZ_STAGES; ++s) {
       oz_mbar_init(&full[s], 1);
-      oz_mbar_init(&empty[s], 1);
+      oz_mbar_init(&empty[s], 2);           // a stage is rewritten by both CTAs of the pair: both must have drained it
     }
     oz_mbar_init(tmem_full, 1);
     oz_mbar_init(tmem_empty, OZ_K1_THREADS - 64);
@@ -651,28 +716,24 @@ __global__ void __launch_bounds__(OZ_K1_THREADS, 1) oz_k1_kernel(const OzK1Param
   }
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
+  oz_cluster_sync();                        // both CTAs' barriers exist before the first multicast copy / arrive
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tmem_base = *tmem_slot;
-  const long per_p = (long)p.nit_run * p.nvec * p.nbt, per_it = (long)p.nvec * p.nbt;
 
   if (warp == 0) {
     if (lane == 0) {
       long it = 0;
-      for (long t = blockIdx.x; t < p.ntiles; t += gridDim.x) {
-        const int P = (int)(t / per_p);
-        const long r0 = t - (long)P * per_p;
-        const int itile = (int)(r0 / per_it);
-        const long r1 = r0 - (long)itile * per_it;
-        const int x = (int)(r1 / p.nbt), bt = (int)(r1 - (long)x * p.nbt);
-        const int8_t* a = p.A + (((long)P * p.nit + p.it0 + itile) * p.nkb1) * A_BYTES;
-        const int8_t* b = p.B + (((long)x * p.nbt + bt) * p.nkb1) * B_BYTES;
+      for (long u = pair0; u < p.npairs; u += npair_ctas) {
+        const OzK1Item t = oz_k1_item(p, u, crank);
+        const int8_t* a = p.A + (((long)t.gl * p.ntg + t.tile) * p.nkb1) * A_BYTES + crank * A_HALF;
+        const int8_t* b = p.B + (((long)t.x * p.nbt + t.bt) * p.nkb1) * B_BYTES;
         for (int kb = 0; kb < p.nkb1; ++kb, ++it) {
           const int s = (int)(it % OZ_STAGES);
           const uint32_t ph = (uint32_t)((it / OZ_STAGES) & 1);
           oz_mbar_wait(&empty[s], ph ^ 1u);
           oz_mbar_expect_tx(&full[s], STAGE);
           uint8_t* sa = oz_smem + s * STAGE;
-          oz_bulk_load(sa, a + (long)kb * A_BYTES, A_BYTES, &full[s]);
+          oz_bulk_load_mc(sa + crank * A_HALF, a + (long)kb * A_BYTES, A_HALF, &full[s], cmask);
           oz_bulk_load(sa + A_BYTES, b + (long)kb * B_BYTES, B_BYTES, &full[s]);
         }
       }
@@ -682,7 +743,7 @@ __global__ void __launch_bounds__(OZ_K1_THREADS, 1) oz_k1_kernel(const OzK1Param
       constexpr uint32_t idesc0 = (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(OZ_BM >> 4) << 24);
       const uint32_t smem_base = oz_smem_u32(oz_smem);
       long it = 0, n = 0;
-      for (long t = blockIdx.x; t < p.ntiles; t += gridDim.x, ++n) {
+      for (long u = pair0; u < p.npairs; u += npair_ctas, ++n) {
         if (n > 0) oz_mbar_wait(tmem_empty, (uint32_t)((n - 1) & 1));      // the epilogue has drained the previous tile
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         for (int kb = 0; kb < p.nkb1; ++kb, ++it) {
@@ -703,7 +764,7 @@ __global__ void __launch_bounds__(OZ_K1_THREADS, 1) oz_k1_kernel(const OzK1Param
               oz_mma_i8(tmem_base + (uint32_t)((i + j0) * OZ_BN), da, db, idesc, (i > 0) ? 1u : later);
             }
           }
-          oz_commit(&empty[s]);
+          oz_commit_mc(&empty[s], cmask);       // frees the stage in both CTAs (each of them writes half of its A part)
         }
         oz_commit(tmem_full);
       }
@@ -713,20 +774,18 @@ __global__ void __launch_bounds__(OZ_K1_THREADS, 1) oz_k1_kernel(const OzK1Param
     const int quad = warp & 3, half = (warp - 2) >> 2;
     const int row = quad * 32 + lane;
     const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16);
-    const double magic = 6755399441055744.0;
-    const int rowsA = p.nit * OZ_BM, rowsB = p.nbt * OZ_BN;
+    const int rowsA = p.ntg * OZ_BM, rowsB = p.nbt * OZ_BN;
     long n = 0;
-    for (long t = blockIdx.x; t < p.ntiles; t += gridDim.x, ++n) {
-      const int P = (int)(t / per_p);
-      const long r0 = t - (long)P * per_p;
-      const int itile = p.it0 + (int)(r0 / per_it);
-      const long r1 = r0 - (long)(itile - p.it0) * per_it;
-      const int x = (int)(r1 / p.nbt), bt = (int)(r1 - (long)x * p.nbt);
-      const int i = itile * OZ_BM + row;
-      const bool valid = i >= p.i_lo && i < p.i_hi;
+    for (long u = pair0; u < p.npairs; u += npair_ctas, ++n) {
+      const OzK1Item t = oz_k1_item(p, u, crank);
+      const int x = t.x, bt = t.bt;
+      const int pr = t.tile * OZ_BM + row;             // packed row of the group
+      int Pl = 0, i = 0;
+      const bool valid = t.live && oz_unpack_row(pr, p.group, p.o2, p.no, Pl, i) && i >= p.i_lo && i < p.i_hi && t.gl * p.group + Pl < p.np;
+      const int P = t.gl * p.group + Pl;               // aux function of the chunk
       const int m = x * p.no + i;
-      const double sa = valid ? p.sa[(long)P * rowsA + i] : 0.0;
-      const double so = valid ? p.so[(long)(P / p.group) * p.Mpad2 + m] : 0.0;
+      const double sa = valid ? p.sa[(long)t.gl * rowsA + pr] : 0.0;
+      const double so = valid ? p.so[(long)t.gl * p.Mpad2 + m] : 0.0;
       const double inv = so > 0.0 ? __hiloint2double(0x7fe00000 - __double2hiint(so), 0) : 0.0;
       const double f = sa * inv;                       // both powers of two: exact
       const double* sb = p.sb + (long)x * rowsB + bt * OZ_BN;
@@ -752,6 +811,7 @@ __global__ void __launch_bounds__(OZ_K1_THREADS, 1) oz_k1_kernel(const OzK1Param
       }
       asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
       oz_mbar_arrive(tmem_empty);
+      if (!__any_sync(0xffffffffu, valid)) continue;   // no row of this warp is stored (chunk or row-block edge, masked partner)
 #pragma unroll
       for (int cc = 0; cc < HC; cc += 16) {
         const int c0 = half * HC + cc;
@@ -771,6 +831,7 @@ __global__ void __launch_bounds__(OZ_K1_THREADS, 1) oz_k1_kernel(const OzK1Param
   }
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
+  oz_cluster_sync();                        // no CTA leaves while its partner may still multicast into it or arrive on its barriers
   if (warp == 1) {
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
@@ -829,30 +890,48 @@ __global__ void oz_bound_scale_kernel(double* __restrict__ so, int Mpad2, const 
   so[(long)g * Mpad2 + m] = s;
 }
 
+inline size_t oz_gemm_smem(int S) { return (size_t)OZ_STAGES * S * (OZ_BM + OZ_BN) * OZ_KB + 256; }
+
+// one cluster of 2 CTAs per pair of SMs that can hold them, as many as there are pair items
 template <int S>
-inline int oz_k1_launch(const OzK1Params& p, int num_sms, cudaStream_t st) {
+inline int oz_k1_launch(const OzK1Params& p, cudaStream_t st) {
   static bool attr_set[64] = {false};
+  static int max_clusters[64] = {0};
   int dev = 0;
   XTD_CUDA(cudaGetDevice(&dev));
+  cudaLaunchConfig_t cfg = {};
+  cfg.blockDim = dim3(OZ_K1_THREADS);
+  cfg.dynamicSmemBytes = oz_gemm_smem(S);
+  cfg.stream = st;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = 2;
+  attr[0].val.clusterDim.y = 1;
+  attr[0].val.clusterDim.z = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
   if (!attr_set[dev & 63]) {
-    XTD_CUDA(cudaFuncSetAttribute(oz_k1_kernel<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)((size_t)OZ_STAGES * S * (OZ_BM + OZ_BN) * OZ_KB + 256)));
+    XTD_CUDA(cudaFuncSetAttribute(oz_k1_kernel<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)oz_gemm_smem(S)));
+    cfg.gridDim = dim3(2);
+    XTD_CUDA(cudaOccupancyMaxActiveClusters(&max_clusters[dev & 63], oz_k1_kernel<S>, &cfg));
+    XTD_REQUIRE(max_clusters[dev & 63] >= 1, XTD_ERR_CUDA, "oz_k1: no 2-CTA cluster of the fused half-transform fits this device");
     attr_set[dev & 63] = true;
   }
-  const unsigned grid = (unsigned)std::min<long>(p.ntiles, num_sms);
-  oz_k1_kernel<S><<<grid, OZ_K1_THREADS, (size_t)OZ_STAGES * S * (OZ_BM + OZ_BN) * OZ_KB + 256, st>>>(p);
+  cfg.gridDim = dim3((unsigned)(2 * std::min<long>(p.npairs, max_clusters[dev & 63])));
+  XTD_CUDA(cudaLaunchKernelEx(&cfg, oz_k1_kernel<S>, p));
   XTD_COUNT_LAUNCH();
   XTD_CUDA(cudaGetLastError());
   return XTD_OK;
 }
 
-inline int oz_k1(int S, const OzK1Params& p, int num_sms, cudaStream_t st) {
+inline int oz_k1(int S, const OzK1Params& p, cudaStream_t st) {
   switch (S) {
-    case 3: return oz_k1_launch<3>(p, num_sms, st);
-    case 4: return oz_k1_launch<4>(p, num_sms, st);
-    case 5: return oz_k1_launch<5>(p, num_sms, st);
-    case 6: return oz_k1_launch<6>(p, num_sms, st);
-    case 7: return oz_k1_launch<7>(p, num_sms, st);
-    case 8: return oz_k1_launch<8>(p, num_sms, st);
+    case 3: return oz_k1_launch<3>(p, st);
+    case 4: return oz_k1_launch<4>(p, st);
+    case 5: return oz_k1_launch<5>(p, st);
+    case 6: return oz_k1_launch<6>(p, st);
+    case 7: return oz_k1_launch<7>(p, st);
+    case 8: return oz_k1_launch<8>(p, st);
   }
   XTD_SET_ERR("oz_k1: %d slices (3..8)", S);
   return XTD_ERR_ARG;
@@ -871,8 +950,6 @@ struct OzShape {
   size_t scale_doubles(long nq, int group) const { return (size_t)cdiv(nq, group) * rows_pad; }
 };
 
-inline size_t oz_gemm_smem(int S) { return (size_t)OZ_STAGES * S * (OZ_BM + OZ_BN) * OZ_KB + 256; }
-
 // the largest group (q-slices sharing one scale and one int32 accumulation) that cannot overflow: per k a level holds at most
 // S products of magnitude <= 2^14
 inline int oz_max_group(int K, int S) {
@@ -883,7 +960,7 @@ inline int oz_max_group(int K, int S) {
 
 template <int S>
 inline int oz_slice_launch(int8_t* out, double* scale, const OzShape& sh, const double* X, long ld, long sq, int nq, int group,
-                           bool trans, long k_valid, cudaStream_t st) {
+                           bool trans, long k_valid, const OzRowPack& pk, cudaStream_t st) {
   const int ng = (int)cdiv(nq, group);
   const int stacked = sh.RT == OZ_BN ? 1 : 0;
   const dim3 sgrid(2 * sh.nkb, sh.rows_pad / 128, nq);
@@ -891,12 +968,12 @@ inline int oz_slice_launch(int8_t* out, double* scale, const OzShape& sh, const 
     oz_rowmax_t_kernel<<<dim3(sh.rows_pad / 32, ng), dim3(32, 32), 0, st>>>(scale, sh.rows_pad, X, ld, sq, sh.rows, sh.K, nq, group, k_valid);
     XTD_COUNT_LAUNCH();
     XTD_CUDA(cudaGetLastError());
-    oz_slice_kernel<S, true><<<sgrid, 128, 0, st>>>(out, scale, sh.rows_pad, X, ld, sq, sh.rows, sh.K, sh.RT, sh.nkb, group, stacked, k_valid);
+    oz_slice_kernel<S, true><<<sgrid, 128, 0, st>>>(out, scale, sh.rows_pad, X, ld, sq, sh.rows, sh.K, sh.RT, sh.nkb, group, stacked, k_valid, pk);
   } else {
-    oz_rowmax_kernel<<<dim3(sh.rows_pad, ng), 256, 0, st>>>(scale, sh.rows_pad, X, ld, sq, sh.rows, sh.K, nq, group, k_valid);
+    oz_rowmax_kernel<<<dim3(sh.rows_pad, ng), 256, 0, st>>>(scale, sh.rows_pad, X, ld, sq, sh.rows, sh.K, nq, group, k_valid, pk);
     XTD_COUNT_LAUNCH();
     XTD_CUDA(cudaGetLastError());
-    oz_slice_kernel<S, false><<<sgrid, 128, 0, st>>>(out, scale, sh.rows_pad, X, ld, sq, sh.rows, sh.K, sh.RT, sh.nkb, group, stacked, k_valid);
+    oz_slice_kernel<S, false><<<sgrid, 128, 0, st>>>(out, scale, sh.rows_pad, X, ld, sq, sh.rows, sh.K, sh.RT, sh.nkb, group, stacked, k_valid, pk);
   }
   XTD_COUNT_LAUNCH();
   XTD_CUDA(cudaGetLastError());
@@ -905,19 +982,21 @@ inline int oz_slice_launch(int8_t* out, double* scale, const OzShape& sh, const 
 
 // trans: the contraction index is the ROW index of the source array (element (row, k) at X[q sq + k ld + row]).
 // k_valid: number of valid contraction indices over all q-slices together (q K + k < k_valid), <= 0 = all.
+// pk: packed rows (K-contiguous sources only); the default reads plain rows.
 inline int oz_slice(int S, int8_t* out, double* scale, const OzShape& sh, const double* X, long ld, long sq, int nq, int group,
-                    cudaStream_t st, bool trans = false, long k_valid = 0) {
+                    cudaStream_t st, bool trans = false, long k_valid = 0, const OzRowPack& pk = OzRowPack()) {
   XTD_REQUIRE(nq >= 1 && nq <= 65535, XTD_ERR_ARG, "oz_slice: %d q-slices per launch (1..65535)", nq);
-  XTD_REQUIRE(trans || (ld % 2 == 0 && sq % 2 == 0 && ((uintptr_t)X & 15) == 0), XTD_ERR_ALIGN,
+  XTD_REQUIRE(trans || (ld % 2 == 0 && sq % 2 == 0 && pk.sp % 2 == 0 && ((uintptr_t)X & 15) == 0), XTD_ERR_ALIGN,
               "oz_slice: operand must be 16-byte aligned with even strides");
+  XTD_REQUIRE(pk.G == 0 || (!trans && pk.o2 >= 1 && pk.o2 <= pk.no && pk.G * pk.no <= sh.rows_pad), XTD_ERR_ARG, "oz_slice: bad row packing");
   if (k_valid <= 0) k_valid = (long)nq * sh.K;
   switch (S) {
-    case 3: return oz_slice_launch<3>(out, scale, sh, X, ld, sq, nq, group, trans, k_valid, st);
-    case 4: return oz_slice_launch<4>(out, scale, sh, X, ld, sq, nq, group, trans, k_valid, st);
-    case 5: return oz_slice_launch<5>(out, scale, sh, X, ld, sq, nq, group, trans, k_valid, st);
-    case 6: return oz_slice_launch<6>(out, scale, sh, X, ld, sq, nq, group, trans, k_valid, st);
-    case 7: return oz_slice_launch<7>(out, scale, sh, X, ld, sq, nq, group, trans, k_valid, st);
-    case 8: return oz_slice_launch<8>(out, scale, sh, X, ld, sq, nq, group, trans, k_valid, st);
+    case 3: return oz_slice_launch<3>(out, scale, sh, X, ld, sq, nq, group, trans, k_valid, pk, st);
+    case 4: return oz_slice_launch<4>(out, scale, sh, X, ld, sq, nq, group, trans, k_valid, pk, st);
+    case 5: return oz_slice_launch<5>(out, scale, sh, X, ld, sq, nq, group, trans, k_valid, pk, st);
+    case 6: return oz_slice_launch<6>(out, scale, sh, X, ld, sq, nq, group, trans, k_valid, pk, st);
+    case 7: return oz_slice_launch<7>(out, scale, sh, X, ld, sq, nq, group, trans, k_valid, pk, st);
+    case 8: return oz_slice_launch<8>(out, scale, sh, X, ld, sq, nq, group, trans, k_valid, pk, st);
   }
   XTD_SET_ERR("oz_slice: %d slices (3..8)", S);
   return XTD_ERR_ARG;

@@ -72,10 +72,12 @@ struct Channel {
   int oz_group = 0;
   int oz_col0[2] = {0, 0};                  // first output column of the emulated block: 0, or the start of the second virtual
                                             // block for block-weighted terms (the narrow first block keeps its DMMA pass)
-  // ... and the occupied-occupied block as the A operand of the fused half-transform (oz_k1_kernel): planes, row scales, row 2-norms
+  // ... and the occupied-occupied block as the A operand of the fused half-transform (oz_k1_kernel): planes and row scales with the
+  // rows (P, i) of oz_group aux functions packed into one q-slice (oz_unpack_row, split at oz_row_split()), row 2-norms [naux_loc][no]
   int8_t* LooS[2] = {nullptr, nullptr};
   double *LooScale[2] = {nullptr, nullptr}, *LooNorm[2] = {nullptr, nullptr};
   OzShape ozL;
+  int oz_row_split() const { return o_blocks.size() > 1 ? o_blocks[1].first : no; }
   // grid path on the emulated GEMMs (one AO component): MO values of the virtual orbitals kept as int8 planes in both operand
   // roles -- rows = grid points, K = virtual index (forward Y = phiv . z^T) and rows = virtual index, K = blocks of OZ_XC_KQ grid
   // points (backward sigma += A^T . phiv) -- instead of the fp64 array
@@ -753,14 +755,17 @@ int xtd_df_begin(xtd_handle h, int tensor, long naux_local) {
       XTD_CUDA(cudaMalloc((void**)&c->LvvS[tensor], std::max<size_t>(c->ozB.slice_bytes(naux_local, h->oz_slices), 16)));
       XTD_CUDA(cudaMalloc((void**)&c->LvvScale[tensor], std::max<size_t>(c->ozB.scale_doubles(naux_local, c->oz_group), 2) * 8));
       c->Lvv[tensor].release();
-      c->ozL.set(c->no, OZ_BM, c->no);
+      // Packing G aux functions per row tile, padded per group rather than per aux function: the chunks of xtd_df_add and of
+      // run_k_emulated start on group boundaries, so no row tile straddles a chunk (config 5: 4 x 277 rows in 9 tiles, against 12)
+      c->ozL.set(c->oz_group * c->no, OZ_BM, c->no);
+      const long loo_groups = cdiv(naux_local, c->oz_group);
       if (c->LooS[tensor]) cudaFree(c->LooS[tensor]);
       if (c->LooScale[tensor]) cudaFree(c->LooScale[tensor]);
       if (c->LooNorm[tensor]) cudaFree(c->LooNorm[tensor]);
       c->LooS[tensor] = nullptr; c->LooScale[tensor] = c->LooNorm[tensor] = nullptr;
-      XTD_CUDA(cudaMalloc((void**)&c->LooS[tensor], std::max<size_t>(c->ozL.slice_bytes(naux_local, h->oz_slices), 16)));
-      XTD_CUDA(cudaMalloc((void**)&c->LooScale[tensor], std::max<size_t>((size_t)naux_local * c->ozL.rows_pad, 2) * 8));
-      XTD_CUDA(cudaMalloc((void**)&c->LooNorm[tensor], std::max<size_t>((size_t)naux_local * c->ozL.rows_pad, 2) * 8));
+      XTD_CUDA(cudaMalloc((void**)&c->LooS[tensor], std::max<size_t>(c->ozL.slice_bytes(loo_groups, h->oz_slices), 16)));
+      XTD_CUDA(cudaMalloc((void**)&c->LooScale[tensor], std::max<size_t>(c->ozL.scale_doubles(loo_groups, 1), 2) * 8));
+      XTD_CUDA(cudaMalloc((void**)&c->LooNorm[tensor], std::max<size_t>((size_t)naux_local * c->no, 2) * 8));
     } else {
       XTD_TRY(c->Lvv[tensor].alloc((size_t)naux_local * c->nv * c->ldvv, h->stream));
     }
@@ -884,12 +889,17 @@ int xtd_df_add(xtd_handle h, int tensor, const double* l_dev, long np, long ld_r
           e.C = c->Loo[tensor].p + P0 * c->no * c->ldoo; e.ldc = c->ldoo; e.c_batch_stride = (long)c->no * c->ldoo;
           XTD_TRY(gemm(h->gemm, e, s));
           if (c->use_oz[tensor]) {
-            // A operand of the fused half-transform: one q-slice per aux function, one scale per (aux function, row)
+            // A operand of the fused half-transform: one q-slice per group of oz_group aux functions (P0 is a group boundary), rows
+            // (P, i) packed, one scale per (aux function, row)
+            const int G = c->oz_group;
+            XTD_REQUIRE(P0 % G == 0, XTD_ERR_ARG, "xtd_df_add: aux chunk at %ld does not start a group of %d", P0, G);
             const double* lc = c->Loo[tensor].p + P0 * c->no * c->ldoo;
-            XTD_TRY(oz_slice(h->oz_slices, c->LooS[tensor] + c->ozL.slice_bytes(P0, h->oz_slices), c->LooScale[tensor] + (size_t)P0 * c->ozL.rows_pad,
-                             c->ozL, lc, c->ldoo, (long)c->no * c->ldoo, pn, 1, s));
-            oz_rownorm_kernel<<<dim3(c->ozL.rows_pad, pn), 128, 0, s>>>(c->LooNorm[tensor] + (size_t)P0 * c->ozL.rows_pad, c->ozL.rows_pad, lc, c->ldoo,
-                                                                        (long)c->no * c->ldoo, c->no, c->no);
+            OzRowPack pk;
+            pk.G = G; pk.o2 = c->oz_row_split(); pk.no = c->no; pk.np = pn; pk.sp = (long)c->no * c->ldoo;
+            XTD_TRY(oz_slice(h->oz_slices, c->LooS[tensor] + c->ozL.slice_bytes(P0 / G, h->oz_slices), c->LooScale[tensor] + (size_t)(P0 / G) * c->ozL.rows_pad,
+                             c->ozL, lc, c->ldoo, (long)G * c->no * c->ldoo, (int)cdiv(pn, G), 1, s, false, 0, pk));
+            oz_rownorm_kernel<<<dim3(c->no, pn), 128, 0, s>>>(c->LooNorm[tensor] + (size_t)P0 * c->no, c->no, lc, c->ldoo, (long)c->no * c->ldoo, c->no,
+                                                              c->no);
             LAUNCH_CHECK();
           }
           if (c->need_split[tensor]) {
@@ -1717,18 +1727,21 @@ static int run_k_emulated(xtd_engine* h, const KTermRec& k, int nvec) {
       PhaseTimer t(h, XTD_T_K1);
       for (int ip = 0; ip < npass; ++ip) {
         const RowPass& rp = passes[ip];
-        oz_bound_scale_kernel<<<dim3((unsigned)cdiv(shA.rows_pad, 256), ng), 256, 0, s>>>(so, shA.rows_pad, ch->LooNorm[k.tensor] + (size_t)P0 * shL.rows_pad,
-                                                                                          shL.rows_pad, zmax[ip], pn, G, nvec, ch->no, rp.i_lo, rp.i_hi);
+        oz_bound_scale_kernel<<<dim3((unsigned)cdiv(shA.rows_pad, 256), ng), 256, 0, s>>>(so, shA.rows_pad, ch->LooNorm[k.tensor] + (size_t)P0 * ch->no,
+                                                                                          ch->no, zmax[ip], pn, G, nvec, ch->no, rp.i_lo, rp.i_hi);
         LAUNCH_CHECK();
+        // the packed row tiles of every group that hold the rows of this pass (P0 is a group boundary: pc is a multiple of G)
+        const int o2 = ch->oz_row_split();
         OzK1Params q;
-        q.A = ch->LooS[k.tensor] + shL.slice_bytes(P0, S); q.B = ztS[ip];
-        q.sa = ch->LooScale[k.tensor] + (size_t)P0 * shL.rows_pad; q.sb = ztScale[ip]; q.so = so; q.out = As;
-        q.np = pn; q.nit = shL.nrt; q.nbt = shZt.nrt; q.nkb1 = shL.nkb; q.nvec = nvec; q.no = ch->no; q.group = G;
+        q.A = ch->LooS[k.tensor] + shL.slice_bytes(P0 / G, S); q.B = ztS[ip];
+        q.sa = ch->LooScale[k.tensor] + (size_t)(P0 / G) * shL.rows_pad; q.sb = ztScale[ip]; q.so = so; q.out = As;
+        q.np = pn; q.ntg = shL.nrt; q.nbt = shZt.nrt; q.nkb1 = shL.nkb; q.nvec = nvec; q.no = ch->no; q.o2 = o2; q.group = G;
         q.nmt2 = shA.nrt; q.nkb2 = shA.nkb; q.Mpad2 = shA.rows_pad;
         q.i_lo = rp.i_lo; q.i_hi = rp.i_hi;
-        q.it0 = rp.i_lo / OZ_BM; q.nit_run = (rp.i_hi - 1) / OZ_BM - q.it0 + 1;
-        q.ntiles = (long)pn * q.nit_run * nvec * q.nbt;
-        XTD_TRY(oz_k1(S, q, h->gemm.num_sms, s));
+        q.t0 = oz_packed_row_lo(rp.i_lo, G, o2) / OZ_BM;
+        q.nt_run = (int)cdiv(oz_packed_row_hi(rp.i_hi, G, o2, ch->no), OZ_BM) - q.t0;
+        q.npairs = (long)ng * q.nt_run * cdiv((long)nvec * q.nbt, 2);
+        XTD_TRY(oz_k1(S, q, s));
         h->gemm.flops += 2.0 * pn * (double)(rp.i_hi - rp.i_lo) * ch->no * ch->nv * nvec;
       }
     }
