@@ -140,6 +140,18 @@ int xtd_xc_split_form(xtd_handle h, int nvec);
  * environment variables XTD_CHUNK_AUX / XTD_CHUNK_GRID (read by xtd_create) bound the chunk sizes from above */
 int xtd_last_chunks(xtd_handle h, long* aux_chunks, long* grid_chunks);
 
+/* Responses of symmetric MO-block densities on the engine's resident blocks (the right-hand side and the W matrix of the Z-vector
+ * equation of the gradients, grad_hb/tdroks_sfu.py:241-254,339-351).  Two-channel plans only.  xtd_enable_block_response (before the
+ * grid commit and xtd_df_begin) keeps the Coulomb Loo / Lvv of tensor 0 for every channel and the fp64 virtual MO values on the grid.
+ * dens_dev, per channel c in order: Doo[no][no] | Dvv[nv][nv] | Dov[no][nv] on the channel's internal positions (Dvo = Dov^T);
+ * out_dev, per channel: the occupied-occupied [no][no] and occupied-virtual [no][nv] blocks of
+ *     coef[0] J[D_0 + D_1] + coef[3] f_xc[D_c] + coef[1] K_0[D_c] + coef[2] K_1[D_c]
+ * (f_xc with the kernel table as uploaded; K_t = exchange with DF tensor t).  x_dev (may be null): X[no_1][nv_0] on (channel-1
+ * occupied) x (channel-0 virtual); xout_dev[no_1 + nv_1][no_0 + nv_0] = coef[4] K_0[X] on (channel-1 occupied, virtual) x (channel-0
+ * occupied, virtual).  Outputs are this rank's partial sums (aux block, grid batch): all-reduce them over the ranks. */
+int xtd_enable_block_response(xtd_handle h);
+int xtd_block_response(xtd_handle h, const double* dens_dev, double* out_dev, const double* coef_host, const double* x_dev, double* xout_dev);
+
 /* Davidson subspace algebra on device vectors (Davidson.py:152-271): all row vectors of length n */
 int xtd_vec_dots(void* stream, double* g_dev, int ldg, const double* a_dev, long lda, int m, const double* b_dev, long ldb, int k, long n);
 int xtd_vec_lincomb(void* stream, double* y_dev, long ldy, const double* x_dev, long ldx, const double* c_dev, int ldc, int m, int k,

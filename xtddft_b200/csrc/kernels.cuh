@@ -649,6 +649,90 @@ __global__ void build_wf_mcol_kernel(double* __restrict__ wf, const double* __re
 }
 
 // ------------------------------------------------------------------------------------------------------
+// Grid kernel weighting of a SYMMETRIC MO-block density (xtd_block_response), UKS kernel tables, both channels:
+//   Wo[c][g,i] = sum_p phi_c[g,p] D[p,i]  (p over the channel's occupied and virtual positions),  Wv[c][g,a] likewise
+//   rho_0 = sum_i phi_0 Wo_0 + sum_a phiv_0 Wv_0      rho_k = 2 (sum_i phi_k Wo_0 + sum_a phiv_k Wv_0)
+//   tau   = 1/2 sum_k (sum_i phi_k Wo_k + sum_a phiv_k Wv_k)                              (TAU: Wo_k, Wv_k of k = 1..3 given)
+//   wv = f_xc . rho,   Bo_0 = wv_0 phi_0 + sum_k wv_k phi_k,   Bo_k = wv_k phi_0 + 1/2 wv_tau phi_k   (written over Wo)
+// so that the response blocks are  V_oo = sum_c Bo_c^T phi_c  and  V_ov = sum_c Bo_c^T phiv_c.  One warp per grid point.
+// ------------------------------------------------------------------------------------------------------
+struct XcBlockArgs {
+  int gb;
+  long g0;
+  double* Wo[2];           // [nvar][gb][ldWo]
+  const double* Wv[2];     // [nvar][gb][ldWv]
+  long ldWo[2], ldWv[2];
+  const double* phi[2];    // [nvar][ng][ldphi]
+  const double* phiv[2];
+  long ldphi[2], ldphiv[2], phi_comp[2], phiv_comp[2];
+  int no[2], nv[2];
+  const double* wf;        // UKS [ng][(2 nk)^2], weighted
+};
+
+template <int NVAR, bool TAU>
+__global__ void __launch_bounds__(256) xc_block_weight_kernel(const XcBlockArgs a) {
+  static_assert(!TAU || NVAR == 4, "the tau component needs value + gradient AO components");
+  const int lane = threadIdx.x & 31;
+  const long g = (long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (g >= a.gb) return;
+  constexpr int NK = TAU ? 5 : NVAR;
+  constexpr int NR = 2 * NK;
+  double fk[NR];
+  const double* row = a.wf + (a.g0 + g) * (long)(NR * NR);
+#pragma unroll
+  for (int q = 0; q < NR; ++q) fk[q] = (lane < NR) ? row[lane * NR + q] : 0.0;
+  double rho[NR];
+#pragma unroll
+  for (int q = 0; q < NR; ++q) rho[q] = 0.0;
+#pragma unroll
+  for (int s = 0; s < 2; ++s) {
+    const long wcmp_o = (long)a.gb * a.ldWo[s], wcmp_v = (long)a.gb * a.ldWv[s];
+    for (int side = 0; side < 2; ++side) {
+      const int n = side ? a.nv[s] : a.no[s];
+      const double* p = side ? a.phiv[s] + (a.g0 + g) * a.ldphiv[s] : a.phi[s] + (a.g0 + g) * a.ldphi[s];
+      const long pc = side ? a.phiv_comp[s] : a.phi_comp[s];
+      const double* w = side ? a.Wv[s] + g * a.ldWv[s] : a.Wo[s] + g * a.ldWo[s];
+      const long wc = side ? wcmp_v : wcmp_o;
+      for (int o = lane; o < n; o += 32) {
+        const double w0 = w[o];
+        rho[s * NK] += p[o] * w0;
+#pragma unroll
+        for (int k = 1; k < NVAR; ++k) {
+          const double pk = p[k * pc + o];
+          rho[s * NK + k] += 2.0 * pk * w0;
+          if (TAU) rho[s * NK + 4] += 0.5 * pk * w[k * wc + o];
+        }
+      }
+    }
+  }
+#pragma unroll
+  for (int q = 0; q < NR; ++q) rho[q] = warp_sum(rho[q]);
+  double mine = 0.0;
+#pragma unroll
+  for (int q = 0; q < NR; ++q) mine += fk[q] * rho[q];      // wv[t,d] = sum_{s,c} wf[g][t,d][s,c] rho[s,c]
+  double wv[NR];
+#pragma unroll
+  for (int q = 0; q < NR; ++q) wv[q] = __shfl_sync(0xffffffffu, mine, q);
+#pragma unroll
+  for (int s = 0; s < 2; ++s) {
+    double* w = a.Wo[s] + g * a.ldWo[s];
+    const long wc = (long)a.gb * a.ldWo[s];
+    const double* p = a.phi[s] + (a.g0 + g) * a.ldphi[s];
+    for (int o = lane; o < a.no[s]; o += 32) {
+      const double p0 = p[o];
+      double b0 = wv[s * NK] * p0;
+#pragma unroll
+      for (int k = 1; k < NVAR; ++k) {
+        const double pk = p[k * a.phi_comp[s] + o];
+        b0 += wv[s * NK + k] * pk;
+        w[k * wc + o] = wv[s * NK + k] * p0 + (TAU ? 0.5 * wv[s * NK + 4] * pk : 0.0);
+      }
+      w[o] = b0;
+    }
+  }
+}
+
+// ------------------------------------------------------------------------------------------------------
 // density-fitted Coulomb blocks
 // ------------------------------------------------------------------------------------------------------
 // R[x][P] = sum_{i,a in block} L[P][i][a] * Z[x][r0+i][c0+a]        one CTA per aux function
@@ -689,6 +773,18 @@ __global__ void j_mix_kernel(double* __restrict__ Rm, const double* __restrict__
     for (int s = 0; s < njb; ++s) acc += mix[t * njb + s] * R[((long)x * njb + s) * ldr + P];
     Rm[((long)x * njb + t) * ldr + P] = acc;
   }
+}
+
+// rho[P] = sum_r w[r] R[r][P]   (the per-block densities of xtd_block_response -> one fitted density)
+struct RhoWeights {
+  double w[6];
+};
+__global__ void rho_combine_kernel(double* __restrict__ rho, const double* __restrict__ R, long ldr, int nrows, long n, const RhoWeights w) {
+  const long P = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (P >= n) return;
+  double acc = 0.0;
+  for (int r = 0; r < nrows; ++r) acc += w.w[r] * R[r * ldr + P];
+  rho[P] = acc;
 }
 
 // S[x][r0+i][c0+a] += sum_P Rm[x][P] * L[P][i][a]      each thread owns one block element, XC vectors at a time

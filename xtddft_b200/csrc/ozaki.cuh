@@ -242,6 +242,23 @@ __global__ void __launch_bounds__(128) oz_slice_kernel(int8_t* __restrict__ out,
   for (int sl = 0; sl < S; ++sl) *reinterpret_cast<uint4*>(dst + sl * plane) = make_uint4(pk[sl][0], pk[sl][1], pk[sl][2], pk[sl][3]);
 }
 
+// The fp64 values a stacked (B operand, 64-row tile) image stands for: out[p][row][k] = scale[(q0 + p) / group][row] *
+// sum_l d_l 2^(-8 l) of q-slice q0 + p -- exactly what the INT8 contraction multiplies.  One thread per element.
+__global__ void oz_unslice_b_kernel(double* __restrict__ out, long ld, long sp, const int8_t* __restrict__ img, const double* __restrict__ scale,
+                                    int S, int rows, int rows_pad, int K, int nkb, int group, long q0, int np) {
+  const long e = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  const long p = blockIdx.y;
+  if (e >= (long)rows * K || p >= np) return;
+  const int row = (int)(e / K), k = (int)(e - (long)row * K);
+  const long q = q0 + p;
+  const int nrt = rows_pad / OZ_BN, rt = row / OZ_BN, r = row - rt * OZ_BN;
+  const int8_t* src = img + (((q * nrt + rt) * nkb + k / OZ_KB) * S) * ((long)OZ_BN * OZ_KB) + (long)((k % OZ_KB) / 16) * S * OZ_BN * 16 +
+                      (long)r * 16 + (k % 16);
+  double acc = 0.0;
+  for (int l = S - 1; l >= 0; --l) acc = acc * (1.0 / 256.0) + (double)src[(long)l * OZ_BN * 16];
+  out[p * sp + (long)row * ld + k] = scale[(q / group) * rows_pad + row] * acc;
+}
+
 // ---- the INT8 tensor-core kernel ------------------------------------------------------------------------------------------
 struct OzGemmParams {
   const int8_t* A;      // [nq][nmt][nkb][S][128 x 32]

@@ -246,6 +246,9 @@ struct xtd_engine {
   };
   std::vector<GraphRec> graphs;
   bool graphs_off = false;        // set when a capture failed: later calls run eagerly
+  // xtd_enable_block_response: Loo / Lvv of tensor 0 stay resident for every channel (Coulomb of occupied-occupied and
+  // virtual-virtual densities) and the fp64 virtual MO values stay on the grid next to their int8 planes
+  bool block_resp = false;
   bool capturing = false;
   cudaStream_t cap_stream = nullptr;   // calls are recorded on this stream (the caller's may be the legacy default stream,
                                        // which cannot be captured) and replayed on the caller's
@@ -354,6 +357,9 @@ int build_channel_matrices(xtd_engine* h, Channel* c) {
   return XTD_OK;
 }
 
+// Loo / Lvv of `tensor` are built for channel c: an exchange term needs them, or the block response keeps the Coulomb ones
+bool oovv_resident(const xtd_engine* h, const Channel* c, int tensor) { return c->need_k[tensor] || (tensor == 0 && h->block_resp); }
+
 MatView view2d(const double* base, long ld, int rows, int cols, int row0 = 0, int col0 = 0) {
   MatView v;
   v.base = base; v.ld = ld; v.sq = 0; v.row0 = row0; v.col0 = col0; v.rows = rows; v.cols = cols; v.q0 = 0; v.nq = 1;
@@ -433,7 +439,7 @@ int grid_commit(xtd_engine* h) {
         if (split_oz) {
           c->xc_oz_split = true;
         } else {
-          c->phiv.release();                 // one component: the fp64 array is not read again
+          if (!h->block_resp) c->phiv.release();   // one component: the sigma path does not read the fp64 array again
           c->xc_oz = true;
         }
       }
@@ -729,7 +735,7 @@ int xtd_df_begin(xtd_handle h, int tensor, long naux_local) {
   for (auto* c : h->ch)
     if (c->need_kt[tensor]) XTD_TRY(c->Lov[tensor].alloc((size_t)naux_local * c->no * c->ldz, h->stream));
   for (auto* c : h->ch) {
-    if (!c->need_k[tensor]) continue;
+    if (!oovv_resident(h, c, tensor)) continue;
     XTD_TRY(c->Loo[tensor].alloc((size_t)naux_local * c->no * c->ldoo, h->stream));
     // emulated path: uniform-weight terms, or block-weighted terms whose first virtual block is narrow (it keeps its DMMA pass;
     // the wide second block is emulated with one half-transform per occupied row block).  Mixed term lists stay on DMMA.
@@ -793,11 +799,11 @@ int xtd_df_add(xtd_handle h, int tensor, const double* l_dev, long np, long ld_r
   // per-aux workspace: staging copy (if needed) + the largest half-transformed block
   int max_n = 0;
   for (auto* c : h->ch) {
-    bool need_o = c->need_k[tensor] || c->need_kt[tensor];
+    bool need_o = oovv_resident(h, c, tensor) || c->need_kt[tensor];
     if (tensor == 0)
       for (auto* j : h->jblocks) need_o = need_o || (h->ch[j->ch] == c);
     if (need_o) max_n = std::max(max_n, c->no);
-    if (c->need_k[tensor]) max_n = std::max(max_n, c->nv);
+    if (oovv_resident(h, c, tensor)) max_n = std::max(max_n, c->nv);
   }
   if (tensor == 0 && h->n_open > 0) max_n = std::max(max_n, 1);
   if (max_n == 0) { h->naux_filled[tensor] += np; return XTD_OK; }
@@ -870,7 +876,7 @@ int xtd_df_add(xtd_handle h, int tensor, const double* l_dev, long np, long ld_r
     }
     for (size_t ci = 0; ci < h->ch.size(); ++ci) {
       Channel* c = h->ch[ci];
-      bool need_o = c->need_k[tensor] || c->need_kt[tensor];
+      bool need_o = oovv_resident(h, c, tensor) || c->need_kt[tensor];
       if (tensor == 0)
         for (auto* j : h->jblocks) need_o = need_o || (j->ch == (int)ci);
       if (need_o) {
@@ -881,7 +887,7 @@ int xtd_df_add(xtd_handle h, int tensor, const double* l_dev, long np, long ld_r
         d.C = half; d.ldc = ldN; d.c_batch_stride = (long)c->no * ldN;
         XTD_TRY(gemm(h->gemm, d, s));
         MatView Hv = view3d(half, ldN, (long)c->no * ldN, pn, c->no, N);
-        if (c->need_k[tensor]) {
+        if (oovv_resident(h, c, tensor)) {
           // Loo[P][i][j] = sum_mu HoT[P][i][mu] CoT[j][mu]
           GemmDesc e;
           e.A = Hv; e.B = view2d(c->CoT.p, ldN, c->no, N); e.M = c->no; e.N = c->no; e.K = N;
@@ -934,7 +940,7 @@ int xtd_df_add(xtd_handle h, int tensor, const double* l_dev, long np, long ld_r
             XTD_TRY(gemm(h->gemm, e, s));
           }
       }
-      if (c->need_k[tensor]) {
+      if (oovv_resident(h, c, tensor)) {
         // HvT[P][a][mu] = sum_nu CvT[a][nu] L[P][mu][nu] ;  Lvv[P][a][b] = sum_mu HvT[P][a][mu] CvT[b][mu]
         GemmDesc d;
         d.A = view2d(c->CvT.p, ldN, c->nv, N); d.B = Lv; d.M = c->nv; d.N = N; d.K = N;
@@ -2713,4 +2719,322 @@ extern "C" int xtd_host_gs_coefficients(const double* g, int n, double lindep, d
   const int nk = gs_coefficients(g, n, lindep, t);
   std::copy(t.begin(), t.end(), t_out);
   return nk;
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// Response of symmetric MO-block densities on the resident blocks (xtd_block_response): the right-hand side and the W matrix of
+// the Z-vector equation.  Per channel c the density D_c has an occupied-occupied block, a virtual-virtual block and an
+// occupied-virtual block (the virtual-occupied one is its transpose); the outputs are the occupied-occupied and occupied-virtual
+// blocks of  c_J J[D_0 + D_1] + c_xc f_xc[D_c] + sum_t c_K[t] K_t[D_c].  With L[P] = [[Loo, Lov], [Lvo, Lvv]] per aux function:
+//   A[P] = Loo Doo + Lov Dov^T,  B[P] = Loo Dov + Lov Dvv       K_oo = sum_P A Loo + B Lov^T,   K_ov = sum_P A Lov + B Lvv
+// ---------------------------------------------------------------------------------------------------------
+namespace {
+
+// occupied-virtual block of `tensor` in channel ci: the transposed-density exchange copy, or a full-channel Coulomb block
+const double* ov_block(const xtd_engine* h, int ci, int tensor, long* ld) {
+  const Channel* c = h->ch[ci];
+  if (c->need_kt[tensor]) { *ld = c->ldz; return c->Lov[tensor].p; }
+  if (tensor == 0)
+    for (auto* j : h->jblocks)
+      if (j->ch == ci && j->r0 == 0 && j->nr == c->no && j->c0 == 0 && j->nc == c->nv) { *ld = j->ld; return j->L.p; }
+  return nullptr;
+}
+
+int mm(xtd_engine* h, const MatView& A, bool akc, const MatView& B, bool bkc, int M, int N, int K, int nouter, int batches, double* Cp,
+       long ldc, long cbs, double alpha, bool acc) {
+  GemmDesc d;
+  d.A = A; d.B = B; d.a_kc = akc; d.b_kc = bkc; d.M = M; d.N = N; d.K = K; d.nouter = nouter;
+  d.batches = batches; d.z_div = 1; d.a_hi = batches > 1 ? 1 : 0; d.b_hi = 0;
+  d.C = Cp; d.ldc = ldc; d.c_batch_stride = cbs; d.alpha = alpha; d.accumulate = acc;
+  return gemm(h->gemm, d, h->stream);
+}
+
+struct BlockBufs {
+  double *Doo, *Dvv, *Dov, *Ooo, *Oov;
+};
+
+int block_response_df(xtd_engine* h, const BlockBufs* bb, const double* coef, const double* X, double* const* XO, double* scratch,
+                      size_t scratch_doubles) {
+  cudaStream_t s = h->stream;
+  const double cj = coef[0], cx = coef[4];
+  for (int t = 0; t < 2; ++t) {
+    const double ck = coef[1 + t];
+    const bool doJ = t == 0 && cj != 0.0, doK = ck != 0.0, doX = t == 0 && X && cx != 0.0;
+    if (!(doJ || doK || doX) || h->naux[t] == 0) continue;
+    const long naux = h->naux[t];
+    const double* Lov[2];
+    long ldov[2];
+    size_t per_p = 8;
+    for (int ci = 0; ci < 2; ++ci) {
+      Channel* c = h->ch[ci];
+      Lov[ci] = ov_block(h, ci, t, &ldov[ci]);
+      XTD_REQUIRE(oovv_resident(h, c, t) && Lov[ci], XTD_ERR_STATE,
+                  "xtd_block_response: channel %d holds no MO blocks of tensor %d (call xtd_enable_block_response before xtd_df_begin)", ci, t);
+      XTD_REQUIRE(!c->use_oz[t] || c->oz_col0[t] == 0, XTD_ERR_UNSUPPORTED, "xtd_block_response: block-weighted emulated exchange image");
+      per_p += (size_t)c->no * c->ldoo + (size_t)c->no * c->ldz + (c->use_oz[t] ? (size_t)c->nv * c->ldvv : 0);
+    }
+    Channel *c0 = h->ch[0], *c1 = h->ch[1];
+    if (doX) per_p += (size_t)c1->no * c0->ldz + (size_t)c1->nv * c0->ldz;
+    long pc = (long)(scratch_doubles / (per_p + 64));
+    if (h->env.max_pc > 0) pc = std::min<long>(pc, h->env.max_pc);
+    pc = std::min<long>(pc, naux);
+    XTD_REQUIRE(pc >= 1, XTD_ERR_NOMEM, "xtd_block_response: workspace too small for one aux function (%zu doubles)", per_p);
+    double* cur = scratch;
+    auto take = [&](size_t n) { double* p = cur; cur += (n + 31) & ~(size_t)31; return p; };
+    double *Ab[2], *Bb[2], *Ldec[2] = {nullptr, nullptr};
+    for (int ci = 0; ci < 2; ++ci) {
+      Channel* c = h->ch[ci];
+      Ab[ci] = take((size_t)pc * c->no * c->ldoo);
+      Bb[ci] = take((size_t)pc * c->no * c->ldz);
+      if (c->use_oz[t]) Ldec[ci] = take((size_t)pc * c->nv * c->ldvv);
+    }
+    double* U = doX ? take((size_t)pc * c1->no * c0->ldz) : nullptr;
+    double* V = doX ? take((size_t)pc * c1->nv * c0->ldz) : nullptr;
+    double* R = take((size_t)6 * pc);
+    double* rho = take((size_t)pc);
+    h->last_aux_chunks = std::max<long>(h->last_aux_chunks, cdiv(naux, pc));
+    for (long P0 = 0; P0 < naux; P0 += pc) {
+      const int pn = (int)std::min<long>(pc, naux - P0);
+      const double *Loo[2], *Lvv[2], *Lo[2];
+      for (int ci = 0; ci < 2; ++ci) {
+        Channel* c = h->ch[ci];
+        Loo[ci] = c->Loo[t].p + P0 * c->no * c->ldoo;
+        Lo[ci] = Lov[ci] + P0 * c->no * ldov[ci];
+        if (c->use_oz[t]) {
+          PhaseTimer tm(h, XTD_T_K2_SLICE);
+          oz_unslice_b_kernel<<<dim3((unsigned)cdiv((long)c->nv * c->nv, 256), pn), 256, 0, s>>>(
+              Ldec[ci], c->ldvv, (long)c->nv * c->ldvv, c->LvvS[t], c->LvvScale[t], h->oz_slices, c->nv, c->ozB.rows_pad, c->nv, c->ozB.nkb,
+              c->oz_group, P0, pn);
+          LAUNCH_CHECK();
+          Lvv[ci] = Ldec[ci];
+        } else {
+          Lvv[ci] = c->Lvv[t].p + P0 * c->nv * c->ldvv;
+        }
+      }
+      if (doJ) {
+        PhaseTimer tm(h, XTD_T_J);
+        // rho_P = sum_c <Loo, Doo> + <Lvv, Dvv> + 2 <Lov, Dov>;  Ooo += c_J sum_P rho_P Loo[P],  Oov += c_J sum_P rho_P Lov[P]
+        for (int ci = 0; ci < 2; ++ci) {
+          Channel* c = h->ch[ci];
+          j_rho_kernel<1><<<pn, 256, 0, s>>>(R + (3 * ci) * pc, 0, Loo[ci], c->ldoo, (long)c->no * c->ldoo, bb[ci].Doo, c->ldoo, 0, c->no, c->no, 1);
+          LAUNCH_CHECK();
+          j_rho_kernel<1><<<pn, 256, 0, s>>>(R + (3 * ci + 1) * pc, 0, Lvv[ci], c->ldvv, (long)c->nv * c->ldvv, bb[ci].Dvv, c->ldvv, 0, c->nv, c->nv, 1);
+          LAUNCH_CHECK();
+          j_rho_kernel<1><<<pn, 256, 0, s>>>(R + (3 * ci + 2) * pc, 0, Lo[ci], ldov[ci], (long)c->no * ldov[ci], bb[ci].Dov, c->ldz, 0, c->no, c->nv, 1);
+          LAUNCH_CHECK();
+        }
+        RhoWeights w = {{cj, cj, 2.0 * cj, cj, cj, 2.0 * cj}};
+        rho_combine_kernel<<<grid1d(pn, 256), 256, 0, s>>>(rho, R, pc, 6, pn, w);
+        LAUNCH_CHECK();
+        for (int ci = 0; ci < 2; ++ci) {
+          Channel* c = h->ch[ci];
+          j_apply_kernel<1><<<dim3((unsigned)cdiv((long)c->no * c->no, 256), 1), 256, 0, s>>>(bb[ci].Ooo, c->ldoo, 0, Loo[ci], c->ldoo,
+                                                                                           (long)c->no * c->ldoo, rho, 0, pn, c->no, c->no, 1);
+          LAUNCH_CHECK();
+          j_apply_kernel<1><<<dim3((unsigned)cdiv((long)c->no * c->nv, 256), 1), 256, 0, s>>>(bb[ci].Oov, c->ldz, 0, Lo[ci], ldov[ci],
+                                                                                           (long)c->no * ldov[ci], rho, 0, pn, c->no, c->nv, 1);
+          LAUNCH_CHECK();
+        }
+      }
+      if (doK)
+        for (int ci = 0; ci < 2; ++ci) {
+          Channel* c = h->ch[ci];
+          const int no = c->no, nv = c->nv;
+          const long soo = (long)no * c->ldoo, sov = (long)no * ldov[ci], svv = (long)nv * c->ldvv, sA = (long)no * c->ldoo, sB = (long)no * c->ldz;
+          {
+            PhaseTimer tm(h, XTD_T_K1);
+            XTD_TRY(mm(h, view3d(Loo[ci], c->ldoo, soo, pn, no, no), true, view2d(bb[ci].Doo, c->ldoo, no, no), false, no, no, no, 1, pn, Ab[ci], c->ldoo, sA, 1.0, false));
+            XTD_TRY(mm(h, view3d(Lo[ci], ldov[ci], sov, pn, no, nv), true, view2d(bb[ci].Dov, c->ldz, no, nv), true, no, no, nv, 1, pn, Ab[ci], c->ldoo, sA, 1.0, true));
+            XTD_TRY(mm(h, view3d(Loo[ci], c->ldoo, soo, pn, no, no), true, view2d(bb[ci].Dov, c->ldz, no, nv), false, no, nv, no, 1, pn, Bb[ci], c->ldz, sB, 1.0, false));
+            XTD_TRY(mm(h, view3d(Lo[ci], ldov[ci], sov, pn, no, nv), true, view2d(bb[ci].Dvv, c->ldvv, nv, nv), false, no, nv, nv, 1, pn, Bb[ci], c->ldz, sB, 1.0, true));
+          }
+          PhaseTimer tm(h, XTD_T_K2);
+          const MatView Av = view3d(Ab[ci], c->ldoo, sA, pn, no, no), Bv = view3d(Bb[ci], c->ldz, sB, pn, no, nv);
+          XTD_TRY(mm(h, Av, true, view3d(Loo[ci], c->ldoo, soo, pn, no, no), false, no, no, no, pn, 1, bb[ci].Ooo, c->ldoo, 0, ck, true));
+          XTD_TRY(mm(h, Bv, true, view3d(Lo[ci], ldov[ci], sov, pn, no, nv), true, no, no, nv, pn, 1, bb[ci].Ooo, c->ldoo, 0, ck, true));
+          XTD_TRY(mm(h, Av, true, view3d(Lo[ci], ldov[ci], sov, pn, no, nv), false, no, nv, no, pn, 1, bb[ci].Oov, c->ldz, 0, ck, true));
+          XTD_TRY(mm(h, Bv, true, view3d(Lvv[ci], c->ldvv, svv, pn, nv, nv), false, no, nv, nv, pn, 1, bb[ci].Oov, c->ldz, 0, ck, true));
+        }
+      if (doX) {
+        // mixed-spin K[X], X on (channel-1 occupied) x (channel-0 virtual):  U[P] = Loo1 X,  V[P] = Lov1^T X
+        //   XO_oo += c_X sum_P U Lov0^T,  XO_ov += c_X sum_P U Lvv0,  XO_vo += c_X sum_P V Lov0^T,  XO_vv += c_X sum_P V Lvv0
+        const int no1 = c1->no, nv1 = c1->nv, no0 = c0->no, nv0 = c0->nv;
+        const long sU = (long)no1 * c0->ldz, sV = (long)nv1 * c0->ldz, sov0 = (long)no0 * ldov[0], svv0 = (long)nv0 * c0->ldvv;
+        {
+          PhaseTimer tm(h, XTD_T_K1);
+          XTD_TRY(mm(h, view3d(Loo[1], c1->ldoo, (long)no1 * c1->ldoo, pn, no1, no1), true, view2d(X, c0->ldz, no1, nv0), false, no1, nv0, no1, 1, pn, U,
+                     c0->ldz, sU, 1.0, false));
+          XTD_TRY(mm(h, view3d(Lo[1], ldov[1], (long)no1 * ldov[1], pn, no1, nv1), false, view2d(X, c0->ldz, no1, nv0), false, nv1, nv0, no1, 1, pn, V,
+                     c0->ldz, sV, 1.0, false));
+        }
+        PhaseTimer tm(h, XTD_T_K2);
+        const MatView Uv = view3d(U, c0->ldz, sU, pn, no1, nv0), Vv = view3d(V, c0->ldz, sV, pn, nv1, nv0);
+        const MatView Lov0 = view3d(Lo[0], ldov[0], sov0, pn, no0, nv0), Lvv0 = view3d(Lvv[0], c0->ldvv, svv0, pn, nv0, nv0);
+        XTD_TRY(mm(h, Uv, true, Lov0, true, no1, no0, nv0, pn, 1, XO[0], c0->ldoo, 0, cx, true));
+        XTD_TRY(mm(h, Uv, true, Lvv0, false, no1, nv0, nv0, pn, 1, XO[1], c0->ldz, 0, cx, true));
+        XTD_TRY(mm(h, Vv, true, Lov0, true, nv1, no0, nv0, pn, 1, XO[2], c0->ldoo, 0, cx, true));
+        XTD_TRY(mm(h, Vv, true, Lvv0, false, nv1, nv0, nv0, pn, 1, XO[3], c0->ldz, 0, cx, true));
+      }
+    }
+  }
+  return XTD_OK;
+}
+
+// grid term: Wo = phi Doo + phiv Dov^T, Wv = phiv Dvv + phi Dov (value component; all four with tau), xc_block_weight_kernel,
+// then Ooo += c_xc sum_c Bo_c^T phi_c, Oov += c_xc sum_c Bo_c^T phiv_c
+int block_response_xc(xtd_engine* h, const BlockBufs* bb, double cxc, double* scratch, size_t scratch_doubles) {
+  cudaStream_t s = h->stream;
+  XTD_REQUIRE(h->fxc_kind == XTD_FXC_UKS, XTD_ERR_UNSUPPORTED, "xtd_block_response: the grid term needs the UKS kernel tables");
+  const int nve = h->nvar_eff, nf = h->tau ? 4 : 1;
+  size_t per_g = 0;
+  for (auto* c : h->ch) {
+    XTD_REQUIRE(c->phiv.p && c->phi.p, XTD_ERR_STATE,
+                "xtd_block_response: fp64 virtual MO values not kept on the grid (call xtd_enable_block_response before the grid commit)");
+    per_g += (size_t)nve * (c->ldoo + c->ldvv);
+  }
+  long GB = (long)(scratch_doubles / per_g) - 64;
+  GB = std::min<long>(GB, 1 << 16);
+  if (h->env.max_gb > 0) GB = std::min<long>(GB, std::max<long>(h->env.max_gb, 128));
+  GB = (GB / 128) * 128;
+  XTD_REQUIRE(GB >= 128, XTD_ERR_NOMEM, "xtd_block_response: workspace too small for a 128-point grid chunk");
+  h->last_grid_chunks = cdiv(h->ng, GB);
+  for (long g0 = 0; g0 < h->ng; g0 += GB) {
+    const int gb = (int)std::min<long>(GB, h->ng - g0);
+    double *Wo[2], *Wv[2];
+    double* cur = scratch;
+    for (int ci = 0; ci < 2; ++ci) {
+      Wo[ci] = cur; cur += (size_t)nve * gb * h->ch[ci]->ldoo;
+      Wv[ci] = cur; cur += (size_t)nve * gb * h->ch[ci]->ldvv;
+    }
+    {
+      PhaseTimer tm(h, XTD_T_XC_GEMM);
+      for (int ci = 0; ci < 2; ++ci) {
+        Channel* c = h->ch[ci];
+        const int no = c->no, nv = c->nv;
+        const MatView ph = view3d(c->phi.p, c->ldphi, h->ng * c->ldphi, nf, gb, no, (int)g0, 0);
+        const MatView pv = view3d(c->phiv.p, c->ldphiv, h->ng * c->ldphiv, nf, gb, nv, (int)g0, 0);
+        const long so = (long)gb * c->ldoo, sv = (long)gb * c->ldvv;
+        XTD_TRY(mm(h, ph, true, view2d(bb[ci].Doo, c->ldoo, no, no), false, gb, no, no, 1, nf, Wo[ci], c->ldoo, so, 1.0, false));
+        XTD_TRY(mm(h, pv, true, view2d(bb[ci].Dov, c->ldz, no, nv), true, gb, no, nv, 1, nf, Wo[ci], c->ldoo, so, 1.0, true));
+        XTD_TRY(mm(h, pv, true, view2d(bb[ci].Dvv, c->ldvv, nv, nv), false, gb, nv, nv, 1, nf, Wv[ci], c->ldvv, sv, 1.0, false));
+        XTD_TRY(mm(h, ph, true, view2d(bb[ci].Dov, c->ldz, no, nv), false, gb, nv, no, 1, nf, Wv[ci], c->ldvv, sv, 1.0, true));
+      }
+    }
+    {
+      PhaseTimer tm(h, XTD_T_XC_STREAM);
+      XcBlockArgs a;
+      a.gb = gb; a.g0 = g0; a.wf = h->wf.p;
+      for (int ci = 0; ci < 2; ++ci) {
+        Channel* c = h->ch[ci];
+        a.Wo[ci] = Wo[ci]; a.Wv[ci] = Wv[ci]; a.ldWo[ci] = c->ldoo; a.ldWv[ci] = c->ldvv;
+        a.phi[ci] = c->phi.p; a.phiv[ci] = c->phiv.p; a.ldphi[ci] = c->ldphi; a.ldphiv[ci] = c->ldphiv;
+        a.phi_comp[ci] = h->ng * c->ldphi; a.phiv_comp[ci] = h->ng * c->ldphiv;
+        a.no[ci] = c->no; a.nv[ci] = c->nv;
+      }
+      const unsigned grid = (unsigned)cdiv(gb, 8);
+      if (nve == 1) xc_block_weight_kernel<1, false><<<grid, 256, 0, s>>>(a);
+      else if (h->tau) xc_block_weight_kernel<4, true><<<grid, 256, 0, s>>>(a);
+      else xc_block_weight_kernel<4, false><<<grid, 256, 0, s>>>(a);
+      LAUNCH_CHECK();
+    }
+    PhaseTimer tm(h, XTD_T_XC_GEMM);
+    for (int ci = 0; ci < 2; ++ci) {
+      Channel* c = h->ch[ci];
+      const int no = c->no, nv = c->nv;
+      const MatView Bo = view3d(Wo[ci], c->ldoo, (long)gb * c->ldoo, nve, gb, no);
+      XTD_TRY(mm(h, Bo, false, view3d(c->phi.p, c->ldphi, h->ng * c->ldphi, nve, gb, no, (int)g0, 0), false, no, no, gb, nve, 1, bb[ci].Ooo, c->ldoo, 0,
+                 cxc, true));
+      XTD_TRY(mm(h, Bo, false, view3d(c->phiv.p, c->ldphiv, h->ng * c->ldphiv, nve, gb, nv, (int)g0, 0), false, no, nv, gb, nve, 1, bb[ci].Oov, c->ldz,
+                 0, cxc, true));
+    }
+  }
+  return XTD_OK;
+}
+
+int copy_block(double* dst, long ldd, const double* src, long lds, int rows, int cols, cudaStream_t s) {
+  if (rows > 0 && cols > 0)
+    XTD_CUDA(cudaMemcpy2DAsync(dst, (size_t)ldd * 8, src, (size_t)lds * 8, (size_t)cols * 8, rows, cudaMemcpyDeviceToDevice, s));
+  return XTD_OK;
+}
+
+}  // namespace
+
+extern "C" int xtd_enable_block_response(xtd_handle h) {
+  XTD_REQUIRE(h && !h->finalized && !h->grid_committed && h->naux[0] == 0 && h->naux[1] == 0, XTD_ERR_STATE,
+              "xtd_enable_block_response must precede xtd_grid_commit, xtd_df_begin and xtd_finalize");
+  h->block_resp = true;
+  return XTD_OK;
+}
+
+extern "C" int xtd_block_response(xtd_handle h, const double* dens_dev, double* out_dev, const double* coef_host, const double* x_dev,
+                                  double* xout_dev) {
+  XTD_REQUIRE(h && h->finalized, XTD_ERR_STATE, "xtd_block_response before xtd_finalize");
+  XTD_REQUIRE(dens_dev && out_dev && coef_host && (!x_dev || xout_dev), XTD_ERR_ARG, "xtd_block_response: bad arguments");
+  XTD_REQUIRE(h->ch.size() == 2, XTD_ERR_UNSUPPORTED, "xtd_block_response needs a two-channel plan");
+  cudaStream_t s = h->stream;
+  h->ev_used = 0;
+  for (int i = 0; i < 12; ++i) h->phase_flops[i] = 0.0;
+  h->last_aux_chunks = h->last_grid_chunks = 0;
+  if (h->ev_ok) cudaEventRecord(h->ev_total[0], s);
+  h->arena.used = 0;
+  BlockBufs bb[2];
+  for (int ci = 0; ci < 2; ++ci) {
+    Channel* c = h->ch[ci];
+    bb[ci].Doo = h->arena.take((size_t)c->no * c->ldoo);
+    bb[ci].Dvv = h->arena.take((size_t)c->nv * c->ldvv);
+    bb[ci].Dov = h->arena.take((size_t)c->no * c->ldz);
+    bb[ci].Ooo = h->arena.take((size_t)c->no * c->ldoo);
+    bb[ci].Oov = h->arena.take((size_t)c->no * c->ldz);
+    XTD_REQUIRE(bb[ci].Doo && bb[ci].Dvv && bb[ci].Dov && bb[ci].Ooo && bb[ci].Oov, XTD_ERR_NOMEM, "xtd_block_response: workspace exhausted");
+  }
+  Channel *c0 = h->ch[0], *c1 = h->ch[1];
+  double* X = nullptr;
+  double* XO[4] = {nullptr, nullptr, nullptr, nullptr};
+  if (x_dev) {
+    X = h->arena.take((size_t)c1->no * c0->ldz);
+    XO[0] = h->arena.take((size_t)c1->no * c0->ldoo);
+    XO[1] = h->arena.take((size_t)c1->no * c0->ldz);
+    XO[2] = h->arena.take((size_t)c1->nv * c0->ldoo);
+    XO[3] = h->arena.take((size_t)c1->nv * c0->ldz);
+    XTD_REQUIRE(X && XO[0] && XO[1] && XO[2] && XO[3], XTD_ERR_NOMEM, "xtd_block_response: workspace exhausted");
+  }
+  const size_t fixed = h->arena.used;
+  {
+    PhaseTimer tm(h, XTD_T_PACK);
+    XTD_CUDA(cudaMemsetAsync(h->arena.base, 0, fixed, s));
+    const double* src = dens_dev;
+    for (int ci = 0; ci < 2; ++ci) {
+      Channel* c = h->ch[ci];
+      XTD_TRY(copy_block(bb[ci].Doo, c->ldoo, src, c->no, c->no, c->no, s)); src += (size_t)c->no * c->no;
+      XTD_TRY(copy_block(bb[ci].Dvv, c->ldvv, src, c->nv, c->nv, c->nv, s)); src += (size_t)c->nv * c->nv;
+      XTD_TRY(copy_block(bb[ci].Dov, c->ldz, src, c->nv, c->no, c->nv, s)); src += (size_t)c->no * c->nv;
+    }
+    if (X) XTD_TRY(copy_block(X, c0->ldz, x_dev, c0->nv, c1->no, c0->nv, s));
+  }
+  size_t split_bytes = std::min<size_t>(h->arena.left() / 4, (size_t)1 << 30);
+  h->gemm.split_ws = h->arena.take(split_bytes / 8);
+  h->gemm.split_ws_bytes = split_bytes;
+  const size_t scratch_doubles = h->arena.left() / 8 - 64;
+  double* scratch = h->arena.take(scratch_doubles);
+  XTD_REQUIRE(scratch, XTD_ERR_NOMEM, "xtd_block_response: workspace exhausted (chunk scratch)");
+  XTD_TRY(block_response_df(h, bb, coef_host, X, XO, scratch, scratch_doubles));
+  if (coef_host[3] != 0.0 && h->fxc_kind != XTD_FXC_NONE && h->ng > 0) XTD_TRY(block_response_xc(h, bb, coef_host[3], scratch, scratch_doubles));
+  {
+    PhaseTimer tm(h, XTD_T_UNPACK);
+    double* dst = out_dev;
+    for (int ci = 0; ci < 2; ++ci) {
+      Channel* c = h->ch[ci];
+      XTD_TRY(copy_block(dst, c->no, bb[ci].Ooo, c->ldoo, c->no, c->no, s)); dst += (size_t)c->no * c->no;
+      XTD_TRY(copy_block(dst, c->nv, bb[ci].Oov, c->ldz, c->no, c->nv, s)); dst += (size_t)c->no * c->nv;
+    }
+    if (X) {
+      const long w = (long)c0->no + c0->nv;
+      XTD_TRY(copy_block(xout_dev, w, XO[0], c0->ldoo, c1->no, c0->no, s));
+      XTD_TRY(copy_block(xout_dev + c0->no, w, XO[1], c0->ldz, c1->no, c0->nv, s));
+      XTD_TRY(copy_block(xout_dev + (size_t)c1->no * w, w, XO[2], c0->ldoo, c1->nv, c0->no, s));
+      XTD_TRY(copy_block(xout_dev + (size_t)c1->no * w + c0->no, w, XO[3], c0->ldz, c1->nv, c0->nv, s));
+    }
+  }
+  if (h->ev_ok) cudaEventRecord(h->ev_total[1], s);
+  return XTD_OK;
 }

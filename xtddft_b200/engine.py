@@ -69,6 +69,8 @@ class SigmaEngine:
         self.exchange_slices = int(exchange_slices)
         if self.exchange_slices:
             _lib.check(self.lib.xtd_set_exchange_emulation(self._h, self.exchange_slices), "xtd_set_exchange_emulation")
+        if plan.block_response:
+            _lib.check(self.lib.xtd_enable_block_response(self._h), "xtd_enable_block_response")
         self.finalized = False
         self.max_nvec = 0
         self.ext_dim = int(plan.ext_dim)
@@ -360,6 +362,32 @@ class SigmaEngine:
                 self._ar_pending.append(ev)
                 _lib.check(self.lib.xtd_sigma_finish(self._h, x1 - x0, _ptr(oo)), "xtd_sigma_finish")
         return out
+
+    def block_response(self, dens: np.ndarray, coef, x: Optional[np.ndarray] = None):
+        """Responses of symmetric MO-block densities on the resident blocks (xtd_block_response; the plan needs `block_response`).
+        dens: per channel [Doo (no x no) | Dvv (nv x nv) | Dov (no x nv)] flattened on the channel's internal positions;
+        coef = (J, K tensor 0, K tensor 1, f_xc, K[X]).  Returns (per channel [Voo | Vov] flattened, K[X] on (channel-1 occ + vir) x
+        (channel-0 occ + vir) or None), summed over the ranks."""
+        torch = self.torch
+        assert self.finalized and self.plan.block_response
+        chs = self.plan.channels
+        d = torch.from_numpy(np.ascontiguousarray(dens, dtype=np.float64).ravel()).to(self.device)
+        assert d.numel() == sum(c.no * c.no + c.nv * c.nv + c.no * c.nv for c in chs)
+        out = torch.empty(sum(c.no * c.no + c.no * c.nv for c in chs), dtype=torch.float64, device=self.device)
+        c = np.ascontiguousarray(coef, dtype=np.float64)
+        assert c.shape == (5,)
+        xd = xo = None
+        if x is not None:
+            xd = torch.from_numpy(np.ascontiguousarray(x, dtype=np.float64).reshape(chs[1].no, chs[0].nv)).to(self.device)
+            xo = torch.empty((chs[1].no + chs[1].nv) * (chs[0].no + chs[0].nv), dtype=torch.float64, device=self.device)
+        self._set_stream()
+        _lib.check(self.lib.xtd_block_response(self._h, _ptr(d), _ptr(out), _np_ptr(c), _ptr(xd) if xd is not None else None,
+                                               _ptr(xo) if xo is not None else None), "xtd_block_response")
+        if self.reducer is not None and self.reducer.enabled:
+            self.reducer.allreduce_(out)
+            if xo is not None:
+                self.reducer.allreduce_(xo)
+        return out.cpu().numpy(), (xo.cpu().numpy() if xo is not None else None)
 
     def sigma_host(self, z: np.ndarray) -> np.ndarray:
         """Reference-facing entry with HOST vectors: H2D + sigma + D2H inside the C-ABI call (single rank)."""

@@ -130,6 +130,8 @@ class Plan:
     hdiag: Optional[np.ndarray] = None
     hdiag_needs_jdiag: Optional[dict] = None        # XSF: finish hdiag with J-block diagonals from the engine
     meta: dict = field(default_factory=dict)
+    # keep what xtd_block_response reads (Coulomb Loo / Lvv of every channel, fp64 virtual MO values on the grid) resident
+    block_response: bool = False
 
     def gather_map(self, ch: int) -> SparseMap:
         """ext -> internal block of channel `ch`, rows = i*nv_int + a."""

@@ -10,9 +10,10 @@ J/K build and one grid pass per iteration.  Here the operator is an engine plan 
 and Coulomb blocks, the MO-on-grid kernel contraction and the ROHF Fock couplings of the sigma path, plus the exchange of the
 transposed density (`xtd_add_kterm_t`); the Krylov vectors live in HBM and the subspace algebra runs in the `xtd_vec_*` kernels.
 
-The right-hand side (the Q matrix: J/K and f_xc images of occupied-occupied and virtual-virtual densities, third-derivative kernel
-for multicollinear functionals) is an INPUT here, as are the integral derivatives that follow the solve; both need pieces outside
-the sigma path (libcint derivative integrals, libxc third derivatives).
+The collinear right-hand side (the Q matrix: J/K and f_xc images of occupied-occupied and virtual-virtual densities) and the W matrix
+come from `xtd_block_response` on the same engine (`ZVector.rhs`, `ZVector.w_matrix`).  The third-derivative kernel of multicollinear
+functionals and the integral derivatives that follow the solve need pieces outside the sigma path (libxc third derivatives, libcint
+derivative integrals).
 """
 from __future__ import annotations
 
@@ -189,6 +190,95 @@ def assemble_w(p, z, inter: dict, apply_response_z):
     return ca @ (im0a + zeta_a * dm1a) @ ca.T + cb @ (im0b + zeta_b * dm1b) @ cb.T
 
 
+def _pos_idx(idx):
+    """(internal positions, MO indices) of the real orbitals of an index list (-1 = zero pad)."""
+    idx = np.asarray(idx)
+    pos = np.nonzero(idx >= 0)[0]
+    return pos, idx[pos]
+
+
+def mo_to_blocks(plan, t) -> np.ndarray:
+    """Symmetric MO-basis densities t[2, nmo, nmo] (one per spin) -> the `xtd_block_response` input: per channel of the two-channel plan
+    [Doo | Dvv | Dov] on the channel's internal positions.  Every channel's occupied and virtual sets together cover all orbitals of its
+    spin, so nothing of t is lost; t must be symmetric (the virtual-occupied block is the transpose of Dov)."""
+    t = np.asarray(t, dtype=np.float64)
+    if not np.allclose(t, t.transpose(0, 2, 1), rtol=0.0, atol=1e-13 * max(1.0, float(np.abs(t).max()))):
+        raise ValueError("mo_to_blocks: the densities must be symmetric")
+    parts = []
+    for ch in plan.channels:
+        assert ch.spin_o == ch.spin_v
+        m = t[ch.spin_o]
+        (op, oi), (vp, vi) = _pos_idx(ch.occ_idx), _pos_idx(ch.vir_idx)
+        for (rp, ri, nr), (cp, ci, ncol) in (((op, oi, ch.no), (op, oi, ch.no)), ((vp, vi, ch.nv), (vp, vi, ch.nv)),
+                                             ((op, oi, ch.no), (vp, vi, ch.nv))):
+            b = np.zeros((nr, ncol))
+            b[np.ix_(rp, cp)] = m[np.ix_(ri, ci)]
+            parts.append(b.ravel())
+    return np.concatenate(parts)
+
+
+def blocks_to_mo(plan, out, nmo: int) -> np.ndarray:
+    """`xtd_block_response` output (per channel [Voo | Vov]) -> [2, nmo, nmo] MO-basis response matrices with the occupied-occupied,
+    occupied-virtual and virtual-occupied blocks filled; the virtual-virtual block is not computed and is NaN."""
+    res = np.full((2, nmo, nmo), np.nan)
+    off = 0
+    for ch in plan.channels:
+        (op, oi), (vp, vi) = _pos_idx(ch.occ_idx), _pos_idx(ch.vir_idx)
+        voo = out[off:off + ch.no * ch.no].reshape(ch.no, ch.no)
+        off += ch.no * ch.no
+        vov = out[off:off + ch.no * ch.nv].reshape(ch.no, ch.nv)
+        off += ch.no * ch.nv
+        r = res[ch.spin_o]
+        r[np.ix_(oi, oi)] = voo[np.ix_(op, op)]
+        r[np.ix_(oi, vi)] = vov[np.ix_(op, vp)]
+        r[np.ix_(vi, oi)] = vov[np.ix_(op, vp)].T
+    return res
+
+
+def x_to_block(plan, x) -> np.ndarray:
+    """Mixed-spin density x[nmo_b, nmo_a] (rows: spin of channel 1, columns: spin of channel 0), nonzero only on (channel-1 occupied) x
+    (channel-0 virtual) -> the X block of `xtd_block_response`."""
+    c0, c1 = plan.channels
+    (op, oi), (vp, vi) = _pos_idx(c1.occ_idx), _pos_idx(c0.vir_idx)
+    blk = np.zeros((c1.no, c0.nv))
+    blk[np.ix_(op, vp)] = x[np.ix_(oi, vi)]
+    rest = np.array(x, dtype=np.float64, copy=True)
+    rest[np.ix_(oi, vi)] = 0.0
+    if np.any(rest != 0.0):
+        raise ValueError("x_to_block: the density has elements outside (channel-1 occupied) x (channel-0 virtual)")
+    return blk
+
+
+def xblock_to_mo(plan, xo, nmo: int) -> np.ndarray:
+    """K[X] on (channel-1 occupied + virtual) x (channel-0 occupied + virtual) -> [nmo_b, nmo_a]."""
+    c0, c1 = plan.channels
+    xo = np.asarray(xo).reshape(c1.no + c1.nv, c0.no + c0.nv)
+    rp, ri = _pos_idx(np.concatenate([c1.occ_idx, c1.vir_idx]))
+    cp, ci = _pos_idx(np.concatenate([c0.occ_idx, c0.vir_idx]))
+    res = np.zeros((nmo, nmo))
+    res[np.ix_(ri, ci)] = xo[np.ix_(rp, cp)]
+    return res
+
+
+def block_callables(p, plan, apply_blocks):
+    """The `apply_response` / `apply_sf_exchange` / `apply_response_z` callables of rhs_intermediates and assemble_w, computed by
+    `apply_blocks(dens, coef, x) -> (out, xout)` -- the `xtd_block_response` contract on the Z-vector operator plan's index sets
+    (alpha: [c|o] x v, beta: c x [o|v]) -- instead of whole-MO-space plans.  Coefficients (J, K full range, K long range, f_xc, K[X]):
+    the operator engine's kernel table carries the plan's `xc_scale`, which the f_xc coefficient takes back out."""
+    nmo = p.nmo
+    cxc = 1.0 / plan.xc_scale if plan.xc_kind != "none" else 0.0
+    ck0 = -p.hyb if p.hybrid else 0.0
+    ck1 = -(p.alpha - p.hyb) if (p.hybrid and p.omega != 0.0 and p.has_df_lr) else 0.0
+
+    def response(coef):
+        return lambda t: blocks_to_mo(plan, apply_blocks(mo_to_blocks(plan, t), coef, None)[0], nmo)
+
+    def sf_exchange(x):
+        return xblock_to_mo(plan, apply_blocks(mo_to_blocks(plan, np.zeros((2, nmo, nmo))), (0.0, 0.0, 0.0, 0.0, 1.0),
+                                               x_to_block(plan, x))[1], nmo)
+    return response((1.0, ck0, 0.0, cxc, 0.0)), (sf_exchange if p.hyb != 0.0 else None), response((1.0, ck0, ck1, cxc, 0.0))
+
+
 class ZVector:
     """Operator and solver of the Z-vector equation for one mean-field reference.
 
@@ -209,6 +299,7 @@ class ZVector:
         self.restricted = bool(p.restricted)
         self.nc, self.no, self.nv = p.nc, p.no, p.nv
         self.plan = planmod.build_zvector_plan(p, with_diag=with_diag)
+        self.plan.block_response = True         # rhs / w_matrix read the operator engine's resident blocks
         self.engine = make_engine(self.plan, p, max_nvec=max_nvec, workspace_bytes=workspace_bytes, distributed=distributed)
         self.hdiag = np.asarray(self.plan.hdiag)
         self.dim = int(self.plan.ext_dim)
@@ -241,20 +332,33 @@ class ZVector:
             self._rhs_engines = (resp, sfx, full)
         return self._rhs_engines
 
-    def rhs(self, v, workspace_bytes: Optional[int] = None):
-        """Right-hand side for the state with spin-flip-up amplitudes v[nc, nv] (collinear kernel), through two more engine plans on
-        the whole MO space (`assemble_rhs`); the engines are built on the first call and the intermediates kept for `w_matrix`.
-        CPU-verified against the reference's own right-hand sides through the plan interpreter (tests/test_zvector_cpu.py); first GPU
-        run pending (DESIGN section 8)."""
-        resp, sfx, _ = self._mo_engines(workspace_bytes)
-        self._inter = rhs_intermediates(self.problem, v, lambda t: resp.sigma_host(t.reshape(1, -1))[0],
-                                        (lambda x: sfx.sigma_host(x.reshape(1, -1))[0]) if sfx is not None else None)
-        return assemble_rhs(self.problem, v, None, None, inter=self._inter)
+    def rhs(self, v, workspace_bytes: Optional[int] = None, route: str = "blocks"):
+        """Right-hand side for the state with spin-flip-up amplitudes v[nc, nv] (collinear kernel); the intermediates are kept for
+        `w_matrix`.  route="blocks": the J / K / f_xc responses come from `xtd_block_response` on the operator engine's resident blocks
+        (no further engine, no whole-MO-space tensor).  route="mo_space": two or three more engines on whole-MO-space plans
+        (`_mo_engines`, built on the first call) -- a cross-check that needs naux x nmo^2 per spin."""
+        p = self.problem
+        if route == "blocks":
+            resp, sfx, _ = block_callables(p, self.plan, self.engine.block_response)
+        elif route == "mo_space":
+            r, x, _ = self._mo_engines(workspace_bytes)
+            resp = lambda t: r.sigma_host(t.reshape(1, -1))[0]
+            sfx = (lambda t: x.sigma_host(t.reshape(1, -1))[0]) if x is not None else None
+        else:
+            raise ValueError(f"route {route!r}: 'blocks' or 'mo_space'")
+        self._route = route
+        self._inter = rhs_intermediates(p, v, resp, sfx)
+        return assemble_rhs(p, v, None, None, inter=self._inter)
 
     def w_matrix(self, z):
-        """W matrix `im0` (AO basis) from the solution of the Z-vector equation of the state `rhs` was last called for (same status)."""
-        _, _, full = self._mo_engines()
-        return assemble_w(self.problem, z, self._inter, lambda t: full.sigma_host(t.reshape(1, -1))[0])
+        """W matrix `im0` (AO basis) from the solution of the Z-vector equation of the state `rhs` was last called for, on the same
+        route."""
+        if self._route == "blocks":
+            full = block_callables(self.problem, self.plan, self.engine.block_response)[2]
+        else:
+            f = self._mo_engines()[2]
+            full = lambda t: f.sigma_host(t.reshape(1, -1))[0]
+        return assemble_w(self.problem, z, self._inter, full)
 
     def split(self, z):
         """The rotation blocks the reference continues with: ROKS (zvc, zvo, zoc) (tdroks_sfu.py:328-330), UKS (z1a, z1b)."""
