@@ -151,6 +151,13 @@ int xtd_last_chunks(xtd_handle h, long* aux_chunks, long* grid_chunks);
  * occupied, virtual).  Outputs are this rank's partial sums (aux block, grid batch): all-reduce them over the ranks. */
 int xtd_enable_block_response(xtd_handle h);
 int xtd_block_response(xtd_handle h, const double* dens_dev, double* out_dev, const double* coef_host, const double* x_dev, double* xout_dev);
+/* The same for ndens densities with one coef: dens_dev, out_dev, x_dev and xout_dev hold ndens blocks of the xtd_block_response
+ * layout one after another.  Each aux chunk (and its decoded int8 Lvv) and each grid chunk is read once for all densities of a pass;
+ * when the workspace cannot hold every density at once (one aux function, one 128-point grid chunk) the call makes several passes,
+ * whose number xtd_last_density_batches reports. */
+int xtd_block_response_batch(xtd_handle h, int ndens, const double* dens_dev, double* out_dev, const double* coef_host,
+                             const double* x_dev, double* xout_dev);
+int xtd_last_density_batches(xtd_handle h, long* nbatches);
 
 /* Davidson subspace algebra on device vectors (Davidson.py:152-271): all row vectors of length n */
 int xtd_vec_dots(void* stream, double* g_dev, int ldg, const double* a_dev, long lda, int m, const double* b_dev, long ldb, int k, long n);

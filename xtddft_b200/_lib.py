@@ -72,6 +72,8 @@ SIGNATURES = {
     "xtd_last_chunks": (_I, [_P, C.POINTER(_L), C.POINTER(_L)]),
     "xtd_enable_block_response": (_I, [_P]),
     "xtd_block_response": (_I, [_P, _P, _P, _P, _P, _P]),
+    "xtd_block_response_batch": (_I, [_P, _I, _P, _P, _P, _P, _P]),
+    "xtd_last_density_batches": (_I, [_P, C.POINTER(_L)]),
     "xtd_vec_dots": (_I, [_P, _P, _I, _P, _L, _I, _P, _L, _I, _L]),
     "xtd_vec_lincomb": (_I, [_P, _P, _L, _P, _L, _P, _I, _I, _I, _L, _D]),
     "xtd_vec_residual": (_I, [_P, _P, _P, _P, _L, _P, _P, _I, _L]),

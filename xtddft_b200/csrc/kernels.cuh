@@ -732,6 +732,92 @@ __global__ void __launch_bounds__(256) xc_block_weight_kernel(const XcBlockArgs 
   }
 }
 
+// The same weighting for nd densities at once (xtd_block_response_batch).  Density x owns columns [x no_c, (x + 1) no_c) of Wo[c]
+// and [x nv_c, (x + 1) nv_c) of Wv[c] (ldWo / ldWv span all nd).  The kernel table row of a point is read once; the MO values of a
+// point once per group of KG densities, whose rho accumulators live in registers together.
+template <int NVAR, bool TAU, int KG>
+__global__ void __launch_bounds__(256) xc_block_weight_batch_kernel(const XcBlockArgs a, int nd) {
+  static_assert(!TAU || NVAR == 4, "the tau component needs value + gradient AO components");
+  const int lane = threadIdx.x & 31;
+  const long g = (long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (g >= a.gb) return;
+  constexpr int NK = TAU ? 5 : NVAR;
+  constexpr int NR = 2 * NK;
+  double fk[NR];
+  const double* row = a.wf + (a.g0 + g) * (long)(NR * NR);
+#pragma unroll
+  for (int q = 0; q < NR; ++q) fk[q] = (lane < NR) ? row[lane * NR + q] : 0.0;
+  for (int x0 = 0; x0 < nd; x0 += KG) {
+    const int nx = min(KG, nd - x0);
+    double rho[KG][NR];
+#pragma unroll
+    for (int x = 0; x < KG; ++x)
+#pragma unroll
+      for (int q = 0; q < NR; ++q) rho[x][q] = 0.0;
+#pragma unroll
+    for (int s = 0; s < 2; ++s) {
+      const long wcmp_o = (long)a.gb * a.ldWo[s], wcmp_v = (long)a.gb * a.ldWv[s];
+      for (int side = 0; side < 2; ++side) {
+        const int n = side ? a.nv[s] : a.no[s];
+        const double* p = side ? a.phiv[s] + (a.g0 + g) * a.ldphiv[s] : a.phi[s] + (a.g0 + g) * a.ldphi[s];
+        const long pc = side ? a.phiv_comp[s] : a.phi_comp[s];
+        const double* w = (side ? a.Wv[s] + g * a.ldWv[s] : a.Wo[s] + g * a.ldWo[s]) + (long)x0 * n;
+        const long wc = side ? wcmp_v : wcmp_o;
+        for (int o = lane; o < n; o += 32) {
+          double pv[NVAR];
+#pragma unroll
+          for (int k = 0; k < NVAR; ++k) pv[k] = p[k * pc + o];
+#pragma unroll
+          for (int x = 0; x < KG; ++x) {
+            if (x >= nx) break;
+            const double* wx = w + (long)x * n;
+            const double w0 = wx[o];
+            rho[x][s * NK] += pv[0] * w0;
+#pragma unroll
+            for (int k = 1; k < NVAR; ++k) {
+              rho[x][s * NK + k] += 2.0 * pv[k] * w0;
+              if (TAU) rho[x][s * NK + 4] += 0.5 * pv[k] * wx[k * wc + o];
+            }
+          }
+        }
+      }
+    }
+    double wv[KG][NR];
+#pragma unroll
+    for (int x = 0; x < KG; ++x) {
+      double mine = 0.0;
+#pragma unroll
+      for (int q = 0; q < NR; ++q) mine += fk[q] * warp_sum(rho[x][q]);
+#pragma unroll
+      for (int q = 0; q < NR; ++q) wv[x][q] = __shfl_sync(0xffffffffu, mine, q);
+    }
+#pragma unroll
+    for (int s = 0; s < 2; ++s) {
+      const int n = a.no[s];
+      double* w = a.Wo[s] + g * a.ldWo[s] + (long)x0 * n;
+      const long wc = (long)a.gb * a.ldWo[s];
+      const double* p = a.phi[s] + (a.g0 + g) * a.ldphi[s];
+      for (int o = lane; o < n; o += 32) {
+        double pv[NVAR];
+#pragma unroll
+        for (int k = 0; k < NVAR; ++k) pv[k] = p[k * a.phi_comp[s] + o];
+#pragma unroll
+        for (int x = 0; x < KG; ++x) {
+          if (x >= nx) break;
+          double* wx = w + (long)x * n;
+          double b0 = wv[x][s * NK] * pv[0];
+#pragma unroll
+          for (int k = 1; k < NVAR; ++k) {
+            b0 += wv[x][s * NK + k] * pv[k];
+            wx[k * wc + o] = wv[x][s * NK + k] * pv[0] + (TAU ? 0.5 * wv[x][s * NK + 4] * pv[k] : 0.0);
+          }
+          wx[o] = b0;
+        }
+      }
+    }
+  }
+}
+
 // ------------------------------------------------------------------------------------------------------
 // density-fitted Coulomb blocks
 // ------------------------------------------------------------------------------------------------------

@@ -237,6 +237,7 @@ struct xtd_engine {
   double phase_flops[12] = {0};   // GEMM flops per phase of the last call
   int oz_slices = 0;              // 0: FP64 DMMA exchange contraction; 3..8: INT8 tensor-core emulation with that many slices
   long last_aux_chunks = 0, last_grid_chunks = 0;
+  long last_dens_batches = 0;     // passes over the densities of the last xtd_block_response_batch (workspace-bound sub-batches)
   // Launch-bound calls (small molecules: ~50-100 launches of a few microseconds each) are replayed as CUDA graphs: the
   // first call with a given (nvec, z, hz) runs eagerly, the second is captured, later ones are one cudaGraphLaunch.
   struct GraphRec {
@@ -2957,6 +2958,299 @@ int copy_block(double* dst, long ldd, const double* src, long lds, int rows, int
   return XTD_OK;
 }
 
+// ---------------------------------------------------------------------------------------------------------
+// xtd_block_response_batch: kb densities per pass over the resident blocks.  Each aux chunk is read (and its int8 Lvv decoded) once
+// for all kb densities, and every GEMM carries the kb densities in one dimension:
+//   stage 1 (per P, rows stacked over the densities)  [A_1^T; ..; A_kb^T] = [Doo_1; ..] Loo + [Dov_1; ..] Lov^T
+//                                                      [B_1^T; ..; B_kb^T] = [Dov_1^T; ..] Loo + [Dvv_1; ..] Lov^T
+//   stored transposed through the two-level output rows, so that density x owns columns [x ldoo, x ldoo + no) of SA[P] / SB[P];
+//   stage 2 (sum over P, M = kb ldoo)  Ooo += SA^T Loo + SB^T Lov^T,  Oov += SA^T Lov + SB^T Lvv  with density x on rows x ldoo + i.
+// K[X] in the same way with U_x^T = X_x^T Loo1, V_x^T = X_x^T Lov1.  Row-stacked (_r) inputs put density x at row x n; the
+// column-stacked copies (_c) of Dov and X put it at column x nv.
+// ---------------------------------------------------------------------------------------------------------
+int mmx(xtd_engine* h, const MatView& A, bool akc, const MatView& B, bool bkc, int M, int N, int K, int nouter, int batches, int a_hi, int b_hi,
+        double* Cp, long ldc, long cbs, double alpha, bool acc, int row_div = 0, long row_hi = 0, long row_lo = 0) {
+  GemmDesc d;
+  d.A = A; d.B = B; d.a_kc = akc; d.b_kc = bkc; d.M = M; d.N = N; d.K = K; d.nouter = nouter;
+  d.batches = batches; d.z_div = 1; d.a_hi = a_hi; d.b_hi = b_hi;
+  d.C = Cp; d.ldc = ldc; d.c_batch_stride = cbs; d.alpha = alpha; d.accumulate = acc;
+  d.c_row_div = row_div; d.c_row_hi = row_hi; d.c_row_lo = row_lo;
+  return gemm(h->gemm, d, h->stream);
+}
+
+struct BatchBufs {
+  double *Doo_r, *Dvv_r, *Dov_r, *Dov_c;   // [kb no][ldoo], [kb nv][ldvv], [kb no][ldz], [no][ldc]
+  double *Ooo, *Oov;                       // [kb ldoo][ldoo], [kb ldoo][ldz]: density x from row x ldoo
+  long ldc;                                // pad_ld(kb nv)
+};
+struct BatchX {
+  double* X_c = nullptr;                   // [no1][ldx], density x at column x nv0
+  double* XO[4] = {nullptr, nullptr, nullptr, nullptr};   // oo, ov: density x from row x su;  vo, vv: from row x sv
+  long ldx = 0, su = 0, sv = 0;
+};
+
+// fixed buffers of a pass over kb densities; false when the arena cannot hold them
+bool batch_take(xtd_engine* h, Arena& ar, int kb, bool with_x, BatchBufs* bb, BatchX* bx) {
+  bool ok = true;
+  auto take = [&](size_t n) { double* p = ar.take(n); ok = ok && p; return p; };
+  for (int ci = 0; ci < 2; ++ci) {
+    Channel* c = h->ch[ci];
+    bb[ci].ldc = pad_ld((long)kb * c->nv);
+    bb[ci].Doo_r = take((size_t)kb * c->no * c->ldoo);
+    bb[ci].Dvv_r = take((size_t)kb * c->nv * c->ldvv);
+    bb[ci].Dov_r = take((size_t)kb * c->no * c->ldz);
+    bb[ci].Dov_c = take((size_t)c->no * bb[ci].ldc);
+    bb[ci].Ooo = take((size_t)kb * c->ldoo * c->ldoo);
+    bb[ci].Oov = take((size_t)kb * c->ldoo * c->ldz);
+  }
+  if (with_x) {
+    Channel *c0 = h->ch[0], *c1 = h->ch[1];
+    bx->ldx = pad_ld((long)kb * c0->nv);
+    bx->su = c1->ldoo;
+    bx->sv = c1->ldz;
+    bx->X_c = take((size_t)c1->no * bx->ldx);
+    bx->XO[0] = take((size_t)kb * bx->su * c0->ldoo);
+    bx->XO[1] = take((size_t)kb * bx->su * c0->ldz);
+    bx->XO[2] = take((size_t)kb * bx->sv * c0->ldoo);
+    bx->XO[3] = take((size_t)kb * bx->sv * c0->ldz);
+  }
+  return ok;
+}
+
+// per aux function scratch of tensor t for kb densities (SA, SB, decoded Lvv per channel; SU, SV; rho rows)
+size_t batch_per_aux(const xtd_engine* h, int t, int kb, bool doX) {
+  size_t per_p = 8 * (size_t)kb + 64;
+  for (int ci = 0; ci < 2; ++ci) {
+    const Channel* c = h->ch[ci];
+    per_p += (size_t)(c->no + c->nv) * kb * c->ldoo + (c->use_oz[t] ? (size_t)c->nv * c->ldvv : 0) + 96;
+  }
+  if (doX) {
+    const Channel *c0 = h->ch[0], *c1 = h->ch[1];
+    per_p += (size_t)c0->nv * kb * (c1->ldoo + c1->ldz) + 64;
+  }
+  return per_p;
+}
+
+size_t batch_per_point(const xtd_engine* h, int kb) {
+  size_t per_g = 0;
+  for (auto* c : h->ch) per_g += (size_t)h->nvar_eff * (pad_ld((long)kb * c->no) + pad_ld((long)kb * c->nv));
+  return per_g;
+}
+
+int block_response_batch_df(xtd_engine* h, int kb, const BatchBufs* bb, const double* coef, const BatchX* bx, double* scratch,
+                            size_t scratch_doubles) {
+  cudaStream_t s = h->stream;
+  const double cj = coef[0], cx = coef[4];
+  Channel *c0 = h->ch[0], *c1 = h->ch[1];
+  for (int t = 0; t < 2; ++t) {
+    const double ck = coef[1 + t];
+    const bool doJ = t == 0 && cj != 0.0, doK = ck != 0.0, doX = t == 0 && bx->X_c && cx != 0.0;
+    if (!(doJ || doK || doX) || h->naux[t] == 0) continue;
+    const long naux = h->naux[t];
+    const double* Lov[2];
+    long ldov[2];
+    for (int ci = 0; ci < 2; ++ci) {
+      Channel* c = h->ch[ci];
+      Lov[ci] = ov_block(h, ci, t, &ldov[ci]);
+      XTD_REQUIRE(oovv_resident(h, c, t) && Lov[ci], XTD_ERR_STATE,
+                  "xtd_block_response_batch: channel %d holds no MO blocks of tensor %d (call xtd_enable_block_response before xtd_df_begin)",
+                  ci, t);
+      XTD_REQUIRE(!c->use_oz[t] || c->oz_col0[t] == 0, XTD_ERR_UNSUPPORTED, "xtd_block_response_batch: block-weighted emulated exchange image");
+    }
+    long pc = (long)(scratch_doubles / batch_per_aux(h, t, kb, doX));
+    if (h->env.max_pc > 0) pc = std::min<long>(pc, h->env.max_pc);
+    pc = std::min<long>(pc, naux);
+    XTD_REQUIRE(pc >= 1, XTD_ERR_NOMEM, "xtd_block_response_batch: workspace too small for one aux function");
+    double* cur = scratch;
+    auto take = [&](size_t n) { double* p = cur; cur += (n + 31) & ~(size_t)31; return p; };
+    double *SA[2], *SB[2], *Ldec[2] = {nullptr, nullptr};
+    long ldS[2], sSA[2], sSB[2];
+    for (int ci = 0; ci < 2; ++ci) {
+      Channel* c = h->ch[ci];
+      ldS[ci] = (long)kb * c->ldoo;
+      sSA[ci] = (long)c->no * ldS[ci];
+      sSB[ci] = (long)c->nv * ldS[ci];
+      SA[ci] = take((size_t)pc * sSA[ci]);
+      SB[ci] = take((size_t)pc * sSB[ci]);
+      if (c->use_oz[t]) Ldec[ci] = take((size_t)pc * c->nv * c->ldvv);
+    }
+    const long ldU = (long)kb * bx->su, ldV = (long)kb * bx->sv, sSU = (long)c0->nv * ldU, sSV = (long)c0->nv * ldV;
+    double* SU = doX ? take((size_t)pc * sSU) : nullptr;
+    double* SV = doX ? take((size_t)pc * sSV) : nullptr;
+    // the stage-1 GEMMs write only the live columns of each density's slot: the padding between slots stays zero
+    XTD_CUDA(cudaMemsetAsync(scratch, 0, (size_t)(cur - scratch) * 8, s));
+    double* R = take((size_t)6 * kb * pc);
+    double* rho = take((size_t)kb * pc);
+    h->last_aux_chunks = std::max<long>(h->last_aux_chunks, cdiv(naux, pc));
+    for (long P0 = 0; P0 < naux; P0 += pc) {
+      const int pn = (int)std::min<long>(pc, naux - P0);
+      const double *Loo[2], *Lvv[2], *Lo[2];
+      for (int ci = 0; ci < 2; ++ci) {
+        Channel* c = h->ch[ci];
+        Loo[ci] = c->Loo[t].p + P0 * c->no * c->ldoo;
+        Lo[ci] = Lov[ci] + P0 * c->no * ldov[ci];
+        if (c->use_oz[t]) {
+          PhaseTimer tm(h, XTD_T_K2_SLICE);
+          oz_unslice_b_kernel<<<dim3((unsigned)cdiv((long)c->nv * c->nv, 256), pn), 256, 0, s>>>(
+              Ldec[ci], c->ldvv, (long)c->nv * c->ldvv, c->LvvS[t], c->LvvScale[t], h->oz_slices, c->nv, c->ozB.rows_pad, c->nv, c->ozB.nkb,
+              c->oz_group, P0, pn);
+          LAUNCH_CHECK();
+          Lvv[ci] = Ldec[ci];
+        } else {
+          Lvv[ci] = c->Lvv[t].p + P0 * c->nv * c->ldvv;
+        }
+      }
+      if (doJ) {
+        PhaseTimer tm(h, XTD_T_J);
+        // R[blk][x][P] for the six blocks (Doo, Dvv, Dov of each channel); rho[x][P]; every L element read once per 4 densities
+        for (int ci = 0; ci < 2; ++ci) {
+          Channel* c = h->ch[ci];
+          j_rho_kernel<4><<<pn, 256, 0, s>>>(R + (size_t)(3 * ci) * kb * pc, pc, Loo[ci], c->ldoo, (long)c->no * c->ldoo, bb[ci].Doo_r, c->ldoo,
+                                             (long)c->no * c->ldoo, c->no, c->no, kb);
+          LAUNCH_CHECK();
+          j_rho_kernel<4><<<pn, 256, 0, s>>>(R + (size_t)(3 * ci + 1) * kb * pc, pc, Lvv[ci], c->ldvv, (long)c->nv * c->ldvv, bb[ci].Dvv_r, c->ldvv,
+                                             (long)c->nv * c->ldvv, c->nv, c->nv, kb);
+          LAUNCH_CHECK();
+          j_rho_kernel<4><<<pn, 256, 0, s>>>(R + (size_t)(3 * ci + 2) * kb * pc, pc, Lo[ci], ldov[ci], (long)c->no * ldov[ci], bb[ci].Dov_r, c->ldz,
+                                             (long)c->no * c->ldz, c->no, c->nv, kb);
+          LAUNCH_CHECK();
+        }
+        RhoWeights w = {{cj, cj, 2.0 * cj, cj, cj, 2.0 * cj}};
+        rho_combine_kernel<<<grid1d((long)kb * pc, 256), 256, 0, s>>>(rho, R, (long)kb * pc, 6, (long)kb * pc, w);
+        LAUNCH_CHECK();
+        for (int ci = 0; ci < 2; ++ci) {
+          Channel* c = h->ch[ci];
+          j_apply_kernel<4><<<dim3((unsigned)cdiv((long)c->no * c->no, 256), (unsigned)cdiv(kb, 4)), 256, 0, s>>>(
+              bb[ci].Ooo, c->ldoo, (long)c->ldoo * c->ldoo, Loo[ci], c->ldoo, (long)c->no * c->ldoo, rho, pc, pn, c->no, c->no, kb);
+          LAUNCH_CHECK();
+          j_apply_kernel<4><<<dim3((unsigned)cdiv((long)c->no * c->nv, 256), (unsigned)cdiv(kb, 4)), 256, 0, s>>>(
+              bb[ci].Oov, c->ldz, (long)c->ldoo * c->ldz, Lo[ci], ldov[ci], (long)c->no * ldov[ci], rho, pc, pn, c->no, c->nv, kb);
+          LAUNCH_CHECK();
+        }
+      }
+      if (doK)
+        for (int ci = 0; ci < 2; ++ci) {
+          Channel* c = h->ch[ci];
+          const int no = c->no, nv = c->nv, Mo = (kb - 1) * c->ldoo + no;
+          const long soo = (long)no * c->ldoo, sov = (long)no * ldov[ci], svv = (long)nv * c->ldvv;
+          const MatView LooV = view3d(Loo[ci], c->ldoo, soo, pn, no, no), LovV = view3d(Lo[ci], ldov[ci], sov, pn, no, nv);
+          {
+            PhaseTimer tm(h, XTD_T_K1);
+            XTD_TRY(mmx(h, view2d(bb[ci].Doo_r, c->ldoo, kb * no, no), true, LooV, false, kb * no, no, no, 1, pn, 0, 1, SA[ci], ldS[ci], sSA[ci], 1.0,
+                        false, no, c->ldoo, ldS[ci]));
+            XTD_TRY(mmx(h, view2d(bb[ci].Dov_r, c->ldz, kb * no, nv), true, LovV, true, kb * no, no, nv, 1, pn, 0, 1, SA[ci], ldS[ci], sSA[ci], 1.0,
+                        true, no, c->ldoo, ldS[ci]));
+            XTD_TRY(mmx(h, view2d(bb[ci].Dov_c, bb[ci].ldc, no, kb * nv), false, LooV, false, kb * nv, no, no, 1, pn, 0, 1, SB[ci], ldS[ci], sSB[ci],
+                        1.0, false, nv, c->ldoo, ldS[ci]));
+            XTD_TRY(mmx(h, view2d(bb[ci].Dvv_r, c->ldvv, kb * nv, nv), true, LovV, true, kb * nv, no, nv, 1, pn, 0, 1, SB[ci], ldS[ci], sSB[ci], 1.0,
+                        true, nv, c->ldoo, ldS[ci]));
+          }
+          PhaseTimer tm(h, XTD_T_K2);
+          const MatView Av = view3d(SA[ci], ldS[ci], sSA[ci], pn, no, Mo), Bv = view3d(SB[ci], ldS[ci], sSB[ci], pn, nv, Mo);
+          XTD_TRY(mmx(h, Av, false, LooV, false, Mo, no, no, pn, 1, 0, 0, bb[ci].Ooo, c->ldoo, 0, ck, true));
+          XTD_TRY(mmx(h, Bv, false, LovV, true, Mo, no, nv, pn, 1, 0, 0, bb[ci].Ooo, c->ldoo, 0, ck, true));
+          XTD_TRY(mmx(h, Av, false, LovV, false, Mo, nv, no, pn, 1, 0, 0, bb[ci].Oov, c->ldz, 0, ck, true));
+          XTD_TRY(mmx(h, Bv, false, view3d(Lvv[ci], c->ldvv, svv, pn, nv, nv), false, Mo, nv, nv, pn, 1, 0, 0, bb[ci].Oov, c->ldz, 0, ck, true));
+        }
+      if (doX) {
+        const int no1 = c1->no, nv1 = c1->nv, no0 = c0->no, nv0 = c0->nv;
+        const int Mu = (kb - 1) * (int)bx->su + no1, Mv = (kb - 1) * (int)bx->sv + nv1;
+        const MatView Xv = view2d(bx->X_c, bx->ldx, no1, kb * nv0);
+        {
+          PhaseTimer tm(h, XTD_T_K1);
+          XTD_TRY(mmx(h, Xv, false, view3d(Loo[1], c1->ldoo, (long)no1 * c1->ldoo, pn, no1, no1), false, kb * nv0, no1, no1, 1, pn, 0, 1, SU, ldU,
+                      sSU, 1.0, false, nv0, bx->su, ldU));
+          XTD_TRY(mmx(h, Xv, false, view3d(Lo[1], ldov[1], (long)no1 * ldov[1], pn, no1, nv1), false, kb * nv0, nv1, no1, 1, pn, 0, 1, SV, ldV,
+                      sSV, 1.0, false, nv0, bx->sv, ldV));
+        }
+        PhaseTimer tm(h, XTD_T_K2);
+        const MatView Uv = view3d(SU, ldU, sSU, pn, nv0, Mu), Vv = view3d(SV, ldV, sSV, pn, nv0, Mv);
+        const MatView Lov0 = view3d(Lo[0], ldov[0], (long)no0 * ldov[0], pn, no0, nv0);
+        const MatView Lvv0 = view3d(Lvv[0], c0->ldvv, (long)nv0 * c0->ldvv, pn, nv0, nv0);
+        XTD_TRY(mmx(h, Uv, false, Lov0, true, Mu, no0, nv0, pn, 1, 0, 0, bx->XO[0], c0->ldoo, 0, cx, true));
+        XTD_TRY(mmx(h, Uv, false, Lvv0, false, Mu, nv0, nv0, pn, 1, 0, 0, bx->XO[1], c0->ldz, 0, cx, true));
+        XTD_TRY(mmx(h, Vv, false, Lov0, true, Mv, no0, nv0, pn, 1, 0, 0, bx->XO[2], c0->ldoo, 0, cx, true));
+        XTD_TRY(mmx(h, Vv, false, Lvv0, false, Mv, nv0, nv0, pn, 1, 0, 0, bx->XO[3], c0->ldz, 0, cx, true));
+      }
+    }
+  }
+  return XTD_OK;
+}
+
+// grid term for kb densities: Wo = phi [Doo_1 ..] + phiv [Dov_1^T ..],  Wv = phiv [Dvv_1 ..] + phi [Dov_1 ..] (density x at column
+// x no / x nv), xc_block_weight_batch_kernel, then  Ooo_x += c_xc sum_c Bo_x^T phi_c,  Oov_x += c_xc sum_c Bo_x^T phiv_c  as one GEMM
+// each with M = kb no (output rows placed at x ldoo + i)
+int block_response_batch_xc(xtd_engine* h, int kb, const BatchBufs* bb, double cxc, double* scratch, size_t scratch_doubles) {
+  cudaStream_t s = h->stream;
+  XTD_REQUIRE(h->fxc_kind == XTD_FXC_UKS, XTD_ERR_UNSUPPORTED, "xtd_block_response_batch: the grid term needs the UKS kernel tables");
+  const int nve = h->nvar_eff, nf = h->tau ? 4 : 1;
+  for (auto* c : h->ch)
+    XTD_REQUIRE(c->phiv.p && c->phi.p, XTD_ERR_STATE,
+                "xtd_block_response_batch: fp64 virtual MO values not kept on the grid (call xtd_enable_block_response before the grid commit)");
+  long ldWo[2], ldWv[2];
+  for (int ci = 0; ci < 2; ++ci) {
+    ldWo[ci] = pad_ld((long)kb * h->ch[ci]->no);
+    ldWv[ci] = pad_ld((long)kb * h->ch[ci]->nv);
+  }
+  long GB = (long)(scratch_doubles / batch_per_point(h, kb)) - 64;
+  GB = std::min<long>(GB, 1 << 16);
+  if (h->env.max_gb > 0) GB = std::min<long>(GB, std::max<long>(h->env.max_gb, 128));
+  GB = (GB / 128) * 128;
+  XTD_REQUIRE(GB >= 128, XTD_ERR_NOMEM, "xtd_block_response_batch: workspace too small for a 128-point grid chunk");
+  h->last_grid_chunks = std::max<long>(h->last_grid_chunks, cdiv(h->ng, GB));
+  for (long g0 = 0; g0 < h->ng; g0 += GB) {
+    const int gb = (int)std::min<long>(GB, h->ng - g0);
+    double *Wo[2], *Wv[2];
+    double* cur = scratch;
+    for (int ci = 0; ci < 2; ++ci) {
+      Wo[ci] = cur; cur += (size_t)nve * gb * ldWo[ci];
+      Wv[ci] = cur; cur += (size_t)nve * gb * ldWv[ci];
+    }
+    {
+      PhaseTimer tm(h, XTD_T_XC_GEMM);
+      for (int ci = 0; ci < 2; ++ci) {
+        Channel* c = h->ch[ci];
+        const int no = c->no, nv = c->nv;
+        const MatView ph = view3d(c->phi.p, c->ldphi, h->ng * c->ldphi, nf, gb, no, (int)g0, 0);
+        const MatView pv = view3d(c->phiv.p, c->ldphiv, h->ng * c->ldphiv, nf, gb, nv, (int)g0, 0);
+        const long so = (long)gb * ldWo[ci], sv = (long)gb * ldWv[ci];
+        XTD_TRY(mm(h, ph, true, view2d(bb[ci].Doo_r, c->ldoo, kb * no, no), true, gb, kb * no, no, 1, nf, Wo[ci], ldWo[ci], so, 1.0, false));
+        XTD_TRY(mm(h, pv, true, view2d(bb[ci].Dov_r, c->ldz, kb * no, nv), true, gb, kb * no, nv, 1, nf, Wo[ci], ldWo[ci], so, 1.0, true));
+        XTD_TRY(mm(h, pv, true, view2d(bb[ci].Dvv_r, c->ldvv, kb * nv, nv), true, gb, kb * nv, nv, 1, nf, Wv[ci], ldWv[ci], sv, 1.0, false));
+        XTD_TRY(mm(h, ph, true, view2d(bb[ci].Dov_c, bb[ci].ldc, no, kb * nv), false, gb, kb * nv, no, 1, nf, Wv[ci], ldWv[ci], sv, 1.0, true));
+      }
+    }
+    {
+      PhaseTimer tm(h, XTD_T_XC_STREAM);
+      XcBlockArgs a;
+      a.gb = gb; a.g0 = g0; a.wf = h->wf.p;
+      for (int ci = 0; ci < 2; ++ci) {
+        Channel* c = h->ch[ci];
+        a.Wo[ci] = Wo[ci]; a.Wv[ci] = Wv[ci]; a.ldWo[ci] = ldWo[ci]; a.ldWv[ci] = ldWv[ci];
+        a.phi[ci] = c->phi.p; a.phiv[ci] = c->phiv.p; a.ldphi[ci] = c->ldphi; a.ldphiv[ci] = c->ldphiv;
+        a.phi_comp[ci] = h->ng * c->ldphi; a.phiv_comp[ci] = h->ng * c->ldphiv;
+        a.no[ci] = c->no; a.nv[ci] = c->nv;
+      }
+      const unsigned grid = (unsigned)cdiv(gb, 8);
+      if (nve == 1) xc_block_weight_batch_kernel<1, false, 4><<<grid, 256, 0, s>>>(a, kb);
+      else if (h->tau) xc_block_weight_batch_kernel<4, true, 4><<<grid, 256, 0, s>>>(a, kb);
+      else xc_block_weight_batch_kernel<4, false, 4><<<grid, 256, 0, s>>>(a, kb);
+      LAUNCH_CHECK();
+    }
+    PhaseTimer tm(h, XTD_T_XC_GEMM);
+    for (int ci = 0; ci < 2; ++ci) {
+      Channel* c = h->ch[ci];
+      const int no = c->no, nv = c->nv;
+      const MatView Bo = view3d(Wo[ci], ldWo[ci], (long)gb * ldWo[ci], nve, gb, kb * no);
+      XTD_TRY(mmx(h, Bo, false, view3d(c->phi.p, c->ldphi, h->ng * c->ldphi, nve, gb, no, (int)g0, 0), false, kb * no, no, gb, nve, 1, 0, 0,
+                  bb[ci].Ooo, c->ldoo, 0, cxc, true, no, (long)c->ldoo * c->ldoo, c->ldoo));
+      XTD_TRY(mmx(h, Bo, false, view3d(c->phiv.p, c->ldphiv, h->ng * c->ldphiv, nve, gb, nv, (int)g0, 0), false, kb * no, nv, gb, nve, 1, 0, 0,
+                  bb[ci].Oov, c->ldz, 0, cxc, true, no, (long)c->ldoo * c->ldz, c->ldz));
+    }
+  }
+  return XTD_OK;
+}
+
 }  // namespace
 
 extern "C" int xtd_enable_block_response(xtd_handle h) {
@@ -3036,5 +3330,105 @@ extern "C" int xtd_block_response(xtd_handle h, const double* dens_dev, double* 
     }
   }
   if (h->ev_ok) cudaEventRecord(h->ev_total[1], s);
+  return XTD_OK;
+}
+
+extern "C" int xtd_block_response_batch(xtd_handle h, int ndens, const double* dens_dev, double* out_dev, const double* coef_host,
+                                        const double* x_dev, double* xout_dev) {
+  XTD_REQUIRE(h && h->finalized, XTD_ERR_STATE, "xtd_block_response_batch before xtd_finalize");
+  XTD_REQUIRE(ndens >= 1 && dens_dev && out_dev && coef_host && (!x_dev || xout_dev), XTD_ERR_ARG, "xtd_block_response_batch: bad arguments");
+  XTD_REQUIRE(h->ch.size() == 2, XTD_ERR_UNSUPPORTED, "xtd_block_response_batch needs a two-channel plan");
+  cudaStream_t s = h->stream;
+  h->ev_used = 0;
+  for (int i = 0; i < 12; ++i) h->phase_flops[i] = 0.0;
+  h->last_aux_chunks = h->last_grid_chunks = 0;
+  if (h->ev_ok) cudaEventRecord(h->ev_total[0], s);
+  Channel *c0 = h->ch[0], *c1 = h->ch[1];
+  const bool with_x = x_dev != nullptr;
+  const bool doxc = coef_host[3] != 0.0 && h->fxc_kind != XTD_FXC_NONE && h->ng > 0;
+  size_t nin = 0, nout = 0;
+  for (auto* c : h->ch) {
+    nin += (size_t)c->no * c->no + (size_t)c->nv * c->nv + (size_t)c->no * c->nv;
+    nout += (size_t)c->no * c->no + (size_t)c->no * c->nv;
+  }
+  const size_t nxin = (size_t)c1->no * c0->nv, nxout = (size_t)(c1->no + c1->nv) * (c0->no + c0->nv);
+  // densities per pass: the largest kb (of ceil(ndens / n) for n = 1, 2, ..) whose fixed buffers, split-K partials and one aux function
+  // / one 128-point grid chunk of scratch fit the workspace; the passes are counted in last_dens_batches
+  int kb = 0;
+  for (int n = 1; n <= ndens && !kb; ++n) {
+    const int k = (int)cdiv(ndens, n);
+    if (n > 1 && k == (int)cdiv(ndens, n - 1)) continue;
+    Arena ar = h->arena;
+    ar.used = 0;
+    BatchBufs bb[2];
+    BatchX bx;
+    if (!batch_take(h, ar, k, with_x, bb, &bx)) continue;
+    const size_t left = ar.left() - std::min<size_t>(ar.left() / 4, (size_t)1 << 30);
+    const size_t scratch = left / 8 > 64 + 512 ? left / 8 - 64 - 512 : 0;
+    bool fits = true;
+    for (int t = 0; t < 2; ++t)
+      if (h->naux[t] > 0) fits = fits && scratch >= batch_per_aux(h, t, k, with_x && t == 0);
+    if (doxc) fits = fits && (long)(scratch / batch_per_point(h, k)) - 64 >= 128;
+    if (fits) kb = k;
+  }
+  XTD_REQUIRE(kb >= 1, XTD_ERR_NOMEM, "xtd_block_response_batch: workspace too small for one density");
+  h->last_dens_batches = cdiv(ndens, kb);
+  for (int x0 = 0; x0 < ndens; x0 += kb) {
+    const int nb = std::min(kb, ndens - x0);
+    h->arena.used = 0;
+    BatchBufs bb[2];
+    BatchX bx;
+    XTD_REQUIRE(batch_take(h, h->arena, nb, with_x, bb, &bx), XTD_ERR_NOMEM, "xtd_block_response_batch: workspace exhausted");
+    const size_t fixed = h->arena.used;
+    {
+      PhaseTimer tm(h, XTD_T_PACK);
+      XTD_CUDA(cudaMemsetAsync(h->arena.base, 0, fixed, s));
+      for (int x = 0; x < nb; ++x) {
+        const double* src = dens_dev + (size_t)(x0 + x) * nin;
+        for (int ci = 0; ci < 2; ++ci) {
+          Channel* c = h->ch[ci];
+          XTD_TRY(copy_block(bb[ci].Doo_r + (size_t)x * c->no * c->ldoo, c->ldoo, src, c->no, c->no, c->no, s)); src += (size_t)c->no * c->no;
+          XTD_TRY(copy_block(bb[ci].Dvv_r + (size_t)x * c->nv * c->ldvv, c->ldvv, src, c->nv, c->nv, c->nv, s)); src += (size_t)c->nv * c->nv;
+          XTD_TRY(copy_block(bb[ci].Dov_r + (size_t)x * c->no * c->ldz, c->ldz, src, c->nv, c->no, c->nv, s));
+          XTD_TRY(copy_block(bb[ci].Dov_c + (size_t)x * c->nv, bb[ci].ldc, src, c->nv, c->no, c->nv, s)); src += (size_t)c->no * c->nv;
+        }
+        if (with_x) XTD_TRY(copy_block(bx.X_c + (size_t)x * c0->nv, bx.ldx, x_dev + (size_t)(x0 + x) * nxin, c0->nv, c1->no, c0->nv, s));
+      }
+    }
+    size_t split_bytes = std::min<size_t>(h->arena.left() / 4, (size_t)1 << 30);
+    h->gemm.split_ws = h->arena.take(split_bytes / 8);
+    h->gemm.split_ws_bytes = split_bytes;
+    const size_t scratch_doubles = h->arena.left() / 8 - 64;
+    double* scratch = h->arena.take(scratch_doubles);
+    XTD_REQUIRE(scratch, XTD_ERR_NOMEM, "xtd_block_response_batch: workspace exhausted (chunk scratch)");
+    XTD_TRY(block_response_batch_df(h, nb, bb, coef_host, &bx, scratch, scratch_doubles));
+    if (doxc) XTD_TRY(block_response_batch_xc(h, nb, bb, coef_host[3], scratch, scratch_doubles));
+    {
+      PhaseTimer tm(h, XTD_T_UNPACK);
+      for (int x = 0; x < nb; ++x) {
+        double* dst = out_dev + (size_t)(x0 + x) * nout;
+        for (int ci = 0; ci < 2; ++ci) {
+          Channel* c = h->ch[ci];
+          XTD_TRY(copy_block(dst, c->no, bb[ci].Ooo + (size_t)x * c->ldoo * c->ldoo, c->ldoo, c->no, c->no, s)); dst += (size_t)c->no * c->no;
+          XTD_TRY(copy_block(dst, c->nv, bb[ci].Oov + (size_t)x * c->ldoo * c->ldz, c->ldz, c->no, c->nv, s)); dst += (size_t)c->no * c->nv;
+        }
+        if (with_x) {
+          const long w = (long)c0->no + c0->nv;
+          double* xo = xout_dev + (size_t)(x0 + x) * nxout;
+          XTD_TRY(copy_block(xo, w, bx.XO[0] + (size_t)x * bx.su * c0->ldoo, c0->ldoo, c1->no, c0->no, s));
+          XTD_TRY(copy_block(xo + c0->no, w, bx.XO[1] + (size_t)x * bx.su * c0->ldz, c0->ldz, c1->no, c0->nv, s));
+          XTD_TRY(copy_block(xo + (size_t)c1->no * w, w, bx.XO[2] + (size_t)x * bx.sv * c0->ldoo, c0->ldoo, c1->nv, c0->no, s));
+          XTD_TRY(copy_block(xo + (size_t)c1->no * w + c0->no, w, bx.XO[3] + (size_t)x * bx.sv * c0->ldz, c0->ldz, c1->nv, c0->nv, s));
+        }
+      }
+    }
+  }
+  if (h->ev_ok) cudaEventRecord(h->ev_total[1], s);
+  return XTD_OK;
+}
+
+extern "C" int xtd_last_density_batches(xtd_handle h, long* nbatches) {
+  XTD_REQUIRE(h && nbatches, XTD_ERR_ARG, "xtd_last_density_batches: bad arguments");
+  *nbatches = h->last_dens_batches;
   return XTD_OK;
 }

@@ -367,27 +367,56 @@ class SigmaEngine:
         """Responses of symmetric MO-block densities on the resident blocks (xtd_block_response; the plan needs `block_response`).
         dens: per channel [Doo (no x no) | Dvv (nv x nv) | Dov (no x nv)] flattened on the channel's internal positions;
         coef = (J, K tensor 0, K tensor 1, f_xc, K[X]).  Returns (per channel [Voo | Vov] flattened, K[X] on (channel-1 occ + vir) x
-        (channel-0 occ + vir) or None), summed over the ranks."""
+        (channel-0 occ + vir) or None), summed over the ranks.
+
+        Several densities at once: dens[k, n] and x[k, no_1, nv_0] (or [k, no_1 * nv_0]) with one coef; the outputs gain the same
+        leading axis.  One xtd_block_response_batch call reads the resident blocks once per pass for all k densities, and with several
+        ranks the whole batch is all-reduced once."""
         torch = self.torch
         assert self.finalized and self.plan.block_response
         chs = self.plan.channels
-        d = torch.from_numpy(np.ascontiguousarray(dens, dtype=np.float64).ravel()).to(self.device)
-        assert d.numel() == sum(c.no * c.no + c.nv * c.nv + c.no * c.nv for c in chs)
-        out = torch.empty(sum(c.no * c.no + c.no * c.nv for c in chs), dtype=torch.float64, device=self.device)
+        nin = sum(c.no * c.no + c.nv * c.nv + c.no * c.nv for c in chs)
+        nout = sum(c.no * c.no + c.no * c.nv for c in chs)
+        nxin, nxout = chs[1].no * chs[0].nv, (chs[1].no + chs[1].nv) * (chs[0].no + chs[0].nv)
+        dens = np.ascontiguousarray(dens, dtype=np.float64)
+        batched = dens.ndim == 2
+        if dens.ndim not in (1, 2) or dens.shape[-1] != nin:
+            raise ValueError(f"block_response: dens must be [{nin}] or [k, {nin}], got {dens.shape}")
+        k = dens.shape[0] if batched else 1
+        if k == 0:
+            raise ValueError("block_response: empty batch")
+        d = torch.from_numpy(dens.ravel()).to(self.device)
         c = np.ascontiguousarray(coef, dtype=np.float64)
         assert c.shape == (5,)
-        xd = xo = None
+        # one buffer for the responses and K[X]: a single all-reduce per call
+        res = torch.empty(k * (nout + (nxout if x is not None else 0)), dtype=torch.float64, device=self.device)
+        out, xo = res[:k * nout], None
+        xd = None
         if x is not None:
-            xd = torch.from_numpy(np.ascontiguousarray(x, dtype=np.float64).reshape(chs[1].no, chs[0].nv)).to(self.device)
-            xo = torch.empty((chs[1].no + chs[1].nv) * (chs[0].no + chs[0].nv), dtype=torch.float64, device=self.device)
+            xh = np.ascontiguousarray(x, dtype=np.float64)
+            if xh.size != k * nxin or (batched and xh.shape[0] != k):
+                raise ValueError(f"block_response: x must hold {k} blocks of {chs[1].no} x {chs[0].nv}, got {xh.shape}")
+            xd = torch.from_numpy(xh.ravel()).to(self.device)
+            xo = res[k * nout:]
         self._set_stream()
-        _lib.check(self.lib.xtd_block_response(self._h, _ptr(d), _ptr(out), _np_ptr(c), _ptr(xd) if xd is not None else None,
-                                               _ptr(xo) if xo is not None else None), "xtd_block_response")
+        xp, xop = (_ptr(xd), _ptr(xo)) if xd is not None else (None, None)
+        if batched:
+            _lib.check(self.lib.xtd_block_response_batch(self._h, k, _ptr(d), _ptr(out), _np_ptr(c), xp, xop), "xtd_block_response_batch")
+        else:
+            _lib.check(self.lib.xtd_block_response(self._h, _ptr(d), _ptr(out), _np_ptr(c), xp, xop), "xtd_block_response")
         if self.reducer is not None and self.reducer.enabled:
-            self.reducer.allreduce_(out)
-            if xo is not None:
-                self.reducer.allreduce_(xo)
-        return out.cpu().numpy(), (xo.cpu().numpy() if xo is not None else None)
+            self.reducer.allreduce_(res)
+        res = res.cpu().numpy()
+        out, xo = res[:k * nout], (res[k * nout:] if x is not None else None)
+        if batched:
+            return out.reshape(k, nout), (xo.reshape(k, nxout) if xo is not None else None)
+        return out, xo
+
+    def last_density_batches(self) -> int:
+        """Passes over the densities the last batched block_response made (more than one when the workspace could not hold them all)."""
+        n = C.c_long()
+        _lib.check(self.lib.xtd_last_density_batches(self._h, C.byref(n)), "xtd_last_density_batches")
+        return n.value
 
     def sigma_host(self, z: np.ndarray) -> np.ndarray:
         """Reference-facing entry with HOST vectors: H2D + sigma + D2H inside the C-ABI call (single rank)."""

@@ -11,7 +11,9 @@ and Coulomb blocks, the MO-on-grid kernel contraction and the ROHF Fock coupling
 transposed density (`xtd_add_kterm_t`); the Krylov vectors live in HBM and the subspace algebra runs in the `xtd_vec_*` kernels.
 
 The collinear right-hand side (the Q matrix: J/K and f_xc images of occupied-occupied and virtual-virtual densities) and the W matrix
-come from `xtd_block_response` on the same engine (`ZVector.rhs`, `ZVector.w_matrix`).  The third-derivative kernel of multicollinear
+come from `xtd_block_response` on the same engine (`ZVector.rhs`, `ZVector.w_matrix`).  Several states at once: `ZVector.rhs_many`,
+`solve_many` and `w_matrices` make one `xtd_block_response_batch` call per response image for all states and solve on one block
+Krylov space (`solve_linear_block`) whose operator calls carry up to the engine's `max_nvec` vectors.  The third-derivative kernel of multicollinear
 functionals and the integral derivatives that follow the solve need pieces outside the sigma path (libxc third derivatives, libcint
 derivative integrals).
 """
@@ -82,6 +84,96 @@ def solve_linear(aop, b, hdiag, *, tol: float = 1e-12, max_cycle: int = 40, lind
     if k:
         vb.lincomb(x, V[:k], c[None], 0.0)
     return vb.to_host(x)[0], bool(conv), k, res
+
+
+def solve_linear_block(aop, b, hdiag, *, tol: float = 1e-12, max_cycle: int = 40, lindep: float = 1e-13, max_nvec: int = 4,
+                       backend=None, verbose: int = 0):
+    """`solve_linear` for k right-hand sides b[k, dim] on one shared Galerkin space.  A cycle takes the preconditioned residuals of
+    up to `max_nvec` unconverged systems (round robin when more are pending), orthonormalises each (CGS2) against the kept directions
+    and the ones accepted before it in the cycle, drops those below `lindep` one by one, and applies `aop` once to the accepted ones.
+When every direction of a cycle drops, the next pending systems are tried; the solve stops when a full round over them adds none.
+    The projected system is solved on the host for all k columns; a system whose residual falls below `tol` leaves the active set and
+    keeps that solution.  Each system contributes at most `max_cycle` directions, so the space holds at most k * max_cycle vectors.
+    With k = 1 the steps are those of `solve_linear`.
+
+    Returns (x_host[k, dim], converged[k], cycles[k], residual[k], aop calls); cycles[i] counts the aop calls up to system i's
+    convergence (all of them if it did not converge)."""
+    b = np.atleast_2d(np.asarray(b, dtype=np.float64))
+    k, dim = b.shape
+    vb = backend
+    if vb is None:
+        from .davidson import CudaVectors
+        vb = CudaVectors(dim)
+    mtot = min(k * max_cycle, dim)
+    V, AV = vb.alloc(max(mtot, 1)), vb.alloc(max(mtot, 1))
+    bd = vb.from_host(b)
+    hd = vb.from_host(np.asarray(hdiag, dtype=np.float64).ravel())
+    T, R, t = vb.alloc(k), vb.alloc(k), vb.alloc(1)
+    vb.copy(T, bd)
+    H = np.zeros((mtot, mtot))
+    G = np.zeros((mtot, k))
+    res = np.linalg.norm(b, axis=1)
+    conv = res < tol
+    coef = [np.zeros(0) for _ in range(k)]            # solution of system i on V[:len(coef[i])]
+    kept = np.zeros(k, dtype=int)
+    cycles = np.zeros(k, dtype=int)
+    m = ncall = 0
+    turn = 0
+    one = np.ones(1)
+    while m < mtot:
+        pending = [i for i in range(k) if not conv[i] and kept[i] < max_cycle]
+        if not pending:
+            break
+        m0 = m
+        tried = 0
+        while m == m0 and tried < len(pending) and m < mtot:   # a group whose directions all drop hands over to the next one
+            turn %= len(pending)
+            pick = (pending[turn:] + pending[:turn])[:min(max_nvec, len(pending) - tried)]
+            turn += len(pick)
+            tried += len(pick)
+            for i in pick:
+                if m >= mtot:
+                    break
+                vb.copy(t, T[i:i + 1])
+                n0 = float(vb.precond(t, hd, np.zeros(1))[0])
+                if n0 <= 0.0:
+                    continue
+                vb.scale(t, one / np.sqrt(n0))
+                for _ in range(2):
+                    if m:
+                        vb.lincomb(t, V[:m], -vb.dots(t, V[:m]), 1.0)
+                nrm2 = float(vb.dots(t, t)[0, 0])
+                if nrm2 <= lindep:
+                    continue
+                vb.scale(t, one / np.sqrt(nrm2))
+                vb.copy(V[m:m + 1], t)
+                kept[i] += 1
+                m += 1
+        if m == m0:
+            break                                      # a full round over the pending systems added nothing
+        vb.copy(AV[m0:m], aop(V[m0:m]))
+        ncall += 1
+        H[:m, m0:m] = vb.dots(V[:m], AV[m0:m])
+        H[m0:m, :m] = vb.dots(V[m0:m], AV[:m])
+        G[m0:m] = vb.dots(V[m0:m], bd)
+        act = np.nonzero(~conv)[0]
+        c = np.linalg.solve(H[:m, :m], G[:m, act])
+        vb.lincomb(R[:len(act)], AV[:m], np.ascontiguousarray(c.T), 0.0)
+        vb.lincomb(R[:len(act)], bd, -np.eye(k)[act], 1.0)          # r = A x - b
+        r2 = np.diag(vb.dots(R[:len(act)], R[:len(act)]))
+        for j, i in enumerate(act):
+            res[i] = float(np.sqrt(r2[j]))
+            coef[i] = c[:, j].copy()
+            cycles[i] = ncall
+            conv[i] = res[i] < tol
+            vb.copy(T[i:i + 1], R[j:j + 1])
+        if verbose:
+            print(f"zvector block solve: call {ncall}  space {m}  max |r| (active) = {res[act].max():.3e}")
+    x = vb.alloc(k)
+    for i in range(k):
+        if coef[i].size:
+            vb.lincomb(x[i:i + 1], V[:coef[i].size], coef[i][None], 0.0)
+    return vb.to_host(x), conv.copy(), cycles, res.copy(), ncall
 
 
 def rhs_intermediates(p, v, apply_response, apply_sf_exchange) -> dict:
@@ -279,6 +371,61 @@ def block_callables(p, plan, apply_blocks):
     return response((1.0, ck0, 0.0, cxc, 0.0)), (sf_exchange if p.hyb != 0.0 else None), response((1.0, ck0, ck1, cxc, 0.0))
 
 
+def block_callables_many(p, plan, apply_blocks):
+    """`block_callables` for k states per call: the callables take t[k, 2, nmo, nmo] / x[k, nmo, nmo] and return [k, 2, nmo, nmo] /
+    [k, nmo, nmo]; each state is converted with `mo_to_blocks` / `x_to_block`, and `apply_blocks(dens[k, n], coef, x[k, ...])` is
+    called once for all of them."""
+    nmo = p.nmo
+    cxc = 1.0 / plan.xc_scale if plan.xc_kind != "none" else 0.0
+    ck0 = -p.hyb if p.hybrid else 0.0
+    ck1 = -(p.alpha - p.hyb) if (p.hybrid and p.omega != 0.0 and p.has_df_lr) else 0.0
+
+    def response(coef):
+        def apply(t):
+            out = apply_blocks(np.stack([mo_to_blocks(plan, ti) for ti in t]), coef, None)[0]
+            return np.stack([blocks_to_mo(plan, o, nmo) for o in out])
+        return apply
+
+    def sf_exchange(x):
+        zero = mo_to_blocks(plan, np.zeros((2, nmo, nmo)))
+        xo = apply_blocks(np.stack([zero] * len(x)), (0.0, 0.0, 0.0, 0.0, 1.0), np.stack([x_to_block(plan, xi) for xi in x]))[1]
+        return np.stack([xblock_to_mo(plan, o, nmo) for o in xo])
+    return response((1.0, ck0, 0.0, cxc, 0.0)), (sf_exchange if p.hyb != 0.0 else None), response((1.0, ck0, ck1, cxc, 0.0))
+
+
+def per_state_batched(k, run_state, *many):
+    """Run the per-state bookkeeping `run_state(i, *callables)` for k states with ONE call of each batched callable in `many`
+    (None stays None).  A first pass records what each state hands each callable (returning zeros) and stops once every callable
+    has been seen, the batched callables map the stacked inputs, and a second pass gives every state its slice.  `run_state` must
+    call each non-None callable exactly once, and its inputs must not depend on the outputs -- true of `rhs_intermediates` (whose
+    `apply_sf_exchange` is None exactly when it is not called) and `assemble_w`."""
+    rec = [[None] * len(many) for _ in range(k)]
+    live = [j for j, fn in enumerate(many) if fn is not None]
+
+    class _AllSeen(Exception):
+        pass
+
+    def recorder(i, j):
+        def f(a):
+            rec[i][j] = np.array(a, dtype=np.float64, copy=True)
+            if all(rec[i][jj] is not None for jj in live):
+                raise _AllSeen                          # the bookkeeping after the last engine call is not needed in this pass
+            return np.zeros_like(rec[i][j])
+        return f
+    for i in range(k):
+        try:
+            run_state(i, *[recorder(i, j) if fn is not None else None for j, fn in enumerate(many)])
+        except _AllSeen:
+            pass
+    images = []
+    for j, fn in enumerate(many):
+        used = [i for i in range(k) if rec[i][j] is not None]
+        img = fn(np.stack([rec[i][j] for i in used])) if (fn is not None and used) else []
+        images.append(dict(zip(used, img)))
+    return [run_state(i, *[(lambda a, im=images[j][i]: im) if rec[i][j] is not None else None for j in range(len(many))])
+            for i in range(k)]
+
+
 class ZVector:
     """Operator and solver of the Z-vector equation for one mean-field reference.
 
@@ -359,6 +506,38 @@ class ZVector:
             f = self._mo_engines()[2]
             full = lambda t: f.sigma_host(t.reshape(1, -1))[0]
         return assemble_w(self.problem, z, self._inter, full)
+
+    # ---- several states at once (block route only) ------------------------------------------------------------------------------
+    def rhs_many(self, V):
+        """Right-hand sides [k, dim] for the states with amplitudes V[k, nc, nv]: one batched `xtd_block_response_batch` call per
+        response image for all k states; the k intermediates are kept for `w_matrices`."""
+        p = self.problem
+        V = np.asarray(V, dtype=np.float64).reshape(-1, self.nc, self.nv)
+        resp, sfx, _ = block_callables_many(p, self.plan, self.engine.block_response)
+        self._inters = per_state_batched(len(V), lambda i, r, x: rhs_intermediates(p, V[i], r, x), resp, sfx)
+        return np.stack([assemble_rhs(p, V[i], None, None, inter=it) for i, it in enumerate(self._inters)])
+
+    def solve_many(self, RHS, tol: Optional[float] = None, max_cycle: Optional[int] = None, lindep: float = 1e-13, verbose: int = 0):
+        """Solutions [k, dim] of the k systems with right-hand sides RHS[k, dim] (sign conventions of `solve`) on one block Krylov
+        space (`solve_linear_block`), each operator call carrying up to the engine's `max_nvec` vectors.  `self.converged`,
+        `self.cycles`, `self.residual` become per-state arrays; `self.aop_calls` counts the operator calls."""
+        rhs = np.atleast_2d(np.asarray(RHS, dtype=np.float64)).reshape(-1, self.dim)
+        if tol is None:
+            tol = 1e-12 if self.restricted else self.cphf_conv_tol
+        b = rhs if self.restricted else -rhs
+        z, self.converged, self.cycles, self.residual, self.aop_calls = solve_linear_block(
+            self.engine.sigma, b, self.hdiag, tol=tol, max_cycle=max_cycle or self.cphf_max_cycle, lindep=lindep,
+            max_nvec=self.engine.max_nvec, verbose=verbose)
+        return z
+
+    def w_matrices(self, Z):
+        """W matrices [k, nao, nao] from the solutions Z[k, dim] of the states of the last `rhs_many`, in the same order."""
+        inters = getattr(self, "_inters", None)
+        Z = np.atleast_2d(np.asarray(Z, dtype=np.float64)).reshape(-1, self.dim)
+        if inters is None or len(inters) != len(Z):
+            raise ValueError(f"w_matrices: {len(Z)} solutions for {0 if inters is None else len(inters)} states of the last rhs_many")
+        full = block_callables_many(self.problem, self.plan, self.engine.block_response)[2]
+        return np.stack(per_state_batched(len(Z), lambda i, f: assemble_w(self.problem, Z[i], inters[i], f), full))
 
     def split(self, z):
         """The rotation blocks the reference continues with: ROKS (zvc, zvo, zoc) (tdroks_sfu.py:328-330), UKS (z1a, z1b)."""
