@@ -6,8 +6,8 @@ from .XTDA import XTDA as _XTDA
 
 
 class XTDA(_XTDA):
-    def __init__(self, mol, mf, nstates=10, so2st=True):
-        super().__init__(mol, mf, nstates=nstates, basis="orbital", so2st=so2st, use_Davidson=True)
+    def __init__(self, mol, mf, nstates=10, so2st=True, core_idx=None):
+        super().__init__(mol, mf, nstates=nstates, basis="orbital", so2st=so2st, use_Davidson=True, core_idx=core_idx)
         self.level_shift = getattr(mf, "level_shift", 0) or 0
         self._settings = "gpu_class"
 

@@ -2467,7 +2467,10 @@ extern "C" int xtd_davidson(xtd_handle h, int nroots, const xtd_solver_opts* o, 
   XTD_REQUIRE(nroots >= 1 && nroots <= dim && n0 >= 1, XTD_ERR_ARG, "xtd_davidson: nroots %d / initial vectors %d", nroots, n0);
   cudaStream_t s = h->stream;
   const double tol = o->tol, toloose = o->tol_residual > 0.0 ? o->tol_residual : std::sqrt(o->tol), lindep = o->lindep;
-  const int max_space = o->max_space + (nroots - 1) * 4;
+  // nroots close to dim (core-valence-separated spaces): the subspace may grow to the whole space, so it never restarts and never
+  // takes more new vectors than there are dimensions left
+  const bool whole = (long)o->max_space + (nroots - 1) * 4 >= dim;
+  const int max_space = (int)std::min<long>(o->max_space + (nroots - 1) * 4, dim);
   const int cap = max_space + nroots + 40;
   const int nxt = std::max(std::max(n0, nroots), 40);
   DavBuf xs, ax, xt, axt, ritz, aritz, tmp, gdev, cdev, ndev, sdev;
@@ -2649,7 +2652,7 @@ extern "C" int xtd_davidson(xtd_handle h, int nroots, const xtd_solver_opts* o, 
       if (ng) {
         std::vector<double> inv(ng);
         for (int a = 0; a < ng; ++a) inv[a] = 1.0 / std::sqrt(gh.p[(size_t)good[a] * nt + good[a]]);
-        const bool will_restart = space + nroots > max_space;
+        const bool will_restart = space + nroots > max_space && !whole;
         if (ng > 1 && !will_restart) {
           std::vector<double> gs((size_t)ng * ng);
           for (int a = 0; a < ng; ++a)
@@ -2682,12 +2685,13 @@ extern "C" int xtd_davidson(xtd_handle h, int nroots, const xtd_solver_opts* o, 
         nt = 0;
       }
     }
+    if (whole) nt = (int)std::min<long>(nt, dim - space);
     if (nt == 0) {
       for (int k = 0; k < nritz; ++k) conv[k] = dxn[k] < toloose ? 1 : 0;
       ++icyc;
       break;
     }
-    fresh = space + nroots > max_space;
+    fresh = space + nroots > max_space && !whole;
     if (fresh) {
       XTD_CUDA(cudaMemcpyAsync(xt.d, ritz.d, (size_t)nritz * dim * 8, cudaMemcpyDeviceToDevice, s));
       nt = nritz;

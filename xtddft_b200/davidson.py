@@ -204,6 +204,10 @@ def davidson1(aop: Callable, x0, precond, tol: float = 1e-12, max_cycle: int = 5
     dim = x0.shape[1]
     vb = backend if backend is not None else CudaVectors(dim)
     max_space = max_space + (nroots - 1) * 4
+    # nroots close to dim (core-valence-separated spaces): the subspace may grow to the whole space, so it never restarts and
+    # never takes more new vectors than there are dimensions left
+    whole = max_space >= dim
+    max_space = min(max_space, dim)
     cap = max_space + nroots + 40
     xs = vb.alloc(cap)
     ax = vb.alloc(cap)
@@ -323,7 +327,7 @@ def davidson1(aop: Callable, x0, precond, tol: float = 1e-12, max_cycle: int = 5
                 inv = 1.0 / np.sqrt(n2[good])
                 sel = np.zeros((len(good), nt))
                 sel[np.arange(len(good)), good] = inv
-                if len(good) > 1 and not (space + nroots > max_space):
+                if len(good) > 1 and not (space + nroots > max_space and not whole):
                     gs = gm[np.ix_(good, good)] * inv[:, None] * inv[None, :]
                     t1 = _gs_coefficients(gs, lindep)
                     vb.transform(xt, nt, t1 @ sel)
@@ -340,10 +344,12 @@ def davidson1(aop: Callable, x0, precond, tol: float = 1e-12, max_cycle: int = 5
                     nt = len(good)
             else:
                 nt = 0
+        if whole:
+            nt = min(nt, dim - space)
         if nt == 0:
             conv = dx_norm < toloose
             break
-        fresh_start = space + nroots > max_space
+        fresh_start = space + nroots > max_space and not whole
         if fresh_start:
             # restart from the current Ritz vectors (reference: x0 = _gen_x0(v, xs) then re-orthogonalised)
             if xt.shape[0] < nritz:

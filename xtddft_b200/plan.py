@@ -206,20 +206,55 @@ def xtda_coeffs(s: float):
     return 0.5 * (1 - r + 1 / (2 * s)), 0.5 * (-1 + r + 1 / (2 * s)), 0.5 / (2 * s)
 
 
-def build_xtda_plan(p: ProblemData) -> Plan:
+def _core_index(idx, n: int, what: str) -> np.ndarray:
+    a = np.asarray(idx)
+    if a.ndim != 1 or a.size == 0 or not np.issubdtype(a.dtype, np.integer):
+        raise ValueError(f"core: {what} must be a non-empty 1-D sequence of integers, got {idx!r}")
+    if np.any(np.diff(a) <= 0):
+        raise ValueError(f"core: {what} must be unique and sorted, got {a.tolist()}")
+    if a[0] < 0 or a[-1] >= n:
+        raise ValueError(f"core: {what} must lie in [0, {n}), got {a.tolist()}")
+    return a.astype(np.int64)
+
+
+def cvs_core(p: ProblemData, core) -> Tuple[np.ndarray, np.ndarray]:
+    """Check a core-valence-separation core set and return (core_a, core_b), the occupied rows each spin channel keeps.
+
+    ROKS: `core` lists closed-shell orbitals (< nc); both spins keep the same rows.  UKS: `core = (core_a, core_b)`, indices into
+    the occupied orbitals of each spin.  Indices must be unique and sorted; anything else raises ValueError."""
+    if p.restricted:
+        c = _core_index(core, p.nc, "closed-shell orbital indices")
+        return c, c.copy()
+    if not isinstance(core, (tuple, list)) or len(core) != 2:
+        raise ValueError(f"core: a UKS reference takes a pair (core_a, core_b), got {core!r}")
+    return _core_index(core[0], p.nocc_a, "core_a"), _core_index(core[1], p.nocc_b, "core_b")
+
+
+def build_xtda_plan(p: ProblemData, core=None) -> Plan:
+    """X-TDA plan.  `core`: core-valence separation (see `cvs_core`) -- the plan of P A P, where P keeps the rows (i, a) whose
+    occupied orbital i is a core orbital; ext vectors are [alpha (core_a i, a) | beta (core_b i, a)] in PySCF order."""
     nc, no, nv = p.nc, p.no, p.nv
     na, nb, nva, nvb = p.nocc_a, p.nocc_b, p.nvir_a, p.nvir_b
-    # alpha: occ = [c | o] (two row blocks, rows need no padding but keep the even rule for transposed use), vir = v
-    occ_a, ob_a = _two_block(nc, no, 0)
+    if core is None:
+        # alpha: occ = [c | o] (two row blocks, rows need no padding but keep the even rule for transposed use), vir = v
+        occ_a, ob_a = _two_block(nc, no, 0)
+        # beta: occ = c, vir = [o | pad | v]
+        occ_b = np.arange(nb, dtype=np.int32)
+        core_a, core_b = np.arange(na), np.arange(nb)
+        ncv = nc                                         # alpha rows of the CV(aa) block
+    else:
+        core_a, core_b = cvs_core(p, core)
+        occ_a, ob_a = core_a.astype(np.int32), [(0, len(core_a))]
+        occ_b = core_b.astype(np.int32)
+        ncv = len(core_a)                                # ROKS: every core row is closed
     vir_a = (na + np.arange(nva)).astype(np.int32)
-    # beta: occ = c, vir = [o | pad | v]
-    occ_b = np.arange(nb, dtype=np.int32)
     vir_b, vb_b = _two_block(no, nv, nb)
+    nra, nrb = len(core_a), len(core_b)
     cha = ChannelSpec(0, occ_a, 0, vir_a, ob_a, [(0, nva)])
-    chb = ChannelSpec(1, occ_b, 1, vir_b, [(0, nb)], vb_b)
+    chb = ChannelSpec(1, occ_b, 1, vir_b, [(0, nrb)], vb_b)
     plan = Plan("xtda", [cha, chb])
     oa_pos, va_pos = _pos(ob_a), np.arange(nva)
-    ob_pos, vb_pos = np.arange(nb), _pos(vb_b)
+    ob_pos, vb_pos = np.arange(nrb), _pos(vb_b)
     v2off = vb_b[1][0] if len(vb_b) > 1 else 0
     o2off = ob_a[1][0] if len(ob_a) > 1 else 0
 
@@ -234,9 +269,9 @@ def build_xtda_plan(p: ProblemData) -> Plan:
     if p.restricted:
         # Fock blocks: sigma += z F_vv^T - F_oo z   (XTDA.py:629-632, 658-661)
         fvv_a = _embed(fa[na:, na:], va_pos, va_pos, cha.nv, cha.nv)
-        foo_a = _embed(fa[:na, :na], oa_pos, oa_pos, cha.no, cha.no)
+        foo_a = _embed(fa[np.ix_(core_a, core_a)], oa_pos, oa_pos, cha.no, cha.no)
         fvv_b = _embed(fb[nb:, nb:], vb_pos, vb_pos, chb.nv, chb.nv)
-        foo_b = _embed(fb[:nb, :nb], ob_pos, ob_pos, chb.no, chb.no)
+        foo_b = _embed(fb[np.ix_(core_b, core_b)], ob_pos, ob_pos, chb.no, chb.no)
         plan.local_gemms += [
             LocalGemm("R", (0, 0, cha.no, 0, cha.nv), (0, 0, 0), fvv_a.T.copy(), 1.0),
             LocalGemm("L", (0, 0, cha.no, 0, cha.nv), (0, 0, 0), foo_a, -1.0),
@@ -247,9 +282,9 @@ def build_xtda_plan(p: ProblemData) -> Plan:
         fha, fhb = p.fock_hf
         c1, c2, c3 = xtda_coeffs(p.spin_s)
         dvv = (fhb[na:, na:] - fha[na:, na:])           # nv x nv
-        dcc = (fhb[:nb, :nb] - fha[:nb, :nb])           # nc x nc
-        cva = (0, 0, nc, 0, nv)                          # CV(aa): rows c of alpha
-        cvb = (1, 0, nc, v2off, nv)                      # CV(bb): cols v of beta
+        dcc = (fhb - fha)[np.ix_(core_b, core_b)]        # nc x nc (CVS: core x core)
+        cva = (0, 0, ncv, 0, nv)                         # CV(aa): rows c of alpha
+        cvb = (1, 0, ncv, v2off, nv)                     # CV(bb): cols v of beta
         plan.local_gemms += [
             LocalGemm("R", cva, (0, 0, 0), dvv.T.copy(), c1), LocalGemm("L", cva, (0, 0, 0), dcc, c2),
             LocalGemm("R", cva, (1, 0, v2off), dvv.T.copy(), -c3), LocalGemm("L", cva, (1, 0, v2off), dcc, -c3),
@@ -259,19 +294,19 @@ def build_xtda_plan(p: ProblemData) -> Plan:
         da, db = fa.diagonal(), fb.diagonal()
     else:
         ea, eb = p.mo_energy
-        e_a = ea[na:] - ea[:na, None]
-        e_b = eb[nb:] - eb[:nb, None]
+        e_a = ea[na:] - ea[core_a, None]
+        e_b = eb[nb:] - eb[core_b, None]
         plan.diags += [DiagTerm(0, _embed(e_a, oa_pos, va_pos, cha.no, cha.nv)),
                        DiagTerm(1, _embed(e_b, ob_pos, vb_pos, chb.no, chb.nv))]
         da, db = ea, eb
-    e_a = da[na:] - da[:na, None]
-    e_b = db[nb:] - db[:nb, None]
+    e_a = da[na:] - da[core_a, None]
+    e_b = db[nb:] - db[core_b, None]
     plan.hdiag = np.hstack([e_a.ravel(), e_b.ravel()])
 
     # layout: PySCF order [alpha (i,a) | beta (i,a)]
     ia, aa = np.meshgrid(oa_pos, va_pos, indexing="ij")
     ib, ab = np.meshgrid(ob_pos, vb_pos, indexing="ij")
-    n_a, n_b = na * nva, nb * nvb
+    n_a, n_b = nra * nva, nrb * nvb
     ent = np.zeros((n_a + n_b, 4), dtype=np.int64)
     ent[:, 0] = np.arange(n_a + n_b)
     ent[:n_a, 1], ent[:n_a, 2], ent[:n_a, 3] = 0, ia.ravel(), aa.ravel()
@@ -279,6 +314,8 @@ def build_xtda_plan(p: ProblemData) -> Plan:
     plan.ext_dim = n_a + n_b
     plan.layout_entries, plan.layout_coefs = ent, np.ones(n_a + n_b)
     plan.meta = dict(nc=nc, no=no, nv=nv, o2off=o2off, v2off=v2off)
+    if core is not None:
+        plan.meta.update(core_a=core_a, core_b=core_b)
     return plan
 
 

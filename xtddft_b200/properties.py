@@ -175,22 +175,26 @@ class PropertyPass:
         return x.contiguous()
 
     # ---- X-TDA: ground -> excited moments (PySCF order rows) ------------------------------------------------
-    def xtda_moments(self, x_rows, ints_ao: np.ndarray) -> np.ndarray:
-        """trans[s, k] (XTDA.py:849-857): Gram product of the amplitude rows with the MO-basis integral rows."""
+    def xtda_moments(self, x_rows, ints_ao: np.ndarray, rows: Optional[np.ndarray] = None) -> np.ndarray:
+        """trans[s, k] (XTDA.py:849-857): Gram product of the amplitude rows with the MO-basis integral rows.  `rows`: the amplitudes
+        live on these rows of the PySCF-order layout only (core-valence separation, `utils.cvs_rows`)."""
         p = self.p
         ca, cb = p.mo_coeff
         na, nb = p.nocc_a, p.nocc_b
         ma = self.mo_transform(ints_ao, ca[:, :na], ca[:, na:]).reshape(len(ints_ao), -1)
         mb = self.mo_transform(ints_ao, cb[:, :nb], cb[:, nb:]).reshape(len(ints_ao), -1)
-        return self._dots(self._rows(x_rows), self._rows(np.hstack([ma, mb])))
+        m = np.hstack([ma, mb])
+        if rows is not None:
+            m = m[:, rows]
+        return self._dots(self._rows(x_rows), self._rows(m))
 
-    def xtda_osc_str(self, e: np.ndarray, x_rows, dip_ao: np.ndarray) -> np.ndarray:
-        td = self.xtda_moments(x_rows, dip_ao)
+    def xtda_osc_str(self, e: np.ndarray, x_rows, dip_ao: np.ndarray, rows: Optional[np.ndarray] = None) -> np.ndarray:
+        td = self.xtda_moments(x_rows, dip_ao, rows)
         return 2.0 / 3.0 * np.asarray(e) * np.einsum("sx,sx->s", td, td)
 
-    def xtda_rot_str(self, e: np.ndarray, x_rows, ipovlp_ao: np.ndarray, irxp_ao: np.ndarray) -> np.ndarray:
-        ele = -self.xtda_moments(x_rows, ipovlp_ao)
-        mag = 0.5 * self.xtda_moments(x_rows, irxp_ao)
+    def xtda_rot_str(self, e: np.ndarray, x_rows, ipovlp_ao: np.ndarray, irxp_ao: np.ndarray, rows: Optional[np.ndarray] = None) -> np.ndarray:
+        ele = -self.xtda_moments(x_rows, ipovlp_ao, rows)
+        mag = 0.5 * self.xtda_moments(x_rows, irxp_ao, rows)
         return np.einsum("s,sx,sx->s", 1.0 / np.asarray(e), ele, mag) / CGS2AU
 
     # ---- spin-flip states: bilinear forms through operator plans ---------------------------------------------

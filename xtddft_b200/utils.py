@@ -26,7 +26,46 @@ def _split_my(v, nc, no, nv):
     return v[:d1], v[d1:d2], v[d2:d3], v[d3:]
 
 
-def so2st(eigvec, nc, no, nv):
+def cvs_rows(nc: int, no: int, nv: int, core_a, core_b) -> np.ndarray:
+    """Rows of the core-valence-separated X-TDA layout inside the full PySCF order: [alpha (i in core_a, a) | beta (i in core_b, a)],
+    the order of `plan.build_xtda_plan(p, core)`."""
+    na, nvb = nc + no, no + nv
+    ra = (np.asarray(core_a, dtype=np.int64)[:, None] * nv + np.arange(nv)).ravel()
+    rb = na * nv + (np.asarray(core_b, dtype=np.int64)[:, None] * nvb + np.arange(nvb)).ravel()
+    return np.concatenate([ra, rb])
+
+
+def cvs_embed(x, rows, dim: int) -> np.ndarray:
+    """Vectors on the rows `rows` of a `dim`-row layout (first axis) zero-padded to the whole layout."""
+    x = np.asarray(x)
+    out = np.zeros((dim,) + x.shape[1:], dtype=x.dtype)
+    out[rows] = x
+    return out
+
+
+def cvs_order_pyscf2my(nc: int, no: int, nv: int, core_a, core_b):
+    """(order, my_rows): `x[order]` takes core-valence-separated vectors from PySCF order to the order of `order_pyscf2my`
+    restricted to the core rows [CV(aa) | OV(aa) | CO(bb) | CV(bb)]; `my_rows` are those rows inside the full order_pyscf2my layout."""
+    rows = cvs_rows(nc, no, nv, core_a, core_b)
+    full = order_pyscf2my(nc, no, nv)
+    inv = np.full(full.size, -1, dtype=np.int64)
+    inv[rows] = np.arange(rows.size)
+    sel = inv[full]
+    keep = sel >= 0
+    return sel[keep], np.nonzero(keep)[0]
+
+
+def so2st(eigvec, nc, no, nv, core=None):
+    """Spin-orbital -> singlet / triplet combinations of the CV blocks.  `core = (core_a, core_b)`: `eigvec` holds core-valence-
+    separated vectors in `cvs_order_pyscf2my` order; the result is the full-space so2st of the zero-padded vectors, on the core rows.
+    The singlet / triplet pairs stay on the core rows only when the closed alpha core rows are exactly the beta core rows."""
+    if core is not None:
+        core_a, core_b = (np.asarray(c) for c in core)
+        if not np.array_equal(core_a[core_a < nc], core_b):
+            raise ValueError("so2st: the closed-shell alpha core orbitals must be the beta core orbitals")
+        _, my_rows = cvs_order_pyscf2my(nc, no, nv, core_a, core_b)
+        full = cvs_embed(eigvec, my_rows, (nc + no) * nv + nc * (no + nv))
+        return so2st(full, nc, no, nv)[my_rows]
     cva, ova, cob, cvb = _split_my(eigvec, nc, no, nv)
     r = np.sqrt(2.0) / 2.0
     return np.concatenate((r * (cva + cvb), ova, cob, r * (cva - cvb)), axis=0)
